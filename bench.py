@@ -8,6 +8,7 @@ global index space (weak scaling: per-GPU work fixed) with no data-path collecti
 the final NCCL all-gather of the points the north star names.
 
   python bench.py [--gpus N --steps K --warmup W] [--impl reference] [--mode matrix|ray] [--precision f64|f32]
+                  [--dump-outputs DIR]
 
 Prints ONE JSON line (rank 0).  `--impl reference` times the CPU restatement of the reference
 (oracle/, all host threads) on a bounded sample of the same workload.
@@ -40,7 +41,14 @@ def parse():
     ap.add_argument("--no-e2e", action="store_true")
     ap.add_argument("--no-cpu", action="store_true")
     ap.add_argument("--cpu-seconds", type=float, default=12.0)
-    return ap.parse_args()
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="write the points the last timed step computed (rank 0's frames) to DIR/<name>.npy (see dump_outputs)")
+    a = ap.parse_args()
+    if a.steps < 1 or a.warmup < 0:
+        ap.error("--steps must be at least 1 and --warmup at least 0")
+    if a.dump_outputs and a.impl != "b200":
+        ap.error("--dump-outputs writes what the GPU path computed; the reference arm keeps no outputs")
+    return a
 
 
 class ClockSampler:
@@ -108,6 +116,27 @@ def bind_to_gpu_numa_node(index):
     except Exception:
         pass
     return None
+
+
+DUMP_SAMPLE = 1 << 21  # frames kept when the whole output is larger than DUMP_BYTES
+DUMP_BYTES = 64 << 20
+
+
+def dump_outputs(path, xyz):
+    """Write the [frames, 3] float32 points of one step as path/xyz_f32.npy.  Above DUMP_BYTES, a fixed, seeded sample
+    of the frames (the same one on every run with the same --frames), with their indices in path/frame_index.npy
+    (float64, exact for any frame count).  The inputs are a pure function of the frame index, so two builds of the
+    project can be compared output for output."""
+    import numpy as np
+    import torch
+    os.makedirs(path, exist_ok=True)
+    n = xyz.shape[0]
+    if n * xyz.element_size() * 3 <= DUMP_BYTES:
+        np.save(os.path.join(path, "xyz_f32.npy"), xyz.cpu().numpy())
+        return
+    idx = np.unique(np.random.default_rng(0).integers(0, n, DUMP_SAMPLE))
+    np.save(os.path.join(path, "xyz_f32.npy"), xyz[torch.from_numpy(idx).to(xyz.device)].cpu().numpy())
+    np.save(os.path.join(path, "frame_index.npy"), idx.astype(np.float64))
 
 
 def oracle_cams(cams):
@@ -312,6 +341,8 @@ def main():
     clk.__enter__()  # sampled over the timed region and the companion kernel timings that follow (all HBM-resident passes)
     total_ms, per, launches = timed(step, a.steps, a.warmup)
     eng.device_status()
+    if a.dump_outputs and rank == 0:  # before the companion timings below write other kernels' points into `out`
+        dump_outputs(a.dump_outputs, out["xyz_f32"])
     ms_per_step = total_ms / a.steps
     value = valid_total / (ms_per_step * 1e-3)
     kernel_ms = sum(per) / len(per)

@@ -113,6 +113,27 @@ def test_classifier_ray_is_the_references(ds, frames):
     assert ref["stats"]["lm_iters"] == orc["stats"]["lm_iters"] and ref["stats"]["solves"] == orc["stats"]["solves"]
 
 
+@pytest.mark.parametrize("ds", list(DATASETS))
+def test_stored_reference_outputs_are_the_references(ds):
+    """tests/golden/golden_ref_<ds>.npz (oracle/make_golden_ref.py), what tests/test_gpu_ref.py compares the CUDA path
+    with, is what the reference's own code computes: classifier runs, accepted errors, margins, batch points."""
+    z = np.load("%s/golden_ref_%s.npz" % (G, ds))
+    xml, cams, offs, xy, nc, nf = load(ds)
+    ref = R.Reference(xml=xml, mode=R.MATRIX).classify(DATASETS[ds], offs, xy, nf)
+    for k in ("assign", "phase", "paths", "err"):
+        assert np.array_equal(ref[k], z["matrix_" + k]), k
+    assert ref["margins"]["error"] == z["matrix_margin_error"] and ref["margins"]["gate"] == z["matrix_margin_gate"]
+    if "ray_paths" in z.files:
+        xml, cams, offs, xy, nc, nf = load(ds, z["ray_paths"].shape[1])
+        ref = R.Reference(xml=xml, mode=R.RAY).classify(DATASETS[ds], offs, xy, nf)
+        for k in ("assign", "phase", "paths"):
+            assert np.array_equal(ref[k], z["ray_" + k]), k
+    if "batch_matrix_xyz" in z.files:
+        pts = O.dets_to_points(offs, xy, nc, nf)
+        for mode, k in ((R.MATRIX, "batch_matrix_xyz"), (R.RAY, "batch_ray_xyz")):
+            assert np.array_equal(R.Reference(xml=xml, mode=mode).triangulate_points(pts), z[k]), k
+
+
 def test_reference_cli_runs_end_to_end(tmp_path):
     """oracle/_ref/ref_main is the reference's main.cpp: same flags, ./results/drone<i>.ply, 'Execution time' line."""
     import subprocess
