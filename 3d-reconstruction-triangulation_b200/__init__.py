@@ -67,7 +67,7 @@ class ClassifyStats(C.Structure):
 
 EXPORTS = ["tri_version", "tri_last_error", "tri_device_count", "tri_create", "tri_destroy", "tri_engine_device",
            "tri_engine_cameras", "tri_kernel_launches", "tri_triangulate_points", "tri_triangulate_points_multi",
-           "tri_triangulate_points_device",
+           "tri_triangulate_points_device", "tri_triangulate_points_robust", "tri_triangulate_points_robust_device",
            "tri_device_status", "tri_enable_peer_access", "tri_ipc_export", "tri_ipc_open", "tri_ipc_close",
            "tri_copy_device", "tri_triangulate_subsets", "tri_dist_from_ray", "tri_classify", "tri_classify_state_bytes",
            "tri_classify_begin", "tri_classify_finish", "tri_classify_multi", "tri_classify_sequences", "tri_host_alloc",
@@ -99,6 +99,10 @@ def lib():
                                                    C.c_int64, C.POINTER(_BatchOut), C.POINTER(C.c_int64)]
         L.tri_triangulate_points_device.argtypes = [C.c_void_p, C.c_int, C.c_uint, C.c_void_p, C.c_int, C.c_int64,
                                                     C.c_int64, C.POINTER(_BatchOut), C.c_void_p]
+        L.tri_triangulate_points_robust.argtypes = [C.c_void_p, C.c_uint, C.c_double, C.c_void_p, C.c_int, C.c_int64, C.c_int64,
+                                                    C.POINTER(_BatchOut), C.POINTER(C.c_int64)]
+        L.tri_triangulate_points_robust_device.argtypes = [C.c_void_p, C.c_uint, C.c_double, C.c_void_p, C.c_int, C.c_int64,
+                                                           C.c_int64, C.POINTER(_BatchOut), C.c_void_p]
         L.tri_enable_peer_access.argtypes = [C.c_void_p, C.c_int]
         L.tri_ipc_export.argtypes = [C.c_void_p, C.c_void_p, C.c_char_p]
         L.tri_ipc_open.argtypes = [C.c_void_p, C.c_char_p, C.POINTER(C.c_void_p)]
@@ -383,6 +387,43 @@ class Engine:
         st = lib().tri_triangulate_points(self._h, mode, flags, C.c_void_p(xy_ptr), npc, nf, stride, C.byref(bo), C.byref(bad))
         _check(st, mode)
         return bad.value
+
+    # ---- outlier-robust matrix-mode batch (two-view consensus, inlier refit; an extension of the reference) ----
+    def triangulate_points_robust(self, xy, max_reproj_px, flags=0, want=("xyz_f64", "mask", "err")):
+        """xy: numpy [n_point_cams, n_frames, 2] float32 | float64 | uint16 (host memory).  mask = the inlier set,
+        err = RMS reprojection error in pixels over it (NaN where no two views agree within max_reproj_px)."""
+        xy = np.asarray(xy)
+        if xy.ndim != 3 or xy.shape[2] != 2:
+            raise TriError(ERR_DIM, MSG_DIM)
+        xy = np.ascontiguousarray(xy)
+        npc, nf = xy.shape[0], xy.shape[1]
+        out = {k: np.empty({"xyz_f32": (nf, 3), "xyz_f64": (nf, 3)}.get(k, (nf,)),
+                           {"xyz_f32": np.float32, "xyz_f64": np.float64, "mask": np.uint32, "err": np.float64}[k]) for k in want}
+        bo = _BatchOut(*[out[k].ctypes.data if k in out else None for k in ("xyz_f32", "xyz_f64", "mask", "err", "iters")])
+        bad = C.c_int64(-1)
+        st = lib().tri_triangulate_points_robust(self._h, flags | _PIX_DTYPES[xy.dtype], float(max_reproj_px), _np_ptr(xy), npc, nf,
+                                                 nf, C.byref(bo), C.byref(bad))
+        out["first_bad_frame"] = bad.value
+        _check(st)
+        return out
+
+    def triangulate_points_robust_device(self, xy, max_reproj_px, flags=0, out=None, want=("xyz_f64", "mask", "err")):
+        """xy: torch tensor [n_point_cams, n_frames, 2] on cuda:<device>, asynchronous on the current stream; the
+        too-few latch is collected by device_status().  Outputs as triangulate_points_robust, as torch tensors."""
+        import torch
+        assert xy.is_cuda and xy.dim() == 3 and xy.shape[2] == 2 and xy.stride(2) == 1 and xy.stride(1) == 2
+        fmt = {torch.float32: 0, torch.float64: PIX_F64, torch.uint16: PIX_U16}[xy.dtype]
+        npc, nf = xy.shape[0], xy.shape[1]
+        stride = xy.stride(0) // 2 if npc > 1 else nf
+        if out is None:
+            out = {k: torch.empty({"xyz_f32": (nf, 3), "xyz_f64": (nf, 3)}.get(k, (nf,)),
+                                  dtype={"xyz_f32": torch.float32, "xyz_f64": torch.float64, "mask": torch.int32,
+                                         "err": torch.float64}[k], device=xy.device) for k in want}
+        bo = _BatchOut(*[out[k].data_ptr() if k in out else None for k in ("xyz_f32", "xyz_f64", "mask", "err", "iters")])
+        stream = torch.cuda.current_stream(xy.device).cuda_stream
+        _check(lib().tri_triangulate_points_robust_device(self._h, flags | fmt, float(max_reproj_px), C.c_void_p(xy.data_ptr()), npc, nf,
+                                                          stride, C.byref(bo), C.c_void_p(stream)))
+        return out
 
     # ---- Triangulator::triangulatePoint over many camera subsets ----
     def triangulate_subsets(self, mode, items, flags=0):

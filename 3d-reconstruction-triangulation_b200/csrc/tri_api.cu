@@ -271,6 +271,98 @@ static int ensure(char** p, size_t* cap, size_t need) {
 
 static size_t align_up(size_t v, size_t a) { return (v + a - 1) / a * a; }
 
+// Device entry points without a single pixel row: every frame has too few views -- zero outputs, frame 0 latched.
+static int too_few_device(tri_engine* e, int64_t n_frames, const BatchOut& out, cudaStream_t stream) {
+  TRI_CUDA(cudaMemsetAsync(e->d_first_bad, 0, sizeof(unsigned long long), stream));
+  if (out.xyz_f32) TRI_CUDA(cudaMemsetAsync(out.xyz_f32, 0, sizeof(float) * 3 * n_frames, stream));
+  if (out.xyz_f64) TRI_CUDA(cudaMemsetAsync(out.xyz_f64, 0, sizeof(double) * 3 * n_frames, stream));
+  if (out.mask) TRI_CUDA(cudaMemsetAsync(out.mask, 0, sizeof(uint32_t) * n_frames, stream));
+  if (out.err) TRI_CUDA(cudaMemsetAsync(out.err, 0, sizeof(double) * n_frames, stream));
+  if (out.iters) TRI_CUDA(cudaMemsetAsync(out.iters, 0, sizeof(int32_t) * n_frames, stream));
+  return TRI_OK;
+}
+
+// Arguments of the robust pair: matrix mode only, its own flag set, a positive threshold, no iteration output.
+static int check_robust_args(tri_engine* e, unsigned flags, double max_reproj_px, const void* xy, int n_point_cams, int64_t n_frames,
+                             int64_t cam_stride, const tri_batch_out* out, int* n_use) {
+  const unsigned allowed = TRI_F32 | TRI_PIX_F64 | TRI_PIX_U16 | TRI_ALLOW_TOO_FEW;
+  if (flags & ~allowed) return fail(TRI_ERR_ARG, "robust triangulation accepts TRI_F32, TRI_PIX_F64, TRI_PIX_U16 and TRI_ALLOW_TOO_FEW only");
+  if (!(max_reproj_px > 0)) return fail(TRI_ERR_ARG, "max_reproj_px must be > 0");
+  if (out && out->iters) return fail(TRI_ERR_ARG, "robust triangulation has no iteration output (iters must be NULL)");
+  return check_batch_args(e, TRI_MATRIX, flags, xy, n_point_cams, n_frames, cam_stride, out, n_use);
+}
+
+// Host-buffer batch: frames stream through N_SLOTS device staging slots, one CUDA stream each, so the
+// H2D copy of a chunk overlaps the kernel of the previous one and the D2H copy of the one before.
+// `launch(ctx, d_xy, n, cam_stride, out)` solves one chunk already on the device.
+template <class Launch>
+static int run_host_pipeline(tri_engine* e, unsigned flags, int fmt, const void* xy, int n_use, int64_t n_frames, int64_t cam_stride,
+                             int64_t chunk, const tri_batch_out* out, int64_t* first_bad_frame, const char* too_few_msg, Launch launch) {
+  const size_t pb = pix_bytes(fmt);
+  if (n_frames <= chunk) chunk = (n_frames + 1) / 2 * 2;  // one chunk
+  const size_t in_row = align_up((size_t)chunk * pb, 256);
+  const size_t o_xyz32 = 0;
+  const size_t o_xyz64 = o_xyz32 + (out->xyz_f32 ? align_up((size_t)chunk * 12, 256) : 0);
+  const size_t o_mask = o_xyz64 + (out->xyz_f64 ? align_up((size_t)chunk * 24, 256) : 0);
+  const size_t o_err = o_mask + (out->mask ? align_up((size_t)chunk * 4, 256) : 0);
+  const size_t o_iters = o_err + (out->err ? align_up((size_t)chunk * 8, 256) : 0);
+  const size_t out_bytes = o_iters + (out->iters ? align_up((size_t)chunk * 4, 256) : 0);
+  const int n_slots = n_frames > chunk ? N_SLOTS : 1;
+  int st;
+  for (int i = 0; i < n_slots; i++) {
+    if ((st = ensure(&e->slots[i].d_in, &e->slots[i].in_cap, in_row * std::max(n_use, 1))) != TRI_OK) return st;
+    if ((st = ensure(&e->slots[i].d_out, &e->slots[i].out_cap, out_bytes)) != TRI_OK) return st;
+  }
+  unsigned long long* latch = e->d_first_bad + 1;  // the host path's own latch: a pending one of the device entry point stays
+  TRI_CUDA(cudaMemsetAsync(latch, 0xff, sizeof(unsigned long long), e->slots[0].stream));
+  TRI_CUDA(cudaStreamSynchronize(e->slots[0].stream));
+  const char* src = static_cast<const char*>(xy);
+  // the chunk loop; on any failure the copies already queued into the caller's buffers are drained before returning
+  auto run = [&]() -> int {
+    int k = 0;
+    for (int64_t f0 = 0; f0 < n_frames; f0 += chunk, k++) {
+      Slot& s = e->slots[k % n_slots];
+      const int64_t n = std::min(chunk, n_frames - f0);
+      TRI_CUDA(cudaStreamSynchronize(s.stream));  // slot free (its previous D2H has landed)
+      for (int c = 0; c < n_use; c++)
+        TRI_CUDA(cudaMemcpyAsync(s.d_in + (size_t)c * in_row, src + ((size_t)c * cam_stride + f0) * pb, (size_t)n * pb,
+                                 cudaMemcpyHostToDevice, s.stream));
+      BatchOut o{out->xyz_f32 ? (float*)(s.d_out + o_xyz32) : nullptr, out->xyz_f64 ? (double*)(s.d_out + o_xyz64) : nullptr,
+                 out->mask ? (uint32_t*)(s.d_out + o_mask) : nullptr, out->err ? (double*)(s.d_out + o_err) : nullptr,
+                 out->iters ? (int32_t*)(s.d_out + o_iters) : nullptr};
+      if (n_use == 0) {
+        TRI_CUDA(cudaMemsetAsync(s.d_out, 0, out_bytes, s.stream));
+        TRI_CUDA(cudaMemsetAsync(latch, 0, sizeof(unsigned long long), s.stream));
+      } else {
+        const int st2 = launch(e->ctx(s.stream, f0, true), (const void*)s.d_in, n, (int64_t)(in_row / pb), o);
+        if (st2 != TRI_OK) return st2;
+      }
+      if (out->xyz_f32) TRI_CUDA(cudaMemcpyAsync(out->xyz_f32 + 3 * f0, o.xyz_f32, (size_t)n * 12, cudaMemcpyDeviceToHost, s.stream));
+      if (out->xyz_f64) TRI_CUDA(cudaMemcpyAsync(out->xyz_f64 + 3 * f0, o.xyz_f64, (size_t)n * 24, cudaMemcpyDeviceToHost, s.stream));
+      if (out->mask) TRI_CUDA(cudaMemcpyAsync(out->mask + f0, o.mask, (size_t)n * 4, cudaMemcpyDeviceToHost, s.stream));
+      if (out->err) TRI_CUDA(cudaMemcpyAsync(out->err + f0, o.err, (size_t)n * 8, cudaMemcpyDeviceToHost, s.stream));
+      if (out->iters) TRI_CUDA(cudaMemcpyAsync(out->iters + f0, o.iters, (size_t)n * 4, cudaMemcpyDeviceToHost, s.stream));
+    }
+    for (int i = 0; i < n_slots; i++) TRI_CUDA(cudaStreamSynchronize(e->slots[i].stream));
+    return TRI_OK;
+  };
+  if ((st = run()) != TRI_OK) {
+    const std::string why = g_error;
+    for (int i = 0; i < n_slots; i++) cudaStreamSynchronize(e->slots[i].stream);  // nothing is left in flight into the caller's memory
+    cudaMemset(latch, 0xff, sizeof(unsigned long long));
+    cudaGetLastError();
+    return fail(st, why);
+  }
+  unsigned long long v = 0;
+  TRI_CUDA(cudaMemcpy(&v, latch, sizeof(v), cudaMemcpyDeviceToHost));
+  if (v != ~0ull) {
+    TRI_CUDA(cudaMemset(latch, 0xff, sizeof(v)));
+    if (first_bad_frame) *first_bad_frame = (int64_t)v;
+    if (!(flags & TRI_ALLOW_TOO_FEW)) return fail(TRI_ERR_TOO_FEW, too_few_msg);
+  }
+  return TRI_OK;
+}
+
 }  // namespace tri
 
 using namespace tri;
@@ -361,15 +453,7 @@ int tri_triangulate_points_device(tri_engine* e, int mode, unsigned flags, const
   if (n_frames == 0) return TRI_OK;
   DeviceGuard g(e->device);
   BatchOut out{d_out->xyz_f32, d_out->xyz_f64, d_out->mask, d_out->err, d_out->iters};
-  if (n_use == 0 && n_frames > 0) {  // no rows at all: every frame has too few views
-    TRI_CUDA(cudaMemsetAsync(e->d_first_bad, 0, sizeof(unsigned long long), (cudaStream_t)stream));
-    if (out.xyz_f32) TRI_CUDA(cudaMemsetAsync(out.xyz_f32, 0, sizeof(float) * 3 * n_frames, (cudaStream_t)stream));
-    if (out.xyz_f64) TRI_CUDA(cudaMemsetAsync(out.xyz_f64, 0, sizeof(double) * 3 * n_frames, (cudaStream_t)stream));
-    if (out.mask) TRI_CUDA(cudaMemsetAsync(out.mask, 0, sizeof(uint32_t) * n_frames, (cudaStream_t)stream));
-    if (out.err) TRI_CUDA(cudaMemsetAsync(out.err, 0, sizeof(double) * n_frames, (cudaStream_t)stream));
-    if (out.iters) TRI_CUDA(cudaMemsetAsync(out.iters, 0, sizeof(int32_t) * n_frames, (cudaStream_t)stream));
-    return TRI_OK;
-  }
+  if (n_use == 0) return too_few_device(e, n_frames, out, (cudaStream_t)stream);
   return launch_batch(e, e->ctx((cudaStream_t)stream), mode, flags, fmt, d_xy, n_use, n_frames, cam_stride, out);
 }
 
@@ -434,8 +518,6 @@ int tri_device_status(tri_engine* e, void* stream, int64_t* first_bad_frame) {
   return TRI_OK;
 }
 
-// Host-buffer batch: frames stream through N_SLOTS device staging slots, one CUDA stream each, so the
-// H2D copy of a chunk overlaps the kernel of the previous one and the D2H copy of the one before.
 int tri_triangulate_points(tri_engine* e, int mode, unsigned flags, const void* xy, int n_point_cams, int64_t n_frames,
                            int64_t cam_stride, const tri_batch_out* out, int64_t* first_bad_frame) {
   int n_use = 0, fmt = 0;
@@ -445,75 +527,51 @@ int tri_triangulate_points(tri_engine* e, int mode, unsigned flags, const void* 
   if (first_bad_frame) *first_bad_frame = -1;
   if (n_frames == 0) return TRI_OK;
   DeviceGuard g(e->device);
-  const size_t pb = pix_bytes(fmt);
   // chunk: large enough to run the copy engines at full rate, small enough to pipeline
   int64_t chunk = n_frames >= (16 << 20) ? (4 << 20) : (1 << 20);  // measured: 4 Mi-frame chunks run PCIe at 63 GB/s, 1 Mi at 60.6
   if (mode == TRI_RAY && (flags & TRI_RAY_REFERENCE_LM)) chunk = 1 << 18;
 #ifdef TRI_TUNING
   if (const char* v = getenv("TRI_CHUNK_FRAMES")) chunk = std::max<int64_t>(2, atoll(v) / 2 * 2);
 #endif
-  if (n_frames <= chunk) chunk = (n_frames + 1) / 2 * 2;  // one chunk
-  const size_t in_row = align_up((size_t)chunk * pb, 256);
-  const size_t o_xyz32 = 0;
-  const size_t o_xyz64 = o_xyz32 + (out->xyz_f32 ? align_up((size_t)chunk * 12, 256) : 0);
-  const size_t o_mask = o_xyz64 + (out->xyz_f64 ? align_up((size_t)chunk * 24, 256) : 0);
-  const size_t o_err = o_mask + (out->mask ? align_up((size_t)chunk * 4, 256) : 0);
-  const size_t o_iters = o_err + (out->err ? align_up((size_t)chunk * 8, 256) : 0);
-  const size_t out_bytes = o_iters + (out->iters ? align_up((size_t)chunk * 4, 256) : 0);
-  const int n_slots = n_frames > chunk ? N_SLOTS : 1;
-  for (int i = 0; i < n_slots; i++) {
-    if ((st = ensure(&e->slots[i].d_in, &e->slots[i].in_cap, in_row * std::max(n_use, 1))) != TRI_OK) return st;
-    if ((st = ensure(&e->slots[i].d_out, &e->slots[i].out_cap, out_bytes)) != TRI_OK) return st;
-  }
-  unsigned long long* latch = e->d_first_bad + 1;  // the host path's own latch: a pending one of the device entry point stays
-  TRI_CUDA(cudaMemsetAsync(latch, 0xff, sizeof(unsigned long long), e->slots[0].stream));
-  TRI_CUDA(cudaStreamSynchronize(e->slots[0].stream));
-  const char* src = static_cast<const char*>(xy);
-  // the chunk loop; on any failure the copies already queued into the caller's buffers are drained before returning
-  auto run = [&]() -> int {
-    int k = 0;
-    for (int64_t f0 = 0; f0 < n_frames; f0 += chunk, k++) {
-      Slot& s = e->slots[k % n_slots];
-      const int64_t n = std::min(chunk, n_frames - f0);
-      TRI_CUDA(cudaStreamSynchronize(s.stream));  // slot free (its previous D2H has landed)
-      for (int c = 0; c < n_use; c++)
-        TRI_CUDA(cudaMemcpyAsync(s.d_in + (size_t)c * in_row, src + ((size_t)c * cam_stride + f0) * pb, (size_t)n * pb,
-                                 cudaMemcpyHostToDevice, s.stream));
-      BatchOut o{out->xyz_f32 ? (float*)(s.d_out + o_xyz32) : nullptr, out->xyz_f64 ? (double*)(s.d_out + o_xyz64) : nullptr,
-                 out->mask ? (uint32_t*)(s.d_out + o_mask) : nullptr, out->err ? (double*)(s.d_out + o_err) : nullptr,
-                 out->iters ? (int32_t*)(s.d_out + o_iters) : nullptr};
-      if (n_use == 0) {
-        TRI_CUDA(cudaMemsetAsync(s.d_out, 0, out_bytes, s.stream));
-        TRI_CUDA(cudaMemsetAsync(latch, 0, sizeof(unsigned long long), s.stream));
-      } else {
-        const int st2 = launch_batch(e, e->ctx(s.stream, f0, true), mode, flags, fmt, s.d_in, n_use, n, (int64_t)(in_row / pb), o);
-        if (st2 != TRI_OK) return st2;
-      }
-      if (out->xyz_f32) TRI_CUDA(cudaMemcpyAsync(out->xyz_f32 + 3 * f0, o.xyz_f32, (size_t)n * 12, cudaMemcpyDeviceToHost, s.stream));
-      if (out->xyz_f64) TRI_CUDA(cudaMemcpyAsync(out->xyz_f64 + 3 * f0, o.xyz_f64, (size_t)n * 24, cudaMemcpyDeviceToHost, s.stream));
-      if (out->mask) TRI_CUDA(cudaMemcpyAsync(out->mask + f0, o.mask, (size_t)n * 4, cudaMemcpyDeviceToHost, s.stream));
-      if (out->err) TRI_CUDA(cudaMemcpyAsync(out->err + f0, o.err, (size_t)n * 8, cudaMemcpyDeviceToHost, s.stream));
-      if (out->iters) TRI_CUDA(cudaMemcpyAsync(out->iters + f0, o.iters, (size_t)n * 4, cudaMemcpyDeviceToHost, s.stream));
-    }
-    for (int i = 0; i < n_slots; i++) TRI_CUDA(cudaStreamSynchronize(e->slots[i].stream));
-    return TRI_OK;
-  };
-  if ((st = run()) != TRI_OK) {
-    const std::string why = g_error;
-    for (int i = 0; i < n_slots; i++) cudaStreamSynchronize(e->slots[i].stream);  // nothing is left in flight into the caller's memory
-    cudaMemset(latch, 0xff, sizeof(unsigned long long));
-    cudaGetLastError();
-    return fail(st, why);
-  }
-  unsigned long long v = 0;
-  TRI_CUDA(cudaMemcpy(&v, latch, sizeof(v), cudaMemcpyDeviceToHost));
-  if (v != ~0ull) {
-    TRI_CUDA(cudaMemset(latch, 0xff, sizeof(v)));
-    if (first_bad_frame) *first_bad_frame = (int64_t)v;
-    if (!(flags & TRI_ALLOW_TOO_FEW))
-      return fail(TRI_ERR_TOO_FEW, mode == TRI_MATRIX ? "Too few rays are found" : "Too few detections are found");
-  }
-  return TRI_OK;
+  return run_host_pipeline(e, flags, fmt, xy, n_use, n_frames, cam_stride, chunk, out, first_bad_frame,
+                           mode == TRI_MATRIX ? "Too few rays are found" : "Too few detections are found",
+                           [&](const LaunchCtx& ctx, const void* d_in, int64_t n, int64_t stride, const BatchOut& o) {
+                             return launch_batch(e, ctx, mode, flags, fmt, d_in, n_use, n, stride, o);
+                           });
+}
+
+int tri_triangulate_points_robust_device(tri_engine* e, unsigned flags, double max_reproj_px, const void* d_xy, int n_point_cams,
+                                         int64_t n_frames, int64_t cam_stride, const tri_batch_out* d_out, void* stream) {
+  int n_use = 0, fmt = 0;
+  int st = check_robust_args(e, flags, max_reproj_px, d_xy, n_point_cams, n_frames, cam_stride, d_out, &n_use);
+  if (st != TRI_OK) return st;
+  if ((st = pix_format(flags, &fmt)) != TRI_OK) return st;
+  if (n_frames == 0) return TRI_OK;
+  DeviceGuard g(e->device);
+  BatchOut out{d_out->xyz_f32, d_out->xyz_f64, d_out->mask, d_out->err, nullptr};
+  if (n_use == 0) return too_few_device(e, n_frames, out, (cudaStream_t)stream);
+  const cudaError_t err = launch_robust(e->ctx((cudaStream_t)stream), (flags & TRI_F32) != 0, fmt, e->rig64, e->rig32, max_reproj_px,
+                                        d_xy, n_use, n_frames, cam_stride, out);
+  return err == cudaSuccess ? TRI_OK : cuda_fail(err, "kernel launch");
+}
+
+int tri_triangulate_points_robust(tri_engine* e, unsigned flags, double max_reproj_px, const void* xy, int n_point_cams,
+                                  int64_t n_frames, int64_t cam_stride, const tri_batch_out* out, int64_t* first_bad_frame) {
+  int n_use = 0, fmt = 0;
+  int st = check_robust_args(e, flags, max_reproj_px, xy, n_point_cams, n_frames, cam_stride, out, &n_use);
+  if (st != TRI_OK) return st;
+  if ((st = pix_format(flags, &fmt)) != TRI_OK) return st;
+  if (first_bad_frame) *first_bad_frame = -1;
+  if (n_frames == 0) return TRI_OK;
+  DeviceGuard g(e->device);
+  // the solve is compute-bound (pairs x views per frame), so the copies hide under it at the plain path's 1 Mi-frame chunk
+  return run_host_pipeline(e, flags, fmt, xy, n_use, n_frames, cam_stride, (int64_t)1 << 20, out, first_bad_frame,
+                           "Too few rays are found",
+                           [&](const LaunchCtx& ctx, const void* d_in, int64_t n, int64_t stride, const BatchOut& o) {
+                             const cudaError_t err = launch_robust(ctx, (flags & TRI_F32) != 0, fmt, e->rig64, e->rig32, max_reproj_px,
+                                                                   d_in, n_use, n, stride, o);
+                             return err == cudaSuccess ? TRI_OK : cuda_fail(err, "kernel launch");
+                           });
 }
 
 int tri_triangulate_points_multi(tri_engine* const* engines, int n_engines, int mode, unsigned flags, const void* xy,

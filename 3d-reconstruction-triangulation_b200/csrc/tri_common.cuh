@@ -157,4 +157,9 @@ cudaError_t launch_dlt(const LaunchCtx& ctx, bool f32, int pixfmt, const DltRig<
                        const DltRig<float>& rig32, const void* d_xy, int n_use, int64_t n_frames,
                        int64_t cam_stride, const BatchOut& out);
 
+// two-view consensus + inlier refit (tri_robust.cu); out.mask = the inlier set, out.err = RMS reprojection error in pixels
+cudaError_t launch_robust(const LaunchCtx& ctx, bool f32, int pixfmt, const DltRig<double>& rig64, const DltRig<float>& rig32,
+                          double max_reproj_px, const void* d_xy, int n_use, int64_t n_frames, int64_t cam_stride,
+                          const BatchOut& out);
+
 }  // namespace tri

@@ -15,6 +15,8 @@
 //     barrier instead of drifting apart.  So the product library ships stream_kernel only.
 // Algorithmic traffic: 8 B x cameras in, 12 B out per frame; nothing is re-read (profiles/: 7.59 GB per 100 M frames).
 #pragma once
+#include <type_traits>
+
 #include "tri_batch.cuh"
 
 namespace tri {
@@ -163,6 +165,13 @@ struct PolicyTile {
   }
 };
 
+// A tile's mask output is its frames' validity bits -- the too-few latch counts them -- unless the tile declares
+// MASK_IS_VALIDITY = false (the robust tile: mask = the inlier set, `iters` carries the number of valid views).
+template <class TS, class = void>
+struct MaskIsValidity { static constexpr bool value = true; };
+template <class TS>
+struct MaskIsValidity<TS, std::void_t<decltype(TS::MASK_IS_VALIDITY)>> { static constexpr bool value = TS::MASK_IS_VALIDITY; };
+
 // ---- barrier-free per-thread async pipeline ---------------------------------------------------------
 // Nothing synchronises across warps: every thread prefetches ITS OWN pixels of the next STAGES tiles with
 // cp.async (LDGSTS, 16 B per camera row, fully coalesced per warp) into a private shared-memory slot, waits only
@@ -272,7 +281,7 @@ stream_kernel(const __grid_constant__ typename TS::Rig rig, const char* __restri
     const int64_t f0 = tile * TILE + (int64_t)tid * FPT;
 #pragma unroll
     for (int j = 0; j < FPT; j++)
-      if (__popc(mask[j]) < 2) atomicMin(first_bad, (unsigned long long)(frame_base + f0 + j));
+      if ((MaskIsValidity<TS>::value ? __popc(mask[j]) : iters[j]) < 2) atomicMin(first_bad, (unsigned long long)(frame_base + f0 + j));
     if (out.mask) {
       if constexpr (FPT == 2) reinterpret_cast<uint2*>(out.mask)[f0 / 2] = make_uint2(mask[0], mask[1]);
       else out.mask[f0] = mask[0];

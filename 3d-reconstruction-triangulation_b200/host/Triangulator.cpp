@@ -86,6 +86,64 @@ unsigned Triangulator::pixelFormatFor(const std::vector<std::vector<cv::Point2d>
   return exact16 ? (unsigned)TRI_PIX_U16 : exact32 ? 0u : (unsigned)TRI_PIX_F64;
 }
 
+namespace {
+// points[cam][frame] packed in the narrowest exact pixel format, then handed to `call(flags, xy)`
+template <class Call>
+int withPackedPixels(const std::vector<std::vector<cv::Point2d>>& points, int64_t n_frames, Call call) {
+  const int n_rows = (int)points.size();
+  const unsigned fmt = Triangulator::pixelFormatFor(points);
+  if (fmt == TRI_PIX_U16) {
+    std::vector<uint16_t> xy(2 * (size_t)n_rows * n_frames);
+    for (int c = 0; c < n_rows; c++)
+      for (int64_t f = 0; f < n_frames; f++) {
+        const cv::Point2d& p = points[c][f];
+        const bool missing = p.x == -1 || p.y == -1;
+        xy[2 * ((size_t)c * n_frames + f)] = missing ? (uint16_t)0xFFFF : (uint16_t)p.x;
+        xy[2 * ((size_t)c * n_frames + f) + 1] = missing ? (uint16_t)0xFFFF : (uint16_t)p.y;
+      }
+    return call(fmt, (const void*)xy.data());
+  }
+  if (fmt == 0) {
+    std::vector<float> xy(2 * (size_t)n_rows * n_frames);
+    for (int c = 0; c < n_rows; c++)
+      for (int64_t f = 0; f < n_frames; f++) {
+        xy[2 * ((size_t)c * n_frames + f)] = (float)points[c][f].x;
+        xy[2 * ((size_t)c * n_frames + f) + 1] = (float)points[c][f].y;
+      }
+    return call(fmt, (const void*)xy.data());
+  }
+  std::vector<double> xy(2 * (size_t)n_rows * n_frames);
+  for (int c = 0; c < n_rows; c++)
+    for (int64_t f = 0; f < n_frames; f++) {
+      xy[2 * ((size_t)c * n_frames + f)] = points[c][f].x;
+      xy[2 * ((size_t)c * n_frames + f) + 1] = points[c][f].y;
+    }
+  return call(fmt, (const void*)xy.data());
+}
+}  // namespace
+
+std::vector<cv::Point3d> MatrixTriangulator::triangulatePointsRobust(const std::vector<std::vector<cv::Point2d>>& points,
+                                                                     double maxReprojPx, std::vector<uint32_t>* inliers,
+                                                                     std::vector<double>* reprojRms) {
+  for (size_t i = 1; i < points.size(); i++)
+    if (points[i - 1].size() != points[i].size()) throw std::runtime_error("Every camera should have the same number of points");
+  const int64_t n_frames = points.empty() ? 0 : (int64_t)points[0].size();
+  std::vector<double> xyz(3 * (size_t)n_frames);
+  tri_batch_out out{};
+  out.xyz_f64 = xyz.data();
+  if (inliers) { inliers->assign((size_t)n_frames, 0); out.mask = inliers->data(); }
+  if (reprojRms) { reprojRms->assign((size_t)n_frames, 0.0); out.err = reprojRms->data(); }
+  int64_t bad = -1;
+  const int st = withPackedPixels(points, n_frames, [&](unsigned fmt, const void* xy) {
+    return tri_triangulate_points_robust(engine_, (flags_ & TRI_F32) | fmt, maxReprojPx, xy, (int)points.size(), n_frames, n_frames,
+                                         &out, &bad);
+  });
+  if (st != TRI_OK) raise(st, TRI_MATRIX);
+  std::vector<cv::Point3d> result((size_t)n_frames);
+  for (int64_t f = 0; f < n_frames; f++) result[f] = cv::Point3d(xyz[3 * f], xyz[3 * f + 1], xyz[3 * f + 2]);
+  return result;
+}
+
 std::vector<cv::Point3d> Triangulator::triangulatePoints(std::vector<std::vector<cv::Point2d>> points) {
   // MatrixTriangulator.cpp:72-76 / RayTriangulator.cpp:54-58
   for (size_t i = 1; i < points.size(); i++)

@@ -3,6 +3,7 @@
 // reference, so src/main.cpp:54-65 and src/DroneClassifier.cpp compile against it unchanged apart from
 // the include; all arithmetic happens on the GPU through include/tri_b200.h (no CPU path).
 #pragma once
+#include <cstdint>
 #include <string>
 #include <utility>
 #include <vector>
@@ -61,6 +62,14 @@ class Triangulator {
 class MatrixTriangulator : public Triangulator {  // src/MatrixTriangulator.h:19, type "matrix"
  public:
   explicit MatrixTriangulator(std::vector<const tdr::Camera*> cameras, int device = 0);
+
+  // Extension (the reference has no such method): triangulatePoints that ignores wrong detections.  Same input, packing
+  // and runtime_error texts as triangulatePoints; per frame, the two-view hypothesis with the most views within
+  // maxReprojPx pixels wins and the point is the DLT over those inlier views (tri_triangulate_points_robust).  A frame
+  // where no two views agree gives (0,0,0).  inliers[f]: bit c = camera c used; reprojRms[f]: RMS reprojection error in
+  // pixels over the inliers (NaN without consensus).
+  std::vector<cv::Point3d> triangulatePointsRobust(const std::vector<std::vector<cv::Point2d>>& points, double maxReprojPx,
+                                                   std::vector<uint32_t>* inliers = nullptr, std::vector<double>* reprojRms = nullptr);
 };
 
 class RayTriangulator : public Triangulator {  // src/RayTriangulator.h:34, type "ray"

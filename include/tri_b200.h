@@ -116,6 +116,27 @@ int tri_triangulate_points(tri_engine* e, int mode, unsigned flags, const void* 
                            int64_t n_frames, int64_t cam_stride, const tri_batch_out* out,
                            int64_t* first_bad_frame);
 
+/* Outlier-robust matrix-mode batch (an extension: the reference has no such call).  Same pixel layout, camera rows
+ * (min(n_point_cams, n_cams)), missing-view test and too-few handling as tri_triangulate_points in TRI_MATRIX mode.
+ * Per frame with valid views V (|V| >= 2): every pair i < j of V gives the two-view DLT X_ij, usable if its projective
+ * depth w_c = P_c[8..10].X + P_c[11] is > 0 on both cameras; its inliers are the views c of V with w_c(X_ij) > 0 and
+ * pixel reprojection error r_c <= max_reproj_px; the winner has the most inliers (>= 2), then the smallest sum of r_c^2
+ * over them, then the first pair in (i, j) order; the result is the DLT over the winner's inlier set I.  One consensus
+ * round, one refit, FP64 (FP32 under TRI_F32).  The fields of tri_batch_out mean, for these two calls:
+ *   xyz_f32 / xyz_f64  the refitted point; (0,0,0) when no hypothesis has 2 inliers (not an error)
+ *   mask               the inlier set I (0 when there is no consensus; the < 2 valid bits on a too-few frame)
+ *   err                RMS pixel reprojection error of the point over I, sqrt(mean r_c^2); NaN without consensus,
+ *                      0 on a too-few frame
+ *   iters              must be NULL
+ * Flags: TRI_F32, TRI_PIX_F64, TRI_PIX_U16, TRI_ALLOW_TOO_FEW; anything else, max_reproj_px <= 0 or NaN, or a
+ * non-NULL iters returns TRI_ERR_ARG.  HOST buffers, streamed in chunks like tri_triangulate_points. */
+int tri_triangulate_points_robust(tri_engine* e, unsigned flags, double max_reproj_px, const void* xy, int n_point_cams,
+                                  int64_t n_frames, int64_t cam_stride, const tri_batch_out* out, int64_t* first_bad_frame);
+/* The same with DEVICE buffers, asynchronous on `stream`; too-few frames are latched for tri_device_status. */
+int tri_triangulate_points_robust_device(tri_engine* e, unsigned flags, double max_reproj_px, const void* d_xy,
+                                         int n_point_cams, int64_t n_frames, int64_t cam_stride,
+                                         const tri_batch_out* d_out, void* stream);
+
 /* The same batch sharded over several engines (one per GPU of the box) from ONE host process: frames
  * are independent, so engine g takes the contiguous range [g*N/G, (g+1)*N/G) and the shards run
  * concurrently (one host thread and one copy/compute pipeline per GPU); results land in the caller's
