@@ -20,7 +20,7 @@ from dataclasses import dataclass, field
 import numpy as np
 
 HERE = os.path.dirname(os.path.abspath(__file__))
-LIB_PATH = os.environ.get("TRI_B200_LIB") or os.path.join(HERE, "libtri_b200.so")  # override: tuning experiments only
+LIB_PATH = os.path.join(HERE, "libtri_b200.so")
 
 MATRIX, RAY = 0, 1
 OK, ERR_DIM, ERR_TOO_FEW, ERR_ARG, ERR_CUDA, ERR_NO_DEVICE, ERR_CAPACITY = range(7)
@@ -32,7 +32,6 @@ PIX_F64 = 1 << 4
 PIX_U16 = 1 << 5
 RAY_ANALYTIC_LM = 1 << 6
 CLS_LAZY = 1 << 7
-DEBUG_STREAM = 1 << 30
 MAX_CAMS = 32
 
 # the runtime_error texts of the reference, re-raised by the adapters

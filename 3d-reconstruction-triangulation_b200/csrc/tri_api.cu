@@ -135,7 +135,6 @@ static cudaError_t upload_ray_table(RayFold<T>& f, int n_cams) {
 // DltRig<T>::absent (host copy): per group of 8 cameras and per 8-bit set m, what the cameras of m add to the normal
 // equations at the canonical pixel (x = y = 0 relative to the rig's pixel origin: rows P[r,0:3], rhs -P[r,3]), accumulated
 // in camera order with the kernels' own fma sequence (acc_row, tri_matrix.cu).
-static inline double fma_h(double a, double b, double c) { return fma(a, b, c); }
 static inline float fma_h(float a, float b, float c) { return fmaf(a, b, c); }
 template <typename T>
 static std::vector<T> dlt_absent_table(const DltRig<T>& r, int n_cams) {
@@ -219,7 +218,7 @@ static int pix_format(unsigned flags, int* fmt) {
   return TRI_OK;
 }
 
-static int check_batch_args(tri_engine* e, int mode, unsigned flags, const void* xy, int n_point_cams, int64_t n_frames,
+static int check_batch_args(tri_engine* e, int mode, const void* xy, int n_point_cams, int64_t n_frames,
                             int64_t cam_stride, const tri_batch_out* out, int* n_use) {
   if (!e) return fail(TRI_ERR_ARG, "null engine");
   if (mode != TRI_MATRIX && mode != TRI_RAY) return fail(TRI_ERR_ARG, "mode must be TRI_MATRIX or TRI_RAY");
@@ -234,18 +233,12 @@ static int check_batch_args(tri_engine* e, int mode, unsigned flags, const void*
       return fail(TRI_ERR_DIM, "ray mode: more pixel rows than cameras");
     *n_use = n_point_cams;
   }
-#ifndef TRI_TUNING
-  if (flags & TRI_DEBUG_STREAM) return fail(TRI_ERR_ARG, "TRI_DEBUG_STREAM is a measurement aid of the tuning build (make -C csrc tuning)");
-#endif
   return TRI_OK;
 }
 
-static int launch_batch(tri_engine* e, LaunchCtx ctx, int mode, unsigned flags, int fmt, const void* d_xy, int n_use,
+static int launch_batch(tri_engine* e, const LaunchCtx& ctx, int mode, unsigned flags, int fmt, const void* d_xy, int n_use,
                         int64_t n_frames, int64_t cam_stride, const BatchOut& out) {
   cudaError_t err;
-#ifdef TRI_TUNING
-  ctx.debug_stream = (flags & TRI_DEBUG_STREAM) != 0;
-#endif
   if (mode == TRI_MATRIX) {
     err = launch_dlt(ctx, (flags & TRI_F32) != 0, fmt, e->rig64, e->rig32, d_xy, n_use, n_frames, cam_stride, out);
   } else {
@@ -289,7 +282,7 @@ static int check_robust_args(tri_engine* e, unsigned flags, double max_reproj_px
   if (flags & ~allowed) return fail(TRI_ERR_ARG, "robust triangulation accepts TRI_F32, TRI_PIX_F64, TRI_PIX_U16 and TRI_ALLOW_TOO_FEW only");
   if (!(max_reproj_px > 0)) return fail(TRI_ERR_ARG, "max_reproj_px must be > 0");
   if (out && out->iters) return fail(TRI_ERR_ARG, "robust triangulation has no iteration output (iters must be NULL)");
-  return check_batch_args(e, TRI_MATRIX, flags, xy, n_point_cams, n_frames, cam_stride, out, n_use);
+  return check_batch_args(e, TRI_MATRIX, xy, n_point_cams, n_frames, cam_stride, out, n_use);
 }
 
 // Host-buffer batch: frames stream through N_SLOTS device staging slots, one CUDA stream each, so the
@@ -398,14 +391,10 @@ int tri_create(int n_cams, const tri_camera* cams, int device, tri_engine** out)
   e->device = device;
   e->n_cams = n_cams;
   e->sm_count = prop.multiProcessorCount;
-#ifdef TRI_TUNING
-  if (const char* v = getenv("TRI_VARIANT")) e->variant = atoi(v);
-#endif
   memcpy(e->cams, cams, sizeof(tri_camera) * n_cams);
   build_rigs(e);
   cudaError_t err = cudaMalloc((void**)&e->d_first_bad, 2 * sizeof(unsigned long long));
   if (err == cudaSuccess) err = cudaMemset(e->d_first_bad, 0xff, 2 * sizeof(unsigned long long));
-  if (err == cudaSuccess) err = upload_dlt_table(e->rig64, n_cams);
   if (err == cudaSuccess) err = upload_dlt_table(e->rig32, n_cams);
   if (err == cudaSuccess) err = upload_ray_table(e->fold64, n_cams);
   if (err == cudaSuccess) err = upload_ray_table(e->fold32, n_cams);
@@ -433,7 +422,6 @@ void tri_destroy(tri_engine* e) {
   if (e->d_scratch) cudaFree(e->d_scratch);
   if (e->stream) cudaStreamDestroy(e->stream);
   if (e->d_first_bad) cudaFree(e->d_first_bad);
-  if (e->rig64.absent) cudaFree(const_cast<double*>(e->rig64.absent));
   if (e->rig32.absent) cudaFree(const_cast<float*>(e->rig32.absent));
   if (e->fold64.mask_table) cudaFree(const_cast<double*>(e->fold64.mask_table));
   if (e->fold32.mask_table) cudaFree(const_cast<float*>(e->fold32.mask_table));
@@ -447,7 +435,7 @@ int64_t tri_kernel_launches(const tri_engine* e) { return e ? e->launches : 0; }
 int tri_triangulate_points_device(tri_engine* e, int mode, unsigned flags, const void* d_xy, int n_point_cams,
                                   int64_t n_frames, int64_t cam_stride, const tri_batch_out* d_out, void* stream) {
   int n_use = 0, fmt = 0;
-  int st = check_batch_args(e, mode, flags, d_xy, n_point_cams, n_frames, cam_stride, d_out, &n_use);
+  int st = check_batch_args(e, mode, d_xy, n_point_cams, n_frames, cam_stride, d_out, &n_use);
   if (st != TRI_OK) return st;
   if ((st = pix_format(flags, &fmt)) != TRI_OK) return st;
   if (n_frames == 0) return TRI_OK;
@@ -521,7 +509,7 @@ int tri_device_status(tri_engine* e, void* stream, int64_t* first_bad_frame) {
 int tri_triangulate_points(tri_engine* e, int mode, unsigned flags, const void* xy, int n_point_cams, int64_t n_frames,
                            int64_t cam_stride, const tri_batch_out* out, int64_t* first_bad_frame) {
   int n_use = 0, fmt = 0;
-  int st = check_batch_args(e, mode, flags, xy, n_point_cams, n_frames, cam_stride, out, &n_use);
+  int st = check_batch_args(e, mode, xy, n_point_cams, n_frames, cam_stride, out, &n_use);
   if (st != TRI_OK) return st;
   if ((st = pix_format(flags, &fmt)) != TRI_OK) return st;
   if (first_bad_frame) *first_bad_frame = -1;
@@ -530,9 +518,6 @@ int tri_triangulate_points(tri_engine* e, int mode, unsigned flags, const void* 
   // chunk: large enough to run the copy engines at full rate, small enough to pipeline
   int64_t chunk = n_frames >= (16 << 20) ? (4 << 20) : (1 << 20);  // measured: 4 Mi-frame chunks run PCIe at 63 GB/s, 1 Mi at 60.6
   if (mode == TRI_RAY && (flags & TRI_RAY_REFERENCE_LM)) chunk = 1 << 18;
-#ifdef TRI_TUNING
-  if (const char* v = getenv("TRI_CHUNK_FRAMES")) chunk = std::max<int64_t>(2, atoll(v) / 2 * 2);
-#endif
   return run_host_pipeline(e, flags, fmt, xy, n_use, n_frames, cam_stride, chunk, out, first_bad_frame,
                            mode == TRI_MATRIX ? "Too few rays are found" : "Too few detections are found",
                            [&](const LaunchCtx& ctx, const void* d_in, int64_t n, int64_t stride, const BatchOut& o) {
@@ -582,7 +567,7 @@ int tri_triangulate_points_multi(tri_engine* const* engines, int n_engines, int 
     if (!engines[g] || engines[g]->n_cams != engines[0]->n_cams) return fail(TRI_ERR_ARG, "engines must hold the same rig");
   if (n_engines == 1) return tri_triangulate_points(engines[0], mode, flags, xy, n_point_cams, n_frames, cam_stride, out, first_bad_frame);
   int fmt = 0, n_use = 0;
-  int st = check_batch_args(engines[0], mode, flags, xy, n_point_cams, n_frames, cam_stride, out, &n_use);
+  int st = check_batch_args(engines[0], mode, xy, n_point_cams, n_frames, cam_stride, out, &n_use);
   if (st != TRI_OK) return st;
   if ((st = pix_format(flags, &fmt)) != TRI_OK) return st;
   const size_t pb = pix_bytes(fmt);

@@ -10,7 +10,7 @@
 //     S::T, S::Rig (a __grid_constant__ parameter: operands come from the constant bank), S::Acc,
 //     S::add(rig, c, x, y, valid, acc)     one view into the accumulator (a no-op when !valid)
 //     S::solve(rig, acc, mask, n, X, opt, iters) the per-frame solve, X in rig coordinates (mask = validity bits:
-//                                          the FP64 DLT takes its absent-view correction from a table row)
+//                                          the FP32 DLT takes its absent-view correction from a table row)
 //     S::residual(rig, c, x, y, X)         that view's contribution to the reported error
 //     S::error(sum, n)                     the reported error from the summed contributions
 //     S::to_world(rig, X)

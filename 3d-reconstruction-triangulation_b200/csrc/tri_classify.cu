@@ -393,10 +393,6 @@ link_kernel(const __grid_constant__ RayRig ray, ClsParams p, const int2* __restr
   }
   u64 n_phase1 = 0, n_phase2 = 0;  // lane 0 of the serial warp
   bool overflow_final = false;
-#ifdef TRI_TUNING
-  u64 prof_acc[12] = {0, 0, 0, 0, 0, 0, 0, 0, 0, 0, 0, 0};
-  long long prof_t = clock64();
-#endif
 
   // ---- the stager: lane 0 of the last warp.  Frame table two frames ahead in registers, the staged copy one frame ahead ----
   const bool stager = tid == LINK_THREADS - 32;
@@ -572,7 +568,6 @@ link_kernel(const __grid_constant__ RayRig ray, ClsParams p, const int2* __restr
           for (int t = 0; t < 2 * W; t++) v = lane == t ? slice[t] : v;
           s_gate[np][lane] = v;
         }
-        CLS_PROF(2);
         if (cams_in_gate >= MIN_CAMERAS) {  // else fillCombinationQueue on the gated container yields nothing
           // leaves with fewer unused cameras than the gate leaves empty cannot lie inside it
           const int pick = scan(zs[C - cams_in_gate], seg, nseg, g, none, last[0], last[1], last[2], nseg > 1 ? &spec[np] : nullptr);
@@ -580,9 +575,7 @@ link_kernel(const __grid_constant__ RayRig ray, ClsParams p, const int2* __restr
         }
       }
     }
-    CLS_PROF(3);
     __syncthreads();  // barrier 2: the speculative picks are in
-    CLS_PROF(4);
 
     // ---- confirm the picks (:119-135), lane <-> path, every warp for itself ----
     u64 used[W];
@@ -644,12 +637,10 @@ link_kernel(const __grid_constant__ RayRig ray, ClsParams p, const int2* __restr
         cand = (lane < D && ((processed >> lane) & 1u)) ? spec[lane] : LINK_NONE;
       }
     }
-    CLS_PROF(8);
     // phase 1's pushes, all confirmed paths at once (lane <-> path), on the last warp: warp 0 goes straight on to phase 2 and
     // classifyPaths, which only touch the paths phase 1 did not serve
     if (warp == LINK_WARPS - 1 && ((processed >> lane) & 1u)) emit(lane, cand, 1);
     if (tid == 32 * LINK_SERIAL_WARP) n_phase1 += __popc(processed);
-    CLS_PROF(5);
     if (__popc(processed) == D) return;  // :137
 
     // ---- phase 2: pickBestCombinations (:200-217), the reference's pop loop in parallel.  Every warp keeps the masks of
@@ -736,7 +727,6 @@ link_kernel(const __grid_constant__ RayRig ray, ClsParams p, const int2* __restr
       }
     }
     __syncwarp();
-    CLS_PROF(6);
 
     // ---- classifyPaths (:262-332), lane <-> kept combination (four rounds of 32 at most) ----
     const unsigned nonempty = __ballot_sync(FULL, lane < D && S.n[lane] != 0);  // S.n after phase 1's pushes
@@ -804,22 +794,18 @@ link_kernel(const __grid_constant__ RayRig ray, ClsParams p, const int2* __restr
       }
     }
     __syncwarp();
-    CLS_PROF(7);
   };
 
   for (int k = 0; k < nf; k++) {
     const int b = k & 1;
     __syncthreads();  // barrier 1: frame k - 1 is linked (state, its buffer free)
-    CLS_PROF(9);
     if (stager) {
       L_n1 = L_n2; off_n1 = off_n2; nd_n1 = nd_n2; doff_n1 = doff_n2;
       if (k + 1 < nf) stage(b ^ 1, fa + k + 1, L_n1, off_n1, nd_n1, doff_n1);
       meta(k + 2, L_n2, off_n2, nd_n2, doff_n2);
     }
     if (warp == 0 && lane < D) s_spec[b ^ 1][lane] = LINK_NONE;  // last read in frame k - 1, next written in frame k + 1
-    CLS_PROF(0);
     cls_mbar_wait(&full[b], (uint32_t)((k >> 1) & 1));
-    CLS_PROF(1);
     const int L = reinterpret_cast<const int*>(link_dyn + (size_t)b * L_::BUF_BYTES + L_::REC_BYTES + L_::DET_BYTES)[C + 1];
     if constexpr (ALL_STAGED) {
       frame(std::true_type{}, k, L);
@@ -830,9 +816,6 @@ link_kernel(const __grid_constant__ RayRig ray, ClsParams p, const int2* __restr
   }
   __syncthreads();
   for (int i = tid; i < (int)(sizeof(LinkState) / sizeof(int)); i += LINK_THREADS) ((int*)st)[i] = ((const int*)&S)[i];
-#ifdef TRI_TUNING
-  if (tid == 0) for (int q = 0; q < 12; q++) atomicAdd(&ctr->prof[q], prof_acc[q]);
-#endif
   if (tid == 32 * LINK_SERIAL_WARP) {
     atomicAdd(&ctr->phase1, n_phase1); atomicAdd(&ctr->phase2, n_phase2);
     if (overflow_final) atomicExch(&ctr->overflow_final, 1);
@@ -962,9 +945,6 @@ int cls_grid(const tri_engine* e, int frames) {
   int per_sm = 2;
   if (cudaFuncSetAttribute(enumerate_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, ENUM_SMEM_BYTES) != cudaSuccess ||
       cudaOccupancyMaxActiveBlocksPerMultiprocessor(&per_sm, enumerate_kernel, CLS_THREADS, ENUM_SMEM_BYTES) != cudaSuccess || per_sm < 1) per_sm = 2;
-#ifdef TRI_TUNING
-  if (const char* v = getenv("TRI_CLS_CTAS_PER_SM")) per_sm = std::max(1, atoi(v));
-#endif
   return std::max(1, std::min(frames, per_sm * e->sm_count));
 }
 
@@ -1168,12 +1148,6 @@ int cls_run(tri_engine* e, int mode, unsigned flags, int n_drones, const int32_t
   TRI_CUDA(cudaStreamSynchronize(s));
   if (hl.overflow_final) return fail(TRI_ERR_CAPACITY, "more than 128 disjoint combinations kept in one frame");
   h.phase1 = hl.phase1; h.phase2 = hl.phase2;
-#ifdef TRI_TUNING
-  for (int q = 0; q < 12; q++) h.prof[q] = hl.prof[q];
-  if (getenv("TRI_CLS_PROFILE"))
-    fprintf(stderr, "link cycles: barrier1 %llu | top %llu | wait %llu | gate %llu | scan %llu | barrier2 %llu | confirm %llu | emit %llu | phase2 %llu | classifyPaths %llu\n",
-            h.prof[9], h.prof[0], h.prof[1], h.prof[2], h.prof[3], h.prof[4], h.prof[8], h.prof[5], h.prof[6], h.prof[7]);
-#endif
   cls_stats(stats, h, max_frontier, W);
   return TRI_OK;
 }

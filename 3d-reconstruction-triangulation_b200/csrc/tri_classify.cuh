@@ -61,15 +61,7 @@ struct ClsParams {
 struct ClsCounters {
   u64 leaf_total, fdet_total, next_frame, nodes, solves, leaves, lm_iters, phase1, phase2, ties;
   int max_frontier, overflow_frontier, overflow_leaves, overflow_final, bad_input;
-  u64 prof[12];  // tuning builds: clock cycles of the linking pass by section (wait, gates, phase 1, phase 2, classifyPaths)
 };
-// tuning builds: thread 0 times its own sections with clock64.  (BAR.SYNC defers blocking -- the warp only waits at its next
-// shared-memory access -- so a section that follows a block barrier also holds the wait for it.)
-#ifdef TRI_TUNING
-#define CLS_PROF(k) do { const long long now__ = clock64(); prof_acc[k] += (u64)(now__ - prof_t); prof_t = now__; } while (0)
-#else
-#define CLS_PROF(k) do { } while (0)
-#endif
 
 struct LinkState {
   double tail[TRI_MAX_DRONES][PATH_TAIL][3];  // oldest .. newest of the last min(n,3) points

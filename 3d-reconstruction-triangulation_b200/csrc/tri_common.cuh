@@ -20,7 +20,8 @@ struct __align__(16) DltRig {
   T origin[3];              // world origin added back to the solution (0 for FP64)
   // device, [TRI_MAX_CAMS / 8][256][DLT_TABLE_ROW]: row (g, m) = what the cameras 8g + {bits of m} add to the normal
   // equations at the canonical pixel (the rig's pixel origin) -- absent views are accumulated there and this row is
-  // subtracted afterwards (tri_matrix.cu); built by the host with the kernels' own fma sequence
+  // subtracted afterwards (tri_matrix.cu); built by the host with the kernels' own fma sequence.  FP32 rig only (null in
+  // the FP64 rig, whose kernels clear an absent view's coefficients instead)
   const T* absent;
   int n_use;  // pixel rows of this launch (set per launch)
 };
@@ -139,10 +140,6 @@ struct LaunchCtx {
   unsigned long long* d_first_bad;  // latched index of the first frame with < 2 views
   int64_t frame_base;               // global index of frame 0 of this launch (chunked host path)
   int64_t* launches;
-#ifdef TRI_TUNING  // tuning builds only (make tuning): never compiled into libtri_b200.so
-  bool debug_stream = false;  // TRI_DEBUG_STREAM: memory-roofline probe instead of the solve
-  int variant = 0;            // TRI_VARIANT environment variable: kernel shape under A/B measurement
-#endif
 };
 
 enum RaySolver { RAY_ANALYTIC_LM = 0, RAY_REFERENCE_LM = 1, RAY_CLOSED_FORM = 2 };

@@ -49,9 +49,6 @@ struct tri_engine {
   unsigned long long* d_first_bad = nullptr;  // [0]: latch of the device entry point (collected by tri_device_status), [1]: of the host-buffer path
   tri::Slot slots[tri::N_SLOTS];
   int64_t launches = 0;
-#ifdef TRI_TUNING
-  int variant = 0;
-#endif
   // scratch for the small host-buffer entry points (subsets, dist_from_ray, classify)
   char* d_scratch = nullptr;
   size_t scratch_cap = 0;
@@ -60,10 +57,6 @@ struct tri_engine {
   void (*cls_work_free)(void*) = nullptr;
 
   tri::LaunchCtx ctx(cudaStream_t s, int64_t frame_base = 0, bool host_path = false) {
-    tri::LaunchCtx c{s, sm_count, d_first_bad + (host_path ? 1 : 0), frame_base, &launches};
-#ifdef TRI_TUNING
-    c.variant = variant;
-#endif
-    return c;
+    return tri::LaunchCtx{s, sm_count, d_first_bad + (host_path ? 1 : 0), frame_base, &launches};
   }
 };

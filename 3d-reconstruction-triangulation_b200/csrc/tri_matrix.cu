@@ -11,11 +11,12 @@
 // the normal-equation solution; cond(A) <= ~5 on real rigs so nothing is lost (SURVEY.md F1).
 // HBM traffic per frame: 8 B x n_cams in, 12 B out.
 //
-// Absent views (round 2): no select, predicate or branch sits in the FMA chain any more.  An absent view's
-// pixel is replaced by a canonical one (the pixel origin of the rig) BEFORE the conversion, every camera is
-// accumulated unconditionally, and what the absent cameras added -- a constant per camera at the canonical
-// pixel -- is taken back after the camera loop from a 256-row table indexed by the complement of the frame's
-// validity mask (one row per group of 8 cameras; built on the host with the same fma sequence, tri_api.cu).
+// Absent views (round 2, FP32; FP64: MASK_SELECT_HI below): no select, predicate or branch sits in the FMA
+// chain any more.  An absent view's pixel is replaced by a canonical one (the pixel origin of the rig) BEFORE
+// the conversion, every camera is accumulated unconditionally, and what the absent cameras added -- a constant
+// per camera at the canonical pixel -- is taken back after the camera loop from a 256-row table indexed by the
+// complement of the frame's validity mask (one row per group of 8 cameras; built on the host with the same fma
+// sequence, tri_api.cu).
 // Round 1 zeroed the three row coefficients with selects: 192 FSEL per pair of frames in the FP64 kernel, in the
 // dependency chain between the row FMAs and the accumulation FMAs (profiles/ncu_r1g.md: issue 66 %, FP64 pipe
 // 67 %, both short of their limits because each starved the other).
@@ -49,11 +50,6 @@ __device__ __forceinline__ const T* absent_row(const DltRig<T>& rig, uint32_t ma
   const uint32_t absent = ~(mask >> (8 * group)) & ((1u << n_in_group) - 1u);
   return rig.absent + ((size_t)group * 256 + absent) * DLT_TABLE_ROW;
 }
-__device__ __forceinline__ void sub_row(const double* row, double (&M)[6], double (&v)[3]) {
-  const double2* r = reinterpret_cast<const double2*>(row);
-  const double2 t0 = __ldg(r), t1 = __ldg(r + 1), t2 = __ldg(r + 2), t3 = __ldg(r + 3), t4 = __ldg(r + 4);
-  M[0] -= t0.x; M[1] -= t0.y; M[2] -= t1.x; M[3] -= t1.y; M[4] -= t2.x; M[5] -= t2.y; v[0] -= t3.x; v[1] -= t3.y; v[2] -= t4.x;
-}
 __device__ __forceinline__ void sub_row(const float* row, float (&M)[6], float (&v)[3]) {
   const float4* r = reinterpret_cast<const float4*>(row);
   const float4 t0 = __ldg(r), t1 = __ldg(r + 1), t2 = __ldg(r + 2);
@@ -61,18 +57,14 @@ __device__ __forceinline__ void sub_row(const float* row, float (&M)[6], float (
 }
 
 // How an absent view is kept out of the sums.
-//   MASK_TABLE      accumulate it at the canonical pixel, subtract its constant contribution from a table afterwards
-//   MASK_SELECT     zero the three row coefficients (both words of a double)
+//   MASK_TABLE      FP32: accumulate it at the canonical pixel, subtract its constant contribution from a table afterwards
 //   MASK_SELECT_HI  FP64: clear only the HIGH word of the three coefficients -- what is left is a denormal below 2^-1042
 //                   whose products with the other coefficients (< 2^40) vanish against the sums; half the selects
-// Measured on the FP64 kernel (100 M frames, profiles/r2_dlt_variants.log): table 1.96 ms, select 1.90 ms, high-word
-// select 1.86 ms -- the kernel is bound by the FP64 pipe (time follows the count of FP64 instructions, 2.9 cycles each),
-// so the table's 18 extra DADD per frame pair cost more than the selects it removes from the other pipes.
-enum { MASK_TABLE = 0, MASK_SELECT = 1, MASK_SELECT_HI = 2 };
-__device__ __forceinline__ double mask_coeff(double a, bool ok, int masking) {
-  return masking == MASK_SELECT_HI ? __hiloint2double(ok ? __double2hiint(a) : 0, __double2loint(a)) : (ok ? a : 0.0);
-}
-__device__ __forceinline__ float mask_coeff(float a, bool ok, int) { return ok ? a : 0.f; }
+// Measured on the FP64 kernel (100 M frames, profiles/r2_dlt_variants.log): table 1.96 ms, select of both words 1.90 ms,
+// high-word select 1.86 ms -- the kernel is bound by the FP64 pipe (time follows the count of FP64 instructions, 2.9 cycles
+// each), so the table's 18 extra DADD per frame pair cost more than the selects it removes from the other pipes.
+enum { MASK_TABLE = 0, MASK_SELECT_HI = 1 };
+__device__ __forceinline__ double mask_coeff(double a, bool ok) { return __hiloint2double(ok ? __double2hiint(a) : 0, __double2loint(a)); }
 
 template <typename T_, bool CENTRED, int MASKING>
 struct DltPolicy {
@@ -97,7 +89,7 @@ struct DltPolicy {
       const T u = r == 0 ? x : y;
       T a0 = fma_(-u, P[8], P[4 * r]), a1 = fma_(-u, P[9], P[4 * r + 1]), a2 = fma_(-u, P[10], P[4 * r + 2]);
       const T b = fma_(u, P[11], -P[4 * r + 3]);
-      if constexpr (MASKING != MASK_TABLE) { a0 = mask_coeff(a0, valid, MASKING); a1 = mask_coeff(a1, valid, MASKING); a2 = mask_coeff(a2, valid, MASKING); }
+      if constexpr (MASKING == MASK_SELECT_HI) { a0 = mask_coeff(a0, valid); a1 = mask_coeff(a1, valid); a2 = mask_coeff(a2, valid); }
       acc_row<T>(a0, a1, a2, b, a.M, a.v);
     }
   }
@@ -123,59 +115,33 @@ struct DltPolicy {
   }
 };
 
-// ---- FP64 streaming tile: two frames per thread, 2..8 cameras (one table row) ----
+// ---- FP64 streaming tile: two frames per thread, 2..8 cameras ----
 // Same operation order as DltPolicy<double> (which serves tails, unaligned rows and more than 8 cameras), so the
-// points are bit-identical whichever kernel a frame lands in.  The canonical-pixel select runs on the raw float
-// (one FSEL per coordinate) ahead of the F2F, off the FP64 dependency chain.
-template <int MASKING, bool SMEM_ADDENDS = false>
+// points are bit-identical whichever kernel a frame lands in.
 struct DltTile64 {
   static constexpr int FPT = 2;
-  using S = DltPolicy<double, false, MASKING>;
+  using S = DltPolicy<double, false, MASK_SELECT_HI>;
   using Rig = DltRig<double>;
   using Real = double;
-  // SMEM_ADDENDS: the eight addends of a camera's rows (P[0..7]) come from shared memory as four LDS.128 instead of
-  // eight LDC.64 (a DFMA takes one operand from the constant bank; the multiplicands P[8..11] keep that slot)
-  static constexpr int CONST_BYTES = SMEM_ADDENDS ? 8 * 8 * (int)sizeof(double) : 0;
-  static __device__ __forceinline__ void stage_consts(const Rig& rig, unsigned char* dst, int tid) {
-    if constexpr (SMEM_ADDENDS)
-      if (tid < 64) reinterpret_cast<double*>(dst)[tid] = rig.P[tid >> 3][tid & 7];
-  }
   template <int NC, int PIX, bool WIDE, class RS>
-  static __device__ __forceinline__ void run(const Rig& rig, const unsigned char* sc, const RS& raw, int,
-                                             double (&X)[2][3], uint32_t (&mask)[2], double (&err)[2], int (&iters)[2]) {
+  static __device__ __forceinline__ void run(const Rig& rig, const RS& raw, int, double (&X)[2][3], uint32_t (&mask)[2],
+                                             double (&err)[2], int (&iters)[2]) {
     typename S::Acc acc[2];
     mask[0] = mask[1] = 0;
 #pragma unroll
     for (int c = 0; c < NC; c++) {
       double P[12];
       load12(rig.P[c], P);
-      if constexpr (SMEM_ADDENDS) {
-        const double2* a = reinterpret_cast<const double2*>(sc) + 4 * c;
-#pragma unroll
-        for (int k = 0; k < 4; k++) { const double2 t = a[k]; P[2 * k] = t.x; P[2 * k + 1] = t.y; }
-      }
       double x[2], y[2];
       bool ok[2];
       if constexpr (PIX == PIX_F32) {
         const Views<float, PIX, 2> q = decode<float, PIX, 2>(raw[c]);
 #pragma unroll
-        for (int j = 0; j < 2; j++) {
-          ok[j] = q.v[j];
-          if constexpr (MASKING == MASK_TABLE) {  // select on the float (one FSEL), then convert: the empty asm keeps that order
-            float xf = ok[j] ? q.x[j] : 0.f, yf = ok[j] ? q.y[j] : 0.f;
-            asm("" : "+f"(xf), "+f"(yf));
-            x[j] = (double)xf; y[j] = (double)yf;
-          }
-          else { x[j] = (double)q.x[j]; y[j] = (double)q.y[j]; }
-        }
+        for (int j = 0; j < 2; j++) { ok[j] = q.v[j]; x[j] = (double)q.x[j]; y[j] = (double)q.y[j]; }
       } else {
         const Views<double, PIX, 2> q = decode<double, PIX, 2>(raw[c]);
 #pragma unroll
-        for (int j = 0; j < 2; j++) {
-          ok[j] = q.v[j];
-          if constexpr (MASKING == MASK_TABLE) { x[j] = ok[j] ? q.x[j] : 0.0; y[j] = ok[j] ? q.y[j] : 0.0; }
-          else { x[j] = q.x[j]; y[j] = q.y[j]; }
-        }
+        for (int j = 0; j < 2; j++) { ok[j] = q.v[j]; x[j] = q.x[j]; y[j] = q.y[j]; }
       }
 #pragma unroll
       for (int j = 0; j < 2; j++) {
@@ -185,7 +151,7 @@ struct DltTile64 {
           const double u = r == 0 ? x[j] : y[j];
           double a0 = fma_(-u, P[8], P[4 * r]), a1 = fma_(-u, P[9], P[4 * r + 1]), a2 = fma_(-u, P[10], P[4 * r + 2]);
           const double b = fma_(u, P[11], -P[4 * r + 3]);
-          if constexpr (MASKING != MASK_TABLE) { a0 = mask_coeff(a0, ok[j], MASKING); a1 = mask_coeff(a1, ok[j], MASKING); a2 = mask_coeff(a2, ok[j], MASKING); }
+          a0 = mask_coeff(a0, ok[j]); a1 = mask_coeff(a1, ok[j]); a2 = mask_coeff(a2, ok[j]);
           acc_row<double>(a0, a1, a2, b, acc[j].M, acc[j].v);
         }
       }
@@ -196,7 +162,6 @@ struct DltTile64 {
       err[j] = 0;
       iters[j] = 0;
       const int n = __popc(mask[j]);
-      if constexpr (MASKING == MASK_TABLE) sub_row(absent_row<double>(rig, mask[j], 0, NC), acc[j].M, acc[j].v);
       if (n >= 2) {
         solve_sym3<double>(acc[j].M, acc[j].v, X[j]);
         if constexpr (WIDE) {
@@ -227,25 +192,13 @@ struct __align__(16) DltRigX2 {
   const float* absent;  // DltRig<float>::absent
 };
 
-template <bool SMEM_CONSTS = false>
-struct DltX2TileT {
+struct DltX2Tile {
   static constexpr int FPT = 2;
   using Rig = DltRigX2;
   using Real = float;
-  // SMEM_CONSTS: a camera's 14 packed constants from shared memory (7 LDS.128) instead of the constant bank
-  static constexpr int CONST_BYTES = SMEM_CONSTS ? 8 * 14 * (int)sizeof(float2) : 0;
-  static __device__ __forceinline__ void stage_consts(const Rig& rig, unsigned char* dst, int tid) {
-    if constexpr (SMEM_CONSTS) {
-      float2* d = reinterpret_cast<float2*>(dst);
-      if (tid < 8 * 14) {
-        const int c = tid / 14, k = tid % 14;
-        d[tid] = k < 8 ? rig.A[c][k] : k < 12 ? rig.N[c][k - 8] : rig.npix0[c][k - 12];
-      }
-    }
-  }
   template <int NC, int PIX, bool WIDE, class RS>
-  static __device__ __forceinline__ void run(const Rig& rig, const unsigned char* sc, const RS& raw, int,
-                                             float (&X)[2][3], uint32_t (&mask)[2], double (&err)[2], int (&iters)[2]) {
+  static __device__ __forceinline__ void run(const Rig& rig, const RS& raw, int, float (&X)[2][3], uint32_t (&mask)[2],
+                                             double (&err)[2], int (&iters)[2]) {
     float2 M[6] = {{0, 0}, {0, 0}, {0, 0}, {0, 0}, {0, 0}, {0, 0}}, v[3] = {{0, 0}, {0, 0}, {0, 0}};
     uint32_t mask0 = 0, mask1 = 0;
 #pragma unroll
@@ -254,20 +207,14 @@ struct DltX2TileT {
       mask0 |= (q.v[0] ? 1u : 0u) << c;
       mask1 |= (q.v[1] ? 1u : 0u) << c;
       float2 K[14];  // this camera's constants
-      if constexpr (SMEM_CONSTS) {
-        const float4* kv = reinterpret_cast<const float4*>(sc) + 7 * c;
+      const float4* kv = reinterpret_cast<const float4*>(rig.A[c]);
 #pragma unroll
-        for (int k = 0; k < 7; k++) { const float4 t = kv[k]; K[2 * k] = make_float2(t.x, t.y); K[2 * k + 1] = make_float2(t.z, t.w); }
-      } else {
-        const float4* kv = reinterpret_cast<const float4*>(rig.A[c]);
+      for (int k = 0; k < 4; k++) { const float4 t = kv[k]; K[2 * k] = make_float2(t.x, t.y); K[2 * k + 1] = make_float2(t.z, t.w); }
+      const float4* nv = reinterpret_cast<const float4*>(rig.N[c]);
 #pragma unroll
-        for (int k = 0; k < 4; k++) { const float4 t = kv[k]; K[2 * k] = make_float2(t.x, t.y); K[2 * k + 1] = make_float2(t.z, t.w); }
-        const float4* nv = reinterpret_cast<const float4*>(rig.N[c]);
-#pragma unroll
-        for (int k = 0; k < 2; k++) { const float4 t = nv[k]; K[8 + 2 * k] = make_float2(t.x, t.y); K[9 + 2 * k] = make_float2(t.z, t.w); }
-        const float4 t = *reinterpret_cast<const float4*>(rig.npix0[c]);
-        K[12] = make_float2(t.x, t.y); K[13] = make_float2(t.z, t.w);
-      }
+      for (int k = 0; k < 2; k++) { const float4 t = nv[k]; K[8 + 2 * k] = make_float2(t.x, t.y); K[9 + 2 * k] = make_float2(t.z, t.w); }
+      const float4 t = *reinterpret_cast<const float4*>(rig.npix0[c]);
+      K[12] = make_float2(t.x, t.y); K[13] = make_float2(t.z, t.w);
       float2 x = __fadd2_rn(make_float2(q.x[0], q.x[1]), K[12]);
       float2 y = __fadd2_rn(make_float2(q.y[0], q.y[1]), K[13]);
       x = make_float2(q.v[0] ? x.x : 0.f, q.v[1] ? x.y : 0.f);  // absent view: the canonical pixel (the rig's pixel origin)
@@ -322,33 +269,6 @@ struct DltX2TileT {
   }
 };
 
-using DltX2Tile = DltX2TileT<false>;
-
-#ifdef TRI_TUNING
-// Memory-roofline probe (TRI_DEBUG_STREAM, tuning builds only): the same pipeline with a near-empty solve -- x = sum
-// of the valid pixel x, y = sum of y, z = number of views -- to measure what the streaming skeleton alone sustains.
-struct StreamProbeTile {
-  static constexpr int FPT = 2;
-  using Rig = DltRigX2;
-  using Real = float;
-  static constexpr int CONST_BYTES = 0;
-  static __device__ __forceinline__ void stage_consts(const Rig&, unsigned char*, int) {}
-  template <int NC, int PIX, bool WIDE, class RS>
-  static __device__ __forceinline__ void run(const Rig&, const unsigned char*, const RS& raw, int, float (&X)[2][3],
-                                             uint32_t (&mask)[2], double (&err)[2], int (&iters)[2]) {
-    mask[0] = mask[1] = 0;
-#pragma unroll
-    for (int j = 0; j < 2; j++) { X[j][0] = X[j][1] = X[j][2] = 0.f; err[j] = 0; iters[j] = 0; }
-#pragma unroll
-    for (int c = 0; c < NC; c++) {
-      const Views<float, PIX, 2> q = decode<float, PIX, 2>(raw[c]);
-#pragma unroll
-      for (int j = 0; j < 2; j++)
-        if (q.v[j]) { X[j][0] += q.x[j]; X[j][1] += q.y[j]; X[j][2] += 1.f; mask[j] |= 1u << c; }
-    }
-  }
-};
-#endif
 
 static DltRigX2 make_x2(const DltRig<float>& r) {
   DltRigX2 x;
@@ -375,58 +295,17 @@ cudaError_t launch_dlt(const LaunchCtx& ctx, bool f32, int pixfmt, const DltRig<
     DltRig<float> rig32 = rig32_;
     rig32.n_use = n_use;
     const DltRigX2 x2 = make_x2(rig32);
-#ifdef TRI_TUNING
-    if (ctx.debug_stream && pixfmt == PIX_F32) {
-      if (ctx.variant == 1) return launch_streamed<StreamProbeTile, P32, PIX_F32, 2, 3, 2, 1>(ctx, x2, rig32, d_xy, n_use, n_frames, cam_stride, out, 0);
-      if (ctx.variant == 2) return launch_streamed<StreamProbeTile, P32, PIX_F32, 2, 4, 2, 1>(ctx, x2, rig32, d_xy, n_use, n_frames, cam_stride, out, 0);
-      return launch_streamed<StreamProbeTile, P32, PIX_F32, 2, 3, 2>(ctx, x2, rig32, d_xy, n_use, n_frames, cam_stride, out, 0);
-    }
-    if (pixfmt == PIX_F32) {
-      switch (ctx.variant) {  // TRI_VARIANT: ring feeders and shapes under A/B measurement (tools/ab_variants.py)
-        case 1: return launch_streamed<DltX2Tile, P32, PIX_F32, 2, 2, 3, 1>(ctx, x2, rig32, d_xy, n_use, n_frames, cam_stride, out, 0);
-        case 2: return launch_streamed<DltX2Tile, P32, PIX_F32, 2, 3, 3, 1>(ctx, x2, rig32, d_xy, n_use, n_frames, cam_stride, out, 0);
-        case 3: return launch_streamed<DltX2Tile, P32, PIX_F32, 2, 3, 2, 1>(ctx, x2, rig32, d_xy, n_use, n_frames, cam_stride, out, 0);
-        case 4: return launch_streamed<DltX2Tile, P32, PIX_F32, 2, 4, 2, 1>(ctx, x2, rig32, d_xy, n_use, n_frames, cam_stride, out, 0);
-        case 5: return launch_streamed<DltX2TileT<true>, P32, PIX_F32, 2, 3, 3, 1>(ctx, x2, rig32, d_xy, n_use, n_frames, cam_stride, out, 0);
-        case 6: return launch_streamed<DltX2Tile, P32, PIX_F32, 2, 2, 3, 2>(ctx, x2, rig32, d_xy, n_use, n_frames, cam_stride, out, 0);
-        case 7: return launch_streamed<DltX2Tile, P32, PIX_F32, 2, 3, 3, 2>(ctx, x2, rig32, d_xy, n_use, n_frames, cam_stride, out, 0);
-        case 8: return launch_streamed<DltX2Tile, P32, PIX_F32, 2, 2, 4, 2>(ctx, x2, rig32, d_xy, n_use, n_frames, cam_stride, out, 0);
-        case 9: return launch_streamed<DltX2Tile, P32, PIX_F32, 2, 3, 4, 2>(ctx, x2, rig32, d_xy, n_use, n_frames, cam_stride, out, 0);
-        default: break;
-      }
-    }
-#endif
     // float2 pixels: read from the slot camera by camera instead of pulled into registers on arrival -- fewer live registers,
     // 1.269 -> 1.224 ms per 100 M frames (profiles/r2_dlt_variants.log); the other solves measured slower that way
-    if (pixfmt == PIX_F32) return launch_streamed<DltX2Tile, P32, PIX_F32, 2, 2, 3, 2>(ctx, x2, rig32, d_xy, n_use, n_frames, cam_stride, out, 0);
+    if (pixfmt == PIX_F32) return launch_streamed<DltX2Tile, P32, PIX_F32, 2, 2, 3, true>(ctx, x2, rig32, d_xy, n_use, n_frames, cam_stride, out, 0);
     if (pixfmt == PIX_F64) return launch_streamed<DltX2Tile, P32, PIX_F64, 2, 2, 3>(ctx, x2, rig32, d_xy, n_use, n_frames, cam_stride, out, 0);
     return launch_streamed<DltX2Tile, P32, PIX_U16, 2, 2, 3>(ctx, x2, rig32, d_xy, n_use, n_frames, cam_stride, out, 0);
   }
   DltRig<double> rig64 = rig64_;
   rig64.n_use = n_use;
-  using T64 = DltTile64<MASK_SELECT_HI>;
-#ifdef TRI_TUNING
-  if (pixfmt == PIX_F32) {
-    switch (ctx.variant) {
-      case 1: return launch_streamed<T64, P64, PIX_F32, 2, 2, 2, 1>(ctx, rig64, rig64, d_xy, n_use, n_frames, cam_stride, out, 0);
-      case 2: return launch_streamed<T64, P64, PIX_F32, 2, 3, 2, 1>(ctx, rig64, rig64, d_xy, n_use, n_frames, cam_stride, out, 0);
-      case 3: return launch_streamed<DltTile64<MASK_TABLE>, P64, PIX_F32, 2, 2, 2>(ctx, rig64, rig64, d_xy, n_use, n_frames, cam_stride, out, 0);
-      case 4: return launch_streamed<DltTile64<MASK_SELECT>, P64, PIX_F32, 2, 2, 2>(ctx, rig64, rig64, d_xy, n_use, n_frames, cam_stride, out, 0);
-      case 5: return launch_streamed<DltTile64<MASK_SELECT_HI, true>, P64, PIX_F32, 2, 2, 2>(ctx, rig64, rig64, d_xy, n_use, n_frames, cam_stride, out, 0);
-      case 6: return launch_streamed<T64, P64, PIX_F32, 2, 2, 2, 2>(ctx, rig64, rig64, d_xy, n_use, n_frames, cam_stride, out, 0);
-      case 7: return launch_streamed<T64, P64, PIX_F32, 2, 3, 2, 2>(ctx, rig64, rig64, d_xy, n_use, n_frames, cam_stride, out, 0);
-      case 8: return launch_streamed<T64, P64, PIX_F32, 2, 2, 3, 2>(ctx, rig64, rig64, d_xy, n_use, n_frames, cam_stride, out, 0);
-      case 9: return launch_streamed<PolicyTile<P64, 1>, P64, PIX_F32, 1, 3, 3, 2>(ctx, rig64, rig64, d_xy, n_use, n_frames, cam_stride, out, 0);
-      case 10: return launch_streamed<PolicyTile<P64, 1>, P64, PIX_F32, 1, 3, 4, 2>(ctx, rig64, rig64, d_xy, n_use, n_frames, cam_stride, out, 0);
-      case 11: return launch_streamed<PolicyTile<P64, 1>, P64, PIX_F32, 1, 3, 4, 0>(ctx, rig64, rig64, d_xy, n_use, n_frames, cam_stride, out, 0);
-      case 12: return launch_streamed<PolicyTile<P64, 1>, P64, PIX_F32, 1, 4, 5, 2>(ctx, rig64, rig64, d_xy, n_use, n_frames, cam_stride, out, 0);
-      default: break;
-    }
-  }
-#endif
-  if (pixfmt == PIX_F32) return launch_streamed<T64, P64, PIX_F32, 2, 2, 2>(ctx, rig64, rig64, d_xy, n_use, n_frames, cam_stride, out, 0);
+  if (pixfmt == PIX_F32) return launch_streamed<DltTile64, P64, PIX_F32, 2, 2, 2>(ctx, rig64, rig64, d_xy, n_use, n_frames, cam_stride, out, 0);
   if (pixfmt == PIX_F64) return launch_batch_policy<P64, PIX_F64, 1, 3>(ctx, rig64, d_xy, n_use, n_frames, cam_stride, out, 0);
-  return launch_streamed<T64, P64, PIX_U16, 2, 3, 2>(ctx, rig64, rig64, d_xy, n_use, n_frames, cam_stride, out, 0);
+  return launch_streamed<DltTile64, P64, PIX_U16, 2, 3, 2>(ctx, rig64, rig64, d_xy, n_use, n_frames, cam_stride, out, 0);
 }
 
 }  // namespace tri

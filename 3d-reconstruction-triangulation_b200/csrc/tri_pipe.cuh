@@ -2,17 +2,13 @@
 //
 // grid = SMs x resident CTAs, each CTA walks tiles t = blockIdx.x, += gridDim.x of BATCH_THREADS x FPT frames; the
 // pixels of the next STAGES tiles are always in flight into a shared-memory ring while the current tile is solved;
-// the 12-byte points leave through a per-warp transpose as 16-byte streaming stores.  Two feeders for the ring:
-//   * stream_kernel: every thread prefetches its own pixels with cp.async (LDGSTS) and waits on its own copy group --
-//     no cross-warp synchronisation at all;
-//   * tma_kernel (TUNING builds only): a producer warp streams each camera's row segment with 1-D bulk async copies
-//     (cp.async.bulk, SASS UBLKCP) that complete on a per-stage `full` mbarrier; the eight consumer warps wait on it,
-//     pull their pixels into registers and release the stage through an `empty` mbarrier (one arrival per warp) -- no
-//     CTA barrier.  Measured in round 2 (profiles/r2_dlt_variants.log): with a near-empty solve it is the faster
-//     feeder (1.10 ms per 100 M frames = 6.9 TB/s, above the driver's copy figure), but under every real solve it
-//     loses to the per-thread feeder (FP32 DLT 1.295 vs 1.269 ms, FP32 ray 1.45 vs 1.32, FP64 DLT 1.96 vs 1.86): the
-//     ninth warp costs registers (288 threads per CTA) and the consumers of a CTA wake together on the stage's
-//     barrier instead of drifting apart.  So the product library ships stream_kernel only.
+// the 12-byte points leave through a per-warp transpose as 16-byte streaming stores.  Every thread prefetches its own
+// pixels with cp.async (LDGSTS) and waits on its own copy group -- no cross-warp synchronisation at all.  A
+// warp-specialised TMA feeder (a producer warp issuing 1-D bulk copies onto per-stage mbarriers) was measured against it
+// in round 2 (profiles/r2_dlt_variants.log): with a near-empty solve it is the faster feeder (1.10 ms per 100 M frames =
+// 6.9 TB/s), but under every real solve it loses (FP32 DLT 1.295 vs 1.269 ms, FP32 ray 1.45 vs 1.32, FP64 DLT 1.96 vs
+// 1.86): the ninth warp costs registers (288 threads per CTA) and the consumers of a CTA wake together on the stage's
+// barrier instead of drifting apart.
 // Algorithmic traffic: 8 B x cameras in, 12 B out per frame; nothing is re-read (profiles/: 7.59 GB per 100 M frames).
 #pragma once
 #include <type_traits>
@@ -21,44 +17,7 @@
 
 namespace tri {
 
-// ---- PTX wrappers (sm_90+ bulk-async / mbarrier; sm_100a here) ----
 __device__ __forceinline__ uint32_t smem_u32(const void* p) { return (uint32_t)__cvta_generic_to_shared(p); }
-__device__ __forceinline__ void mbar_init(uint64_t* bar, uint32_t count) {
-  asm volatile("mbarrier.init.shared::cta.b64 [%0], %1;" ::"r"(smem_u32(bar)), "r"(count));
-}
-__device__ __forceinline__ void fence_barrier_init() { asm volatile("fence.mbarrier_init.release.cluster;" ::: "memory"); }
-__device__ __forceinline__ void fence_proxy_async() { asm volatile("fence.proxy.async.shared::cta;" ::: "memory"); }
-__device__ __forceinline__ void mbar_expect_tx(uint64_t* bar, uint32_t bytes) {
-  asm volatile("mbarrier.arrive.expect_tx.shared::cta.b64 _, [%0], %1;" ::"r"(smem_u32(bar)), "r"(bytes) : "memory");
-}
-__device__ __forceinline__ void mbar_arrive(uint64_t* bar) {
-  asm volatile("mbarrier.arrive.shared::cta.b64 _, [%0];" ::"r"(smem_u32(bar)) : "memory");
-}
-__device__ __forceinline__ void mbar_wait(uint64_t* bar, uint32_t parity) {
-  asm volatile(
-      "{\n"
-      ".reg .pred p;\n"
-      "WAIT_%=:\n"
-      "mbarrier.try_wait.parity.shared::cta.b64 p, [%0], %1;\n"
-      "@p bra DONE_%=;\n"
-      "bra WAIT_%=;\n"
-      "DONE_%=:\n"
-      "}\n" ::"r"(smem_u32(bar)),
-      "r"(parity)
-      : "memory");
-}
-__device__ __forceinline__ void bulk_load(void* smem_dst, const void* gmem_src, uint32_t bytes, uint64_t* bar) {
-  asm volatile("cp.async.bulk.shared::cluster.global.mbarrier::complete_tx::bytes [%0], [%1], %2, [%3];" ::"r"(smem_u32(smem_dst)),
-               "l"(gmem_src), "r"(bytes), "r"(smem_u32(bar))
-               : "memory");
-}
-__device__ __forceinline__ void bulk_store(void* gmem_dst, const void* smem_src, uint32_t bytes) {
-  asm volatile("cp.async.bulk.global.shared::cta.bulk_group [%0], [%1], %2;" ::"l"(gmem_dst), "r"(smem_u32(smem_src)), "r"(bytes)
-               : "memory");
-}
-__device__ __forceinline__ void bulk_commit() { asm volatile("cp.async.bulk.commit_group;" ::: "memory"); }
-template <int N>
-__device__ __forceinline__ void bulk_wait_read() { asm volatile("cp.async.bulk.wait_group.read %0;" ::"n"(N) : "memory"); }
 
 // raw pixels of FPT consecutive frames of one camera, as they sit in the shared-memory stage
 template <int PIX, int FPT> struct RawPix;
@@ -114,56 +73,10 @@ struct RawSrc {
 // ---- tile interface of the streaming kernels ------------------------------------------------------
 // A tile solver TS turns the raw pixels of FPT consecutive frames (one RawPix per camera) into points:
 //     TS::FPT, TS::Rig (a __grid_constant__ parameter), TS::Real (the arithmetic type of the result)
-//     TS::CONST_BYTES, TS::stage_consts(rig, dst, tid)   optional: rig constants the tile wants in shared memory
-//     TS::run<NC, PIX, WIDE>(rig, sc, raw, opt, X, mask, err, iters)     (sc = that shared copy)
+//     TS::run<NC, PIX, WIDE>(rig, raw, opt, X, mask, err, iters)
 // WIDE is a compile-time switch for the optional outputs of tri_batch_out (double3 points, the `error` of
 // triangulatePoint, LM iterations): the lean instantiation (float3 + mask) is what the throughput metric runs,
 // the wide one serves the C++ adapter, whose interface returns cv::Point3d (Triangulator.h:51-52).
-
-// Tile solver built from a scalar policy (tri_batch.cuh): FPT frames per thread, one after the other.
-template <class S, int FPT_>
-struct PolicyTile {
-  static constexpr int FPT = FPT_;
-  using Rig = typename S::Rig;
-  using Real = typename S::T;
-  static constexpr int CONST_BYTES = 0;
-  static __device__ __forceinline__ void stage_consts(const Rig&, unsigned char*, int) {}
-  template <int NC, int PIX, bool WIDE, class RS>
-  static __device__ __forceinline__ void run(const Rig& rig, const unsigned char*, const RS& raw, int opt,
-                                             Real (&X)[FPT][3], uint32_t (&mask)[FPT], double (&err)[FPT], int (&iters)[FPT]) {
-    using T = typename S::T;
-    typename S::Acc acc[FPT];
-#pragma unroll
-    for (int j = 0; j < FPT; j++) mask[j] = 0;
-#pragma unroll
-    for (int c = 0; c < NC; c++) {
-      const Views<T, PIX, FPT> w = decode<T, PIX, FPT>(raw[c]);
-#pragma unroll
-      for (int j = 0; j < FPT; j++)
-        { S::add(rig, c, w.x[j], w.y[j], w.v[j], acc[j]); mask[j] |= (w.v[j] ? 1u : 0u) << c; }
-    }
-#pragma unroll
-    for (int j = 0; j < FPT; j++) {
-      X[j][0] = X[j][1] = X[j][2] = 0;
-      iters[j] = 0;
-      err[j] = 0;
-      const int n = __popc(mask[j]);
-      if (n >= 2) {
-        S::solve(rig, acc[j], mask[j], n, X[j], opt, iters[j]);
-        if constexpr (WIDE) {
-          T e = 0;
-#pragma unroll
-          for (int c = 0; c < NC; c++) {
-            const Views<T, PIX, FPT> w = decode<T, PIX, FPT>(raw[c]);
-            if (w.v[j]) e += S::residual(rig, c, w.x[j], w.y[j], X[j]);
-          }
-          err[j] = S::error(e, n);
-        }
-        S::to_world(rig, X[j]);
-      }
-    }
-  }
-};
 
 // A tile's mask output is its frames' validity bits -- the too-few latch counts them -- unless the tile declares
 // MASK_IS_VALIDITY = false (the robust tile: mask = the inlier set, `iters` carries the number of valid views).
@@ -233,11 +146,6 @@ stream_kernel(const __grid_constant__ typename TS::Rig rig, const char* __restri
   const int tid = threadIdx.x, lane = tid & 31;
   const int64_t stride = gridDim.x;
   int64_t tile = blockIdx.x;
-  unsigned char* sc = smem + STAGES * NC * BATCH_THREADS * RB + (BATCH_THREADS / 32) * (32 * FPT * 12);
-  if constexpr (TS::CONST_BYTES > 0) {  // the only CTA-wide barrier of the kernel, before the first tile
-    TS::stage_consts(rig, sc, tid);
-    __syncthreads();
-  }
 
   auto prefetch = [&](int s, int64_t t) {
     const char* src = xy + (t * BATCH_THREADS + tid) * RB;
@@ -272,7 +180,7 @@ stream_kernel(const __grid_constant__ typename TS::Rig rig, const char* __restri
     uint32_t mask[FPT];
     double err[FPT];
     int iters[FPT];
-    TS::template run<NC, PIX, WIDE>(rig, sc, raw, opt, X, mask, err, iters);
+    TS::template run<NC, PIX, WIDE>(rig, raw, opt, X, mask, err, iters);
     if constexpr (LAZY) {  // the slot is free only now
       if (tile + STAGES * stride < n_tiles) prefetch(s, tile + STAGES * stride);
       cp_async_commit();
@@ -309,100 +217,6 @@ stream_kernel(const __grid_constant__ typename TS::Rig rig, const char* __restri
   cp_async_wait<0>();
 }
 
-
-// ---- warp-specialised TMA feeder (tuning builds) ---------------------------------------------------
-#ifdef TRI_TUNING
-constexpr int TMA_THREADS = BATCH_THREADS + 32;  // eight consumer warps + one producer warp
-
-template <class TS, int NC, int PIX, int STAGES, int MINB, bool WIDE>
-__global__ void __launch_bounds__(TMA_THREADS, WIDE ? 1 : MINB)
-tma_kernel(const __grid_constant__ typename TS::Rig rig, const char* __restrict__ xy, int64_t row_bytes, int64_t n_tiles,
-           BatchOut out, int opt, unsigned long long* first_bad, int64_t frame_base) {
-  constexpr int FPT = TS::FPT;
-  using Raw = typename RawPix<PIX, FPT>::type;
-  using Real = typename TS::Real;
-  constexpr int TILE = BATCH_THREADS * FPT;
-  constexpr int ROW = BATCH_THREADS * (int)sizeof(Raw);  // bytes of one camera's segment of a tile
-  constexpr int STAGE = NC * ROW;
-  extern __shared__ __align__(128) unsigned char smem[];
-  // layout: [STAGES][NC][BATCH_THREADS] Raw | [warps][32 * FPT * 3] float | tile constants | full[STAGES] empty[STAGES]
-  unsigned char* sc = smem + STAGES * STAGE + (BATCH_THREADS / 32) * (32 * FPT * 12);
-  uint64_t* full = reinterpret_cast<uint64_t*>(sc + ((TS::CONST_BYTES + 15) & ~15));
-  uint64_t* empty = full + STAGES;
-  const int tid = threadIdx.x, lane = tid & 31;
-  const int64_t stride = gridDim.x;
-
-  if (tid == 0) {
-#pragma unroll
-    for (int s = 0; s < STAGES; s++) { mbar_init(&full[s], 1); mbar_init(&empty[s], BATCH_THREADS / 32); }
-    fence_barrier_init();
-  }
-  if constexpr (TS::CONST_BYTES > 0) if (tid < BATCH_THREADS) TS::stage_consts(rig, sc, tid);
-  __syncthreads();  // the only CTA-wide barrier: before the first tile
-
-  if (tid >= BATCH_THREADS) {  // ---- producer warp: one elected lane keeps the ring full ----
-    if (lane == 0) {
-      int k = 0;
-      for (int64_t tile = blockIdx.x; tile < n_tiles; tile += stride, k++) {
-        const int s = k % STAGES;
-        if (k >= STAGES) mbar_wait(&empty[s], (uint32_t)((k / STAGES - 1) & 1));  // every consumer warp has pulled tile k - STAGES
-        mbar_expect_tx(&full[s], STAGE);
-        const char* src = xy + tile * ROW;
-#pragma unroll
-        for (int c = 0; c < NC; c++) bulk_load(smem + s * STAGE + c * ROW, src + c * row_bytes, ROW, &full[s]);
-      }
-    }
-    return;
-  }
-
-  float* outw = reinterpret_cast<float*>(smem + STAGES * STAGE) + (tid >> 5) * (32 * FPT * 3);
-  int k = 0;
-  for (int64_t tile = blockIdx.x; tile < n_tiles; tile += stride, k++) {
-    const int s = k % STAGES;
-    mbar_wait(&full[s], (uint32_t)((k / STAGES) & 1));
-    RawSrc<Raw, NC, false> raw;
-#pragma unroll
-    for (int c = 0; c < NC; c++) raw.regs[c] = reinterpret_cast<const Raw*>(smem + s * STAGE + c * ROW)[tid];
-    __syncwarp();
-    if (lane == 0) mbar_arrive(&empty[s]);  // this warp holds its pixels: one of the eight arrivals that free the stage
-
-    Real X[FPT][3];
-    uint32_t mask[FPT];
-    double err[FPT];
-    int iters[FPT];
-    TS::template run<NC, PIX, WIDE>(rig, sc, raw, opt, X, mask, err, iters);
-
-    const int64_t f0 = tile * TILE + (int64_t)tid * FPT;
-#pragma unroll
-    for (int j = 0; j < FPT; j++)
-      if (__popc(mask[j]) < 2) atomicMin(first_bad, (unsigned long long)(frame_base + f0 + j));
-    if (out.mask) {
-      if constexpr (FPT == 2) reinterpret_cast<uint2*>(out.mask)[f0 / 2] = make_uint2(mask[0], mask[1]);
-      else out.mask[f0] = mask[0];
-    }
-    if constexpr (WIDE) {
-      store_wide<FPT, Real>(out, f0, X, err, iters);
-      if (!out.xyz_f32) continue;
-    }
-    __syncwarp();
-    if constexpr (FPT == 2) {
-      float2* o2 = reinterpret_cast<float2*>(outw) + 3 * lane;
-      o2[0] = make_float2((float)X[0][0], (float)X[0][1]); o2[1] = make_float2((float)X[0][2], (float)X[1][0]);
-      o2[2] = make_float2((float)X[1][1], (float)X[1][2]);
-    } else {
-      outw[3 * lane] = (float)X[0][0]; outw[3 * lane + 1] = (float)X[0][1]; outw[3 * lane + 2] = (float)X[0][2];
-    }
-    __syncwarp();
-    float4* dst = reinterpret_cast<float4*>(out.xyz_f32 + 3 * (tile * TILE + (int64_t)(tid - lane) * FPT));
-    const float4* src4 = reinterpret_cast<const float4*>(outw);
-    constexpr int N4 = 32 * FPT * 3 / 4;
-#pragma unroll
-    for (int i = lane; i < N4; i += 32) __stcs(dst + i, src4[i]);
-  }
-}
-
-#endif  // TRI_TUNING
-
 // which optional outputs the caller wants -> the WIDE instantiation; alignment of whatever is written
 static inline bool wants_wide(const BatchOut& out) { return out.xyz_f64 || out.err || out.iters; }
 static inline bool stream_aligned(const void* xy, int64_t row_bytes, int align, const BatchOut& out) {
@@ -410,18 +224,8 @@ static inline bool stream_aligned(const void* xy, int64_t row_bytes, int align, 
            ((uintptr_t)out.mask & 7) || ((uintptr_t)out.err & 15) || ((uintptr_t)out.iters & 7));
 }
 
-// FEED: 0 = cp.async feeder, pixels to registers on arrival; 1 = the TMA feeder (tuning builds); 2 = cp.async feeder, pixels
-// read from the slot as the solve needs them
-template <class TS, int N, int PIX, int STAGES, int MINB, bool WIDE, int FEED>
-static auto feeder_kernel() {
-#ifdef TRI_TUNING
-  if constexpr (FEED == 1) return tma_kernel<TS, N, PIX, STAGES, MINB, WIDE>;
-  else
-#endif
-  return stream_kernel<TS, N, PIX, STAGES, MINB, WIDE, FEED == 2>;
-}
-
-template <class TS, int PIX, int STAGES, int MINB, bool WIDE, int FEED>
+// LAZY: the pixels are read from the slot as the solve needs them (RawSrc) instead of pulled into registers on arrival
+template <class TS, int PIX, int STAGES, int MINB, bool WIDE, bool LAZY>
 static cudaError_t launch_stream_w(const LaunchCtx& ctx, const typename TS::Rig& rig, const char* xy, int n_use, int64_t n_tiles,
                                    int64_t row_bytes, const BatchOut& out, int opt) {
   constexpr int FPT = TS::FPT;
@@ -429,17 +233,15 @@ static cudaError_t launch_stream_w(const LaunchCtx& ctx, const typename TS::Rig&
   cudaError_t err = cudaSuccess;
 #define TRI_CASE(N)                                                                                                     \
   case N: {                                                                                                             \
-    auto kern = feeder_kernel<TS, N, PIX, STAGES, MINB, WIDE, FEED>();                                                    \
-    constexpr int threads = FEED == 1 ? BATCH_THREADS + 32 : BATCH_THREADS;                                                  \
-    constexpr int bytes = STAGES * N * BATCH_THREADS * (int)sizeof(Raw) + (BATCH_THREADS / 32) * 32 * FPT * 12 +         \
-                          ((TS::CONST_BYTES + 15) & ~15) + (FEED == 1 ? 2 * STAGES * 8 : 0);                                  \
+    auto kern = stream_kernel<TS, N, PIX, STAGES, MINB, WIDE, LAZY>;                                                    \
+    constexpr int bytes = STAGES * N * BATCH_THREADS * (int)sizeof(Raw) + (BATCH_THREADS / 32) * 32 * FPT * 12;          \
     err = cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, bytes);                               \
     if (err != cudaSuccess) return err;                                                                                 \
     int per_sm = 1;                                                                                                     \
-    err = cudaOccupancyMaxActiveBlocksPerMultiprocessor(&per_sm, kern, threads, bytes);                                 \
+    err = cudaOccupancyMaxActiveBlocksPerMultiprocessor(&per_sm, kern, BATCH_THREADS, bytes);                           \
     if (err != cudaSuccess) return err;                                                                                 \
     const int64_t grid = std::min<int64_t>(n_tiles, (int64_t)ctx.sm_count * std::max(per_sm, 1));                       \
-    kern<<<(unsigned)grid, threads, bytes, ctx.stream>>>(rig, xy, row_bytes, n_tiles, out, opt, ctx.d_first_bad,        \
+    kern<<<(unsigned)grid, BATCH_THREADS, bytes, ctx.stream>>>(rig, xy, row_bytes, n_tiles, out, opt, ctx.d_first_bad,  \
                                                          ctx.frame_base);                                               \
   } break;
   switch (n_use) { TRI_CASE(2) TRI_CASE(3) TRI_CASE(4) TRI_CASE(5) TRI_CASE(6) TRI_CASE(7) TRI_CASE(8) }
@@ -450,7 +252,7 @@ static cudaError_t launch_stream_w(const LaunchCtx& ctx, const typename TS::Rig&
 
 // Launch the streaming kernel on the full tiles of [0, n_frames); *covered = the number of frames it took
 // (0 if the layout does not qualify: unaligned rows or outputs, fewer frames than a tile).
-template <class TS, int PIX, int STAGES, int MINB, int FEED = 0>
+template <class TS, int PIX, int STAGES, int MINB, bool LAZY = false>
 static cudaError_t launch_stream(const LaunchCtx& ctx, const typename TS::Rig& rig, const void* d_xy, int n_use, int64_t n_frames,
                                  int64_t cam_stride, const BatchOut& out, int opt, int64_t* covered) {
   *covered = 0;
@@ -460,9 +262,9 @@ static cudaError_t launch_stream(const LaunchCtx& ctx, const typename TS::Rig& r
   const int64_t row_bytes = cam_stride * pix_bytes(PIX);
   const int64_t n_tiles = n_frames / TILE;
   if (n_tiles == 0 || n_use < 2 || n_use > 8) return cudaSuccess;
-  if (!stream_aligned(xy, row_bytes, FEED == 1 ? 16 : (int)sizeof(Raw), out)) return cudaSuccess;
-  const cudaError_t err = wants_wide(out) ? launch_stream_w<TS, PIX, STAGES, MINB, true, FEED>(ctx, rig, xy, n_use, n_tiles, row_bytes, out, opt)
-                                          : launch_stream_w<TS, PIX, STAGES, MINB, false, FEED>(ctx, rig, xy, n_use, n_tiles, row_bytes, out, opt);
+  if (!stream_aligned(xy, row_bytes, (int)sizeof(Raw), out)) return cudaSuccess;
+  const cudaError_t err = wants_wide(out) ? launch_stream_w<TS, PIX, STAGES, MINB, true, LAZY>(ctx, rig, xy, n_use, n_tiles, row_bytes, out, opt)
+                                          : launch_stream_w<TS, PIX, STAGES, MINB, false, LAZY>(ctx, rig, xy, n_use, n_tiles, row_bytes, out, opt);
   if (err == cudaSuccess) *covered = n_tiles * TILE;
   return err;
 }
@@ -647,7 +449,7 @@ inline BatchOut advance(const BatchOut& o, int64_t frames) {
 
 
 // streaming kernel on the full tiles, the scalar policy kernel on whatever is left (tails, unaligned rows)
-template <class TS, class S, int PIX, int FPT, int STAGES, int MINB, int FEED = 0>
+template <class TS, class S, int PIX, int FPT, int STAGES, int MINB, bool LAZY = false>
 static cudaError_t launch_streamed(const LaunchCtx& ctx, const typename TS::Rig& tile_rig, const typename S::Rig& rig,
                                    const void* d_xy, int n_use, int64_t n_frames, int64_t cam_stride, const BatchOut& out, int opt) {
   int64_t covered = 0;
@@ -656,7 +458,7 @@ static cudaError_t launch_streamed(const LaunchCtx& ctx, const typename TS::Rig&
     if (S::CHUNKED && n_use > CHUNK_CAMS)  // 9..32 cameras: camera-chunked pipeline over the scalar policy
       err = launch_chunk<S, PIX, S::CHUNK_FPT, 3, 2>(ctx, rig, d_xy, n_use, n_frames, cam_stride, out, opt, &covered);
     else
-      err = launch_stream<TS, PIX, STAGES, MINB, FEED>(ctx, tile_rig, d_xy, n_use, n_frames, cam_stride, out, opt, &covered);
+      err = launch_stream<TS, PIX, STAGES, MINB, LAZY>(ctx, tile_rig, d_xy, n_use, n_frames, cam_stride, out, opt, &covered);
     if (err != cudaSuccess || covered == n_frames) return err;
   }
   LaunchCtx rest = ctx;

@@ -163,10 +163,8 @@ struct RayTableTile {
   using S = RayPolicy<T_>;
   using Rig = typename S::Rig;
   using Real = T_;
-  static constexpr int CONST_BYTES = 0;
-  static __device__ __forceinline__ void stage_consts(const Rig&, unsigned char*, int) {}
   template <int NC, int PIX, bool WIDE, class RS>
-  static __device__ __forceinline__ void run(const Rig& rig, const unsigned char*, const RS& raw, int, T_ (&X)[FPT][3],
+  static __device__ __forceinline__ void run(const Rig& rig, const RS& raw, int, T_ (&X)[FPT][3],
                                              uint32_t (&mask)[FPT], double (&err)[FPT], int (&iters)[FPT]) {
     using T = T_;
     static_assert(NC <= TRI_RAY_TABLE_CAMS, "the mask table covers 8 cameras");
@@ -240,10 +238,8 @@ struct RayX2Tile {
   static constexpr int FPT = 2;
   using Rig = RayRigX2;
   using Real = float;
-  static constexpr int CONST_BYTES = 0;
-  static __device__ __forceinline__ void stage_consts(const Rig&, unsigned char*, int) {}
   template <int NC, int PIX, bool WIDE, class RS>
-  static __device__ __forceinline__ void run(const Rig& r, const unsigned char*, const RS& raw, int, float (&X)[2][3],
+  static __device__ __forceinline__ void run(const Rig& r, const RS& raw, int, float (&X)[2][3],
                                              uint32_t (&mask)[2], double (&err)[2], int (&iters)[2]) {
     const float2 z = make_float2(0.f, 0.f);
     float2 uu[6] = {z, z, z, z, z, z}, cu[3] = {z, z, z};
@@ -335,18 +331,9 @@ cudaError_t launch_ray_fold(const LaunchCtx& ctx, bool lm, bool f32, int pixfmt,
       case PIX_F32:
         // 3 stages x 2 CTAs per SM: 1.32 ms per 100 M frames; 2 stages x 3 CTAs (the DLT's choice): 1.47 ms -- with the
         // lighter solve the kernel waits on memory (ncu r1f: long_scoreboard on top), so depth beats occupancy
-#ifdef TRI_TUNING
-        if (ctx.variant == 1) return launch_streamed<RayX2Tile, P32, PIX_F32, 2, 3, 2, 1>(ctx, x2, r32, d_xy, n_use, n_frames, cam_stride, out, 0);
-        if (ctx.variant == 2) return launch_streamed<RayX2Tile, P32, PIX_F32, 2, 4, 2, 1>(ctx, x2, r32, d_xy, n_use, n_frames, cam_stride, out, 0);
-        if (ctx.variant == 3) return launch_streamed<RayX2Tile, P32, PIX_F32, 2, 3, 3, 1>(ctx, x2, r32, d_xy, n_use, n_frames, cam_stride, out, 0);
-        if (ctx.variant == 4) return launch_streamed<RayX2Tile, P32, PIX_F32, 2, 3, 2, 2>(ctx, x2, r32, d_xy, n_use, n_frames, cam_stride, out, 0);
-        if (ctx.variant == 5) return launch_streamed<RayX2Tile, P32, PIX_F32, 2, 3, 3, 2>(ctx, x2, r32, d_xy, n_use, n_frames, cam_stride, out, 0);
-        if (ctx.variant == 6) return launch_streamed<RayX2Tile, P32, PIX_F32, 2, 2, 4, 2>(ctx, x2, r32, d_xy, n_use, n_frames, cam_stride, out, 0);
-        if (ctx.variant == 7) return launch_streamed<RayX2Tile, P32, PIX_F32, 2, 4, 3, 2>(ctx, x2, r32, d_xy, n_use, n_frames, cam_stride, out, 0);
-#endif
         // one pass over the views, pixels read from the slot as they are needed: 1.32 -> 1.26 ms per 100 M frames
         // (profiles/r2_dlt_variants.log; with the pixels pulled into registers on arrival the single pass measured 1.37)
-        return launch_streamed<RayX2Tile, P32, PIX_F32, 2, 3, 2, 2>(ctx, x2, r32, d_xy, n_use, n_frames, cam_stride, out, 0);
+        return launch_streamed<RayX2Tile, P32, PIX_F32, 2, 3, 2, true>(ctx, x2, r32, d_xy, n_use, n_frames, cam_stride, out, 0);
       case PIX_F64: return launch_streamed<RayX2Tile, P32, PIX_F64, 2, 3, 2>(ctx, x2, r32, d_xy, n_use, n_frames, cam_stride, out, 0);
       default: return launch_streamed<RayX2Tile, P32, PIX_U16, 2, 3, 2>(ctx, x2, r32, d_xy, n_use, n_frames, cam_stride, out, 0);
     }
@@ -358,15 +345,6 @@ cudaError_t launch_ray_fold(const LaunchCtx& ctx, bool lm, bool f32, int pixfmt,
   using CFT = RayTableTile<double, false, 2>;
   switch (pixfmt) {
     case PIX_F32:
-#ifdef TRI_TUNING
-      if (ctx.variant == 1) return lm ? launch_streamed<LMT, P64, PIX_F32, 2, 2, 2, 1>(ctx, r64, r64, d_xy, n_use, n_frames, cam_stride, out, opt)
-                                      : launch_streamed<CFT, P64, PIX_F32, 2, 3, 2, 1>(ctx, r64, r64, d_xy, n_use, n_frames, cam_stride, out, opt);
-      if (ctx.variant == 2) return lm ? launch_streamed<LMT, P64, PIX_F32, 2, 2, 2, 2>(ctx, r64, r64, d_xy, n_use, n_frames, cam_stride, out, opt)
-                                      : launch_streamed<CFT, P64, PIX_F32, 2, 3, 2, 2>(ctx, r64, r64, d_xy, n_use, n_frames, cam_stride, out, opt);
-      if (ctx.variant == 3) return lm ? launch_streamed<LMT, P64, PIX_F32, 2, 3, 3, 2>(ctx, r64, r64, d_xy, n_use, n_frames, cam_stride, out, opt)
-                                      : launch_streamed<CFT, P64, PIX_F32, 2, 3, 3, 2>(ctx, r64, r64, d_xy, n_use, n_frames, cam_stride, out, opt);
-      if (ctx.variant == 4) return launch_streamed<RayTableTile<double, false, 1>, P64, PIX_F32, 1, 3, 4, 2>(ctx, r64, r64, d_xy, n_use, n_frames, cam_stride, out, opt);
-#endif
       // (4- and 6-stage rings measured the same: these two are FP64-pipe-bound)
       return lm ? launch_streamed<LMT, P64, PIX_F32, 2, 2, 2>(ctx, r64, r64, d_xy, n_use, n_frames, cam_stride, out, opt)
                 : launch_streamed<CFT, P64, PIX_F32, 2, 3, 2>(ctx, r64, r64, d_xy, n_use, n_frames, cam_stride, out, opt);

@@ -148,11 +148,9 @@ struct RobustTile {
   static constexpr int FPT = 1;
   using Rig = RobustRig<T>;
   using Real = T;
-  static constexpr int CONST_BYTES = 0;
   static constexpr bool MASK_IS_VALIDITY = false;  // mask = the inlier set; `iters` carries the valid-view count
-  static __device__ __forceinline__ void stage_consts(const Rig&, unsigned char*, int) {}
   template <int NC, int PIX, bool WIDE, class RS>
-  static __device__ __forceinline__ void run(const Rig& rig, const unsigned char*, const RS& raw, int, T (&X)[1][3],
+  static __device__ __forceinline__ void run(const Rig& rig, const RS& raw, int, T (&X)[1][3],
                                              uint32_t (&mask)[1], double (&err)[1], int (&iters)[1]) {
     auto pix = [&](int c, T& x, T& y) -> bool {
       const Views<T, PIX, 1> q = decode<T, PIX, 1>(raw[c]);
@@ -214,7 +212,7 @@ static cudaError_t robust_streamed(const LaunchCtx& ctx, const RobustRig<T>& rig
                                    int64_t cam_stride, const BatchOut& out) {
   int64_t covered = 0;
   if constexpr (PIX != PIX_F64) {
-    const cudaError_t err = launch_stream<RobustTile<T>, PIX, 2, 2, 2>(ctx, rig, d_xy, n_use, n_frames, cam_stride, out, 0, &covered);
+    const cudaError_t err = launch_stream<RobustTile<T>, PIX, 2, 2, true>(ctx, rig, d_xy, n_use, n_frames, cam_stride, out, 0, &covered);
     if (err != cudaSuccess || covered == n_frames) return err;
   }
   const int64_t rest = n_frames - covered;

@@ -52,10 +52,8 @@ enum tri_flags {
   TRI_CLS_LAZY = 1u << 7,         /* tri_classify / tri_classify_sequences: the lazy best-first search instead of the candidate
                                      enumeration -- always used above 16 cameras, where the enumeration (like the reference's
                                      own, DroneClassifier.cpp:156-198) is out of reach; same results where both can run   */
-  TRI_RAY_ANALYTIC_LM = 1u << 6,  /* ray batch: Levenberg-Marquardt with the analytic Jacobian and cv::LMSolver's damping
+  TRI_RAY_ANALYTIC_LM = 1u << 6   /* ray batch: Levenberg-Marquardt with the analytic Jacobian and cv::LMSolver's damping
                                      schedule, register resident (3 iterations; same minimiser as the default)      */
-  TRI_DEBUG_STREAM = 1u << 30     /* tuning build only (libtri_b200_tuning.so; TRI_ERR_ARG otherwise): the streaming
-                                     pipeline with a near-empty solve, xyz = (sum x, sum y, views)  */
 };
 /* Ray solver defaults.  tri_triangulate_points*: the closed form -- the reference returns only the point from
  * triangulatePoints (RayTriangulator.cpp:51-81), the objective is quadratic and its LM stops within ~1e-3 mm of this

@@ -7,7 +7,7 @@ from tri_b200 import synthetic as S
 name = sys.argv[1] if len(sys.argv) > 1 else "dlt_f32"
 reps = int(sys.argv[2]) if len(sys.argv) > 2 else 400
 frames = int(sys.argv[3]) if len(sys.argv) > 3 else 100_000_000
-variants = {"dlt_f64": (T.MATRIX, 0), "dlt_f32": (T.MATRIX, T.F32), "stream_probe": (T.MATRIX, T.F32 | T.DEBUG_STREAM), "ray_f64": (T.RAY, 0)}
+variants = {"dlt_f64": (T.MATRIX, 0), "dlt_f32": (T.MATRIX, T.F32), "ray_f64": (T.RAY, 0)}
 mode, fl = variants[name]
 cams = S.ring_rig(8)
 eng = T.Engine(cams, 0)

@@ -1,4 +1,4 @@
-"""End-to-end (pinned host buffers -> tri_triangulate_points -> pinned host result) timing, for chunk tuning."""
+"""End-to-end (pinned host buffers -> tri_triangulate_points -> pinned host result) timing."""
 import os, sys, time
 sys.path.insert(0, os.path.dirname(os.path.dirname(os.path.abspath(__file__))))
 import torch
@@ -15,4 +15,4 @@ for rep in range(4):
     t0 = time.perf_counter()
     eng.triangulate_points_raw(T.MATRIX, T.ALLOW_TOO_FEW, h_xy.data_ptr(), 8, F, F, xyz_f32_ptr=h_out.data_ptr())
     dt = time.perf_counter() - t0
-    print("chunk=%s  %.1f ms  %.2e frames/s  %.1f GB/s" % (os.environ.get("TRI_CHUNK_FRAMES", "default"), dt * 1e3, F / dt, 76 * F / dt / 1e9), flush=True)
+    print("%.1f ms  %.2e frames/s  %.1f GB/s" % (dt * 1e3, F / dt, 76 * F / dt / 1e9), flush=True)

@@ -1,5 +1,5 @@
 """Linking-pass timing loop: S09_D6 (3000 frames x 6 drones) and a synthetic 6-drone sequence, link_us from the call's own events.
-  [TRI_B200_LIB=.../libtri_b200_tuning.so TRI_CLS_PROFILE=1] python tools/link_iter.py [--frames N]"""
+  python tools/link_iter.py [--frames N]"""
 import argparse
 import os
 import sys

@@ -22,7 +22,7 @@ eng = T.Engine(cams, 0)
 xy = S.generate_frames(cams, a.frames, device="cuda:0")
 out = {"xyz_f32": torch.empty((a.frames, 3), dtype=torch.float32, device="cuda:0")}
 variants = {"dlt_f64": (T.MATRIX, 0), "dlt_f32": (T.MATRIX, T.F32), "ray_f64": (T.RAY, T.RAY_ANALYTIC_LM), "ray_f32": (T.RAY, T.F32),
-            "ray_closed_f64": (T.RAY, 0), "stream_probe": (T.MATRIX, T.F32 | T.DEBUG_STREAM), "ray_ref": (T.RAY, T.RAY_REFERENCE_LM)}
+            "ray_closed_f64": (T.RAY, 0), "ray_ref": (T.RAY, T.RAY_REFERENCE_LM)}
 for name in a.only.split(","):
     mode, fl = variants[name]
     n = a.frames if name != "ray_ref" else min(a.frames, 200_000)
