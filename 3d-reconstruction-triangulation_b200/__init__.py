@@ -67,9 +67,9 @@ class ClassifyStats(C.Structure):
 EXPORTS = ["tri_version", "tri_last_error", "tri_device_count", "tri_create", "tri_destroy", "tri_engine_device",
            "tri_engine_cameras", "tri_kernel_launches", "tri_triangulate_points", "tri_triangulate_points_multi",
            "tri_triangulate_points_device", "tri_triangulate_points_robust", "tri_triangulate_points_robust_device",
-           "tri_device_status", "tri_enable_peer_access", "tri_ipc_export", "tri_ipc_open", "tri_ipc_close",
-           "tri_copy_device", "tri_triangulate_subsets", "tri_dist_from_ray", "tri_classify", "tri_classify_state_bytes",
-           "tri_classify_begin", "tri_classify_finish", "tri_classify_multi", "tri_classify_sequences", "tri_host_alloc",
+           "tri_project_points", "tri_project_points_device", "tri_device_status", "tri_enable_peer_access",
+           "tri_ipc_export", "tri_ipc_open", "tri_ipc_close", "tri_copy_device", "tri_triangulate_subsets", "tri_dist_from_ray",
+           "tri_classify", "tri_classify_state_bytes", "tri_classify_begin", "tri_classify_finish", "tri_classify_multi", "tri_classify_sequences", "tri_host_alloc",
            "tri_host_free", "tri_device_alloc", "tri_device_free", "tri_copy_to_device", "tri_copy_to_host"]
 
 _lib = None
@@ -102,6 +102,9 @@ def lib():
                                                     C.POINTER(_BatchOut), C.POINTER(C.c_int64)]
         L.tri_triangulate_points_robust_device.argtypes = [C.c_void_p, C.c_uint, C.c_double, C.c_void_p, C.c_int, C.c_int64,
                                                            C.c_int64, C.POINTER(_BatchOut), C.c_void_p]
+        L.tri_project_points.argtypes = [C.c_void_p, C.c_uint, C.c_void_p, C.c_void_p, C.c_int64, C.c_void_p, C.c_int64, C.c_void_p]
+        L.tri_project_points_device.argtypes = [C.c_void_p, C.c_uint, C.c_void_p, C.c_void_p, C.c_int64, C.c_void_p, C.c_int64,
+                                                C.c_void_p, C.c_void_p]
         L.tri_enable_peer_access.argtypes = [C.c_void_p, C.c_int]
         L.tri_ipc_export.argtypes = [C.c_void_p, C.c_void_p, C.c_char_p]
         L.tri_ipc_open.argtypes = [C.c_void_p, C.c_char_p, C.POINTER(C.c_void_p)]
@@ -422,6 +425,69 @@ class Engine:
         stream = torch.cuda.current_stream(xy.device).cuda_stream
         _check(lib().tri_triangulate_points_robust_device(self._h, flags | fmt, float(max_reproj_px), C.c_void_p(xy.data_ptr()), npc, nf,
                                                           stride, C.byref(bo), C.c_void_p(stream)))
+        return out
+
+    # ---- forward projection: points -> per-camera pixels in the batch input layout (an extension of the reference) ----
+    def project_points(self, xyz, flags=0, pix_dtype=np.float32):
+        """xyz: numpy [n, 3] float32 | float64 (host memory; the dtype picks the input).  FP64 unless flags has F32.
+        -> {"xy": [n_cams, n, 2] pix_dtype (float32 | float64 | uint16), "mask": uint32 [n] (bit c = camera c sees the
+        point)}; views a camera does not see hold the missing marker ((-1,-1), 0xFFFF pairs for uint16)."""
+        xyz = np.ascontiguousarray(xyz)
+        if xyz.ndim != 2 or xyz.shape[1] != 3 or xyz.dtype not in (np.float32, np.float64):
+            raise TriError(ERR_ARG, "xyz must be a float32 or float64 array of shape [n, 3]")
+        n = xyz.shape[0]
+        fmt = _PIX_DTYPES[np.dtype(pix_dtype)]
+        out = {"xy": np.empty((len(self.cameras), n, 2), pix_dtype), "mask": np.empty(n, np.uint32)}
+        f32 = xyz.dtype == np.float32
+        _check(lib().tri_project_points(self._h, flags | fmt, _np_ptr(xyz) if f32 else None, None if f32 else _np_ptr(xyz), n,
+                                        _np_ptr(out["xy"]), n, _np_ptr(out["mask"])))
+        return out
+
+    def project_points_device(self, xyz, flags=0, pix_dtype=None, out=None, want=("xy", "mask")):
+        """xyz: torch tensor [n, 3] float32 | float64 on cuda:<device>, rows packed (stride (3, 1)); asynchronous on the
+        current stream.  out: optional dict with "xy" [n_cams, n, 2] (pairs packed, any camera stride >= n) and / or
+        "mask" int32 [n] tensors, written in place.  Returns the dict (torch tensors)."""
+        import torch
+        pix_dtype = pix_dtype or torch.float32
+        nc = len(self.cameras)
+        dev = torch.device("cuda", self.device)
+
+        def need(ok, what):
+            if not ok:
+                raise TriError(ERR_ARG, "project_points_device: " + what)
+
+        # the kernel reads 12 or 24 B per point and writes all n_cams rows: every buffer is checked against that
+        need(xyz.is_cuda and xyz.device == dev, "xyz must be on the engine's GPU")
+        need(xyz.dtype in (torch.float32, torch.float64), "xyz must be float32 or float64")
+        need(xyz.dim() == 2 and xyz.shape[1] == 3 and (xyz.shape[0] <= 1 or xyz.stride() == (3, 1)), "xyz must be packed [n, 3]")
+        n = xyz.shape[0]
+        if out is None:
+            out = {}
+            if "xy" in want:
+                out["xy"] = torch.empty((nc, n, 2), dtype=pix_dtype, device=dev)
+            if "mask" in want:
+                out["mask"] = torch.empty((n,), dtype=torch.int32, device=dev)
+        xy, mask = out.get("xy"), out.get("mask")
+        stride = n
+        fmt = 0
+        if xy is not None:
+            need(xy.is_cuda and xy.device == dev, "out['xy'] must be on the engine's GPU")
+            need(xy.dtype in (torch.float32, torch.float64, torch.uint16), "out['xy'] must be float32, float64 or uint16")
+            need(xy.dim() == 3 and tuple(xy.shape) == (nc, n, 2), "out['xy'] must be [n_cams, n, 2]")
+            need(n == 0 or (xy.stride(2) == 1 and xy.stride(1) == 2), "out['xy'] must hold packed pixel pairs")
+            need(nc == 1 or (xy.stride(0) % 2 == 0 and xy.stride(0) // 2 >= n), "out['xy'] camera rows must not overlap")
+            fmt = {torch.float32: 0, torch.float64: PIX_F64, torch.uint16: PIX_U16}[xy.dtype]
+            stride = xy.stride(0) // 2 if nc > 1 else n
+        if mask is not None:
+            need(mask.is_cuda and mask.device == dev, "out['mask'] must be on the engine's GPU")
+            need(mask.dtype in (torch.int32, torch.uint32) and mask.dim() == 1 and mask.numel() == n
+                 and (n <= 1 or mask.stride(0) == 1), "out['mask'] must be a contiguous int32 / uint32 tensor of n elements")
+        f32 = xyz.dtype == torch.float32
+        p = C.c_void_p(xyz.data_ptr())
+        stream = torch.cuda.current_stream(xyz.device).cuda_stream
+        _check(lib().tri_project_points_device(self._h, flags | fmt, p if f32 else None, None if f32 else p, n,
+                                               C.c_void_p(xy.data_ptr()) if xy is not None else None, stride,
+                                               C.c_void_p(mask.data_ptr()) if mask is not None else None, C.c_void_p(stream)))
         return out
 
     # ---- Triangulator::triangulatePoint over many camera subsets ----

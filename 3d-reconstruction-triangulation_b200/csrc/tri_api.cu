@@ -356,6 +356,77 @@ static int run_host_pipeline(tri_engine* e, unsigned flags, int fmt, const void*
   return TRI_OK;
 }
 
+// Arguments of the projection pair (tri_project_points*).
+static int check_project_args(tri_engine* e, unsigned flags, const float* xyz_f32, const double* xyz_f64, int64_t n_points,
+                              const void* xy, int64_t cam_stride, const uint32_t* mask, int* fmt) {
+  if (!e) return fail(TRI_ERR_ARG, "null engine");
+  if (flags & ~(unsigned)(TRI_F32 | TRI_PIX_F64 | TRI_PIX_U16))
+    return fail(TRI_ERR_ARG, "projection accepts TRI_F32, TRI_PIX_F64 and TRI_PIX_U16 only");
+  int st = pix_format(flags, fmt);
+  if (st != TRI_OK) return st;
+  if (n_points < 0) return fail(TRI_ERR_ARG, "negative size");
+  if (n_points > 0 && (!xyz_f32) == (!xyz_f64)) return fail(TRI_ERR_ARG, "exactly one of xyz_f32 / xyz_f64 must be given");
+  if (n_points > 0 && !xy && !mask) return fail(TRI_ERR_ARG, "no output buffer (xy and mask are both null)");
+  if (cam_stride < n_points) return fail(TRI_ERR_DIM, "Every camera should have the same number of points");
+  if (*fmt == PIX_U16)
+    for (int c = 0; c < e->n_cams; c++)
+      if (e->cams[c].width > 65535 || e->cams[c].height > 65535)
+        return fail(TRI_ERR_ARG, "TRI_PIX_U16: a camera is larger than 65535 pixels, its pixels could collide with the missing marker");
+  return TRI_OK;
+}
+
+// Host-buffer projection: the batch pipeline with the copy directions swapped.  Points go H2D chunk by chunk through
+// the N_SLOTS staging slots, the kernel writes the chunk's pixel rows and masks into the slot, and one D2H copy per
+// camera row (plus one for the masks) lands them in the caller's cam_stride-strided rows.
+static int run_project_pipeline(tri_engine* e, bool f32, int fmt, const float* xyz_f32, const double* xyz_f64, int64_t n_points,
+                                void* xy, int64_t cam_stride, uint32_t* mask) {
+  const size_t pb = pix_bytes(fmt), in_pp = xyz_f32 ? 12 : 24;
+  const int nc = e->n_cams;
+  // ~64 MB of output rows per slot: large enough for full-rate copies, small enough to pipeline
+  const size_t out_pp = (xy ? nc * pb : 0) + (mask ? 4 : 0);
+  int64_t chunk = std::min<int64_t>(std::max<int64_t>((int64_t)((64u << 20) / out_pp) / 256 * 256, 1 << 16), 4 << 20);
+  if (n_points <= chunk) chunk = n_points;
+  const size_t row = align_up((size_t)chunk * pb, 256);
+  const size_t o_mask = xy ? row * nc : 0;
+  const size_t out_bytes = o_mask + (mask ? align_up((size_t)chunk * 4, 256) : 0);
+  const int n_slots = n_points > chunk ? N_SLOTS : 1;
+  int st;
+  for (int i = 0; i < n_slots; i++) {
+    if ((st = ensure(&e->slots[i].d_in, &e->slots[i].in_cap, align_up((size_t)chunk * in_pp, 256))) != TRI_OK) return st;
+    if ((st = ensure(&e->slots[i].d_out, &e->slots[i].out_cap, out_bytes)) != TRI_OK) return st;
+  }
+  const char* src = xyz_f32 ? (const char*)xyz_f32 : (const char*)xyz_f64;
+  char* dst = static_cast<char*>(xy);
+  auto run = [&]() -> int {
+    int k = 0;
+    for (int64_t p0 = 0; p0 < n_points; p0 += chunk, k++) {
+      Slot& s = e->slots[k % n_slots];
+      const int64_t n = std::min(chunk, n_points - p0);
+      TRI_CUDA(cudaStreamSynchronize(s.stream));  // slot free (its previous D2H has landed)
+      TRI_CUDA(cudaMemcpyAsync(s.d_in, src + (size_t)p0 * in_pp, (size_t)n * in_pp, cudaMemcpyHostToDevice, s.stream));
+      uint32_t* d_mask = mask ? (uint32_t*)(s.d_out + o_mask) : nullptr;
+      const cudaError_t err = launch_project(e->ctx(s.stream, p0, true), f32, fmt, e->rig64, e->rig32, e->cams, nc,
+                                             xyz_f32 ? (const float*)s.d_in : nullptr, xyz_f64 ? (const double*)s.d_in : nullptr, n,
+                                             xy ? s.d_out : nullptr, (int64_t)(row / pb), d_mask);
+      if (err != cudaSuccess) return cuda_fail(err, "kernel launch");
+      if (xy)
+        for (int c = 0; c < nc; c++)
+          TRI_CUDA(cudaMemcpyAsync(dst + ((size_t)c * cam_stride + p0) * pb, s.d_out + (size_t)c * row, (size_t)n * pb,
+                                   cudaMemcpyDeviceToHost, s.stream));
+      if (mask) TRI_CUDA(cudaMemcpyAsync(mask + p0, d_mask, (size_t)n * 4, cudaMemcpyDeviceToHost, s.stream));
+    }
+    for (int i = 0; i < n_slots; i++) TRI_CUDA(cudaStreamSynchronize(e->slots[i].stream));
+    return TRI_OK;
+  };
+  if ((st = run()) != TRI_OK) {
+    const std::string why = g_error;
+    for (int i = 0; i < n_slots; i++) cudaStreamSynchronize(e->slots[i].stream);  // nothing is left in flight into the caller's memory
+    cudaGetLastError();
+    return fail(st, why);
+  }
+  return TRI_OK;
+}
+
 }  // namespace tri
 
 using namespace tri;
@@ -557,6 +628,26 @@ int tri_triangulate_points_robust(tri_engine* e, unsigned flags, double max_repr
                                                                    d_in, n_use, n, stride, o);
                              return err == cudaSuccess ? TRI_OK : cuda_fail(err, "kernel launch");
                            });
+}
+
+int tri_project_points_device(tri_engine* e, unsigned flags, const float* d_xyz_f32, const double* d_xyz_f64, int64_t n_points,
+                              void* d_xy, int64_t cam_stride, uint32_t* d_mask, void* stream) {
+  int fmt = 0;
+  const int st = check_project_args(e, flags, d_xyz_f32, d_xyz_f64, n_points, d_xy, cam_stride, d_mask, &fmt);
+  if (st != TRI_OK || n_points == 0) return st;
+  DeviceGuard g(e->device);
+  const cudaError_t err = launch_project(e->ctx((cudaStream_t)stream), (flags & TRI_F32) != 0, fmt, e->rig64, e->rig32, e->cams, e->n_cams,
+                                         d_xyz_f32, d_xyz_f64, n_points, d_xy, cam_stride, d_mask);
+  return err == cudaSuccess ? TRI_OK : cuda_fail(err, "kernel launch");
+}
+
+int tri_project_points(tri_engine* e, unsigned flags, const float* xyz_f32, const double* xyz_f64, int64_t n_points, void* xy,
+                       int64_t cam_stride, uint32_t* mask) {
+  int fmt = 0;
+  const int st = check_project_args(e, flags, xyz_f32, xyz_f64, n_points, xy, cam_stride, mask, &fmt);
+  if (st != TRI_OK || n_points == 0) return st;
+  DeviceGuard g(e->device);
+  return run_project_pipeline(e, (flags & TRI_F32) != 0, fmt, xyz_f32, xyz_f64, n_points, xy, cam_stride, mask);
 }
 
 int tri_triangulate_points_multi(tri_engine* const* engines, int n_engines, int mode, unsigned flags, const void* xy,

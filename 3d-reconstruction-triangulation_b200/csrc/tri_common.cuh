@@ -159,4 +159,10 @@ cudaError_t launch_robust(const LaunchCtx& ctx, bool f32, int pixfmt, const DltR
                           double max_reproj_px, const void* d_xy, int n_use, int64_t n_frames, int64_t cam_stride,
                           const BatchOut& out);
 
+// forward projection (tri_project.cu): points [n][3] (exactly one of d_xyz_f32 / d_xyz_f64) to the pixel rows of all
+// n_cams cameras in format `pixfmt` (d_xy may be null) and the visibility masks (d_mask may be null)
+cudaError_t launch_project(const LaunchCtx& ctx, bool f32, int pixfmt, const DltRig<double>& rig64, const DltRig<float>& rig32,
+                           const tri_camera* cams, int n_cams, const float* d_xyz_f32, const double* d_xyz_f64, int64_t n_points,
+                           void* d_xy, int64_t cam_stride, uint32_t* d_mask);
+
 }  // namespace tri

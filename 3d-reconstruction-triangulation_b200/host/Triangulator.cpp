@@ -190,6 +190,25 @@ std::vector<cv::Point3d> Triangulator::triangulatePoints(std::vector<std::vector
   return result;
 }
 
+std::vector<std::vector<cv::Point2d>> Triangulator::projectPoints(const std::vector<cv::Point3d>& points, std::vector<uint32_t>* visible) {
+  const int64_t n = (int64_t)points.size();
+  const size_t nc = cameras.size();
+  std::vector<double> xyz(3 * (size_t)n), xy(2 * nc * (size_t)n);
+  for (int64_t i = 0; i < n; i++) {
+    xyz[3 * i] = points[i].x;
+    xyz[3 * i + 1] = points[i].y;
+    xyz[3 * i + 2] = points[i].z;
+  }
+  if (visible) visible->assign((size_t)n, 0);
+  const int st = tri_project_points(engine_, (flags_ & TRI_F32) | TRI_PIX_F64, nullptr, xyz.data(), n, xy.data(), n,
+                                    visible ? visible->data() : nullptr);
+  if (st != TRI_OK) throw std::runtime_error(std::string("tri_b200: ") + tri_last_error());
+  std::vector<std::vector<cv::Point2d>> out(nc, std::vector<cv::Point2d>((size_t)n));
+  for (size_t c = 0; c < nc; c++)
+    for (int64_t i = 0; i < n; i++) out[c][i] = cv::Point2d(xy[2 * (c * n + i)], xy[2 * (c * n + i) + 1]);
+  return out;
+}
+
 double Triangulator::getDistFromRay(CamPointPair pair, cv::Point3d point) {
   Triangulator* owner = nullptr;
   int idx = -1;

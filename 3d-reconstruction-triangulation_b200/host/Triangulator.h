@@ -39,6 +39,12 @@ class Triangulator {
   // below 65535; a pair with x == -1 or y == -1 becomes the missing marker), 0 (float2) or TRI_PIX_F64
   static unsigned pixelFormatFor(const std::vector<std::vector<cv::Point2d>>& points);
 
+  // Extension (the reference has no such method): the forward model of the rig, points -> pixels
+  // (tri_project_points).  Returns points[cam][frame] for every camera of the triangulator, (-1,-1) where the camera
+  // does not see the point (behind it or outside the image) -- exactly triangulatePoints' input.  visible[f]: bit c =
+  // camera c sees point f.  FP64 (FP32 if flags() has TRI_F32).
+  std::vector<std::vector<cv::Point2d>> projectPoints(const std::vector<cv::Point3d>& points, std::vector<uint32_t>* visible = nullptr);
+
   // :58 -- distance of `point` to the pixel ray of `pair`
   static double getDistFromRay(CamPointPair pair, cv::Point3d point);
 

@@ -135,6 +135,23 @@ int tri_triangulate_points_robust_device(tri_engine* e, unsigned flags, double m
                                          int n_point_cams, int64_t n_frames, int64_t cam_stride,
                                          const tri_batch_out* d_out, void* stream);
 
+/* Forward projection (an extension: the reference has no batch call for it).  Point i, camera c of the engine:
+ * (x, y, w) = P_c (X_i, 1), pixel (u, v) = (x / w, y / w).  The view is VISIBLE iff w > 0 and
+ * -0.5 <= u < width_c - 0.5 and -0.5 <= v < height_c - 0.5 (the pixel areas of the integer pixels 0..width-1, 0..height-1).
+ * xy: [n_cams][cam_stride] pixel pairs (same layout and formats as tri_triangulate_points' input); visible views get
+ * (u, v) (TRI_PIX_U16: rounded half to even), invisible ones the missing marker ((-1,-1), or 0xFFFF pairs for U16).
+ * mask[i]: bit c <=> visible.  A point with a non-finite coordinate is visible nowhere.
+ * Rows are written for all n_cams cameras of the engine; xyz_f32 / xyz_f64 is packed [n_points][3] (the batch calls'
+ * point outputs feed straight back in).  FP64 on the cameraPerspectiveMatrix, TRI_F32 on the FP32 centred rig.
+ * Flags: TRI_F32, TRI_PIX_F64, TRI_PIX_U16; anything else, F64 together with U16, not exactly one of xyz_f32 / xyz_f64,
+ * or neither xy nor mask (when n_points > 0), or TRI_PIX_U16 with a camera wider or taller than 65535 returns
+ * TRI_ERR_ARG; cam_stride < n_points returns TRI_ERR_DIM; n_points == 0 does nothing.  No data-dependent error.
+ * The host call, the device call and every kernel path return bit-identical pixels and masks for the same point. */
+int tri_project_points(tri_engine* e, unsigned flags, const float* xyz_f32, const double* xyz_f64, int64_t n_points,
+                       void* xy, int64_t cam_stride, uint32_t* mask);            /* HOST buffers, chunked */
+int tri_project_points_device(tri_engine* e, unsigned flags, const float* d_xyz_f32, const double* d_xyz_f64,
+                              int64_t n_points, void* d_xy, int64_t cam_stride, uint32_t* d_mask, void* stream);
+
 /* The same batch sharded over several engines (one per GPU of the box) from ONE host process: frames
  * are independent, so engine g takes the contiguous range [g*N/G, (g+1)*N/G) and the shards run
  * concurrently (one host thread and one copy/compute pipeline per GPU); results land in the caller's
