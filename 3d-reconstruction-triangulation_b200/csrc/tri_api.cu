@@ -134,8 +134,7 @@ static cudaError_t upload_ray_table(RayFold<T>& f, int n_cams) {
 
 // DltRig<T>::absent (host copy): per group of 8 cameras and per 8-bit set m, what the cameras of m add to the normal
 // equations at the canonical pixel (x = y = 0 relative to the rig's pixel origin: rows P[r,0:3], rhs -P[r,3]), accumulated
-// in camera order with the kernels' own fma sequence (acc_row, tri_matrix.cu).
-static inline float fma_h(float a, float b, float c) { return fmaf(a, b, c); }
+// in camera order with the kernels' own function (dlt_view of an absent view).
 template <typename T>
 static std::vector<T> dlt_absent_table(const DltRig<T>& r, int n_cams) {
   const int groups = (n_cams + 7) / 8;
@@ -143,16 +142,8 @@ static std::vector<T> dlt_absent_table(const DltRig<T>& r, int n_cams) {
   for (int g = 0; g < groups; g++)
     for (int m = 0; m < 256; m++) {
       T M[6] = {0, 0, 0, 0, 0, 0}, v[3] = {0, 0, 0};
-      for (int k = 0; k < 8 && 8 * g + k < n_cams; k++) {
-        if (!(m >> k & 1)) continue;
-        const T* P = r.P[8 * g + k];
-        for (int row = 0; row < 2; row++) {
-          const T a0 = P[4 * row], a1 = P[4 * row + 1], a2 = P[4 * row + 2], b = -P[4 * row + 3];
-          M[0] = fma_h(a0, a0, M[0]); M[1] = fma_h(a0, a1, M[1]); M[2] = fma_h(a0, a2, M[2]); v[0] = fma_h(a0, b, v[0]);
-          M[3] = fma_h(a1, a1, M[3]); M[4] = fma_h(a1, a2, M[4]); v[1] = fma_h(a1, b, v[1]);
-          M[5] = fma_h(a2, a2, M[5]); v[2] = fma_h(a2, b, v[2]);
-        }
-      }
+      for (int k = 0; k < 8 && 8 * g + k < n_cams; k++)
+        if (m >> k & 1) dlt_view<MASK_TABLE>(r.P[8 * g + k], T(0), T(0), false, M, v);
       T* row = &tab[((size_t)g * 256 + m) * DLT_TABLE_ROW];
       for (int k = 0; k < 6; k++) row[k] = M[k];
       for (int k = 0; k < 3; k++) row[6 + k] = v[k];

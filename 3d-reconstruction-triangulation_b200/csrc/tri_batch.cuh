@@ -45,16 +45,16 @@ __device__ __forceinline__ View2<T> fetch2(const char* row, int64_t pair) {
     r.x0 = (T)a.x; r.y0 = (T)a.y; r.x1 = (T)b.x; r.y1 = (T)b.y;
   } else {
     uint2 q = ld_stream(reinterpret_cast<const uint2*>(row) + pair);
-    r.v0 = q.x != 0xffffffffu;
-    r.v1 = q.y != 0xffffffffu;
+    r.v0 = pix_valid(q.x);
+    r.v1 = pix_valid(q.y);
     if constexpr (sizeof(T) == 8) {  // integers < 2^16 -> double without touching the conversion pipe
       const double magic = 4503599627370496.0;  // 2^52
-      r.x0 = __hiloint2double(0x43300000, (int)(q.x & 0xffffu)) - magic;
-      r.y0 = __hiloint2double(0x43300000, (int)(q.x >> 16)) - magic;
-      r.x1 = __hiloint2double(0x43300000, (int)(q.y & 0xffffu)) - magic;
-      r.y1 = __hiloint2double(0x43300000, (int)(q.y >> 16)) - magic;
+      r.x0 = __hiloint2double(0x43300000, (int)u16_x(q.x)) - magic;
+      r.y0 = __hiloint2double(0x43300000, (int)u16_y(q.x)) - magic;
+      r.x1 = __hiloint2double(0x43300000, (int)u16_x(q.y)) - magic;
+      r.y1 = __hiloint2double(0x43300000, (int)u16_y(q.y)) - magic;
     } else {
-      r.x0 = (T)(q.x & 0xffffu); r.y0 = (T)(q.x >> 16); r.x1 = (T)(q.y & 0xffffu); r.y1 = (T)(q.y >> 16);
+      r.x0 = (T)u16_x(q.x); r.y0 = (T)u16_y(q.x); r.x1 = (T)u16_x(q.y); r.y1 = (T)u16_y(q.y);
     }
   }
   return r;
@@ -70,7 +70,7 @@ __device__ __forceinline__ void fetch1(const char* row, int64_t f, T& x, T& y, b
     v = pix_valid(q.x, q.y); x = (T)q.x; y = (T)q.y;
   } else {
     unsigned q = ld_stream(reinterpret_cast<const unsigned*>(row) + f);
-    v = q != 0xffffffffu; x = (T)(q & 0xffffu); y = (T)(q >> 16);
+    v = pix_valid(q); x = (T)u16_x(q); y = (T)u16_y(q);
   }
 }
 

@@ -20,7 +20,7 @@ struct __align__(16) DltRig {
   T origin[3];              // world origin added back to the solution (0 for FP64)
   // device, [TRI_MAX_CAMS / 8][256][DLT_TABLE_ROW]: row (g, m) = what the cameras 8g + {bits of m} add to the normal
   // equations at the canonical pixel (the rig's pixel origin) -- absent views are accumulated there and this row is
-  // subtracted afterwards (tri_matrix.cu); built by the host with the kernels' own fma sequence.  FP32 rig only (null in
+  // subtracted afterwards (tri_matrix.cu); built by the host with the kernels' own dlt_view.  FP32 rig only (null in
   // the FP64 rig, whose kernels clear an absent view's coefficients instead)
   const T* absent;
   int n_use;  // pixel rows of this launch (set per launch)
@@ -70,6 +70,10 @@ __host__ __device__ inline int pix_bytes(int fmt) { return fmt == PIX_F32 ? 8 : 
 // The sentinel test of MatrixTriangulator.cpp:86 / RayTriangulator.cpp:66 on the stored type.
 __device__ __forceinline__ bool pix_valid(float x, float y) { return x != -1.0f && y != -1.0f; }
 __device__ __forceinline__ bool pix_valid(double x, double y) { return x != -1.0 && y != -1.0; }
+// ushort2 pixels, one 32-bit word each (x in the low half): (0xFFFF, 0xFFFF) marks "no detection"
+__device__ __forceinline__ bool pix_valid(unsigned q) { return q != 0xffffffffu; }
+__device__ __forceinline__ unsigned u16_x(unsigned q) { return q & 0xffffu; }
+__device__ __forceinline__ unsigned u16_y(unsigned q) { return q >> 16; }
 
 template <typename T> __device__ __forceinline__ T to_real(float v);
 template <> __device__ __forceinline__ float to_real<float>(float v) { return v; }
@@ -87,9 +91,10 @@ __device__ __forceinline__ unsigned ld_stream(const unsigned* p) { return __ldcs
 // cv::invert(DECOMP_SVD) X = pinv(A) b (MatrixTriangulator.cpp:53-54) to ~1e-15 relative in FP64.
 // Explicit fused multiply-adds everywhere below (and in the policies): the rounding sequence is then
 // fixed by the source, so every kernel variant (vector / scalar path, any camera-count template)
-// returns bit-identical points for the same frame.
-__device__ __forceinline__ double fma_(double a, double b, double c) { return fma(a, b, c); }
-__device__ __forceinline__ float fma_(float a, float b, float c) { return fmaf(a, b, c); }
+// returns bit-identical points for the same frame.  fma_ is also the host's correctly rounded fma, so the
+// host builds its tables with the kernels' own functions.
+__host__ __device__ __forceinline__ double fma_(double a, double b, double c) { return fma(a, b, c); }
+__host__ __device__ __forceinline__ float fma_(float a, float b, float c) { return fmaf(a, b, c); }
 __device__ __forceinline__ double mul_(double a, double b) { return __dmul_rn(a, b); }
 __device__ __forceinline__ float mul_(float a, float b) { return __fmul_rn(a, b); }
 
@@ -127,6 +132,59 @@ __device__ __forceinline__ void solve_sym3(const T M[6], const T v[3], T X[3]) {
   X[0] = mul_(fma_(c00, v[0], fma_(c01, v[1], mul_(c02, v[2]))), inv);
   X[1] = mul_(fma_(c01, v[0], fma_(c11, v[1], mul_(c12, v[2]))), inv);
   X[2] = mul_(fma_(c02, v[0], fma_(c12, v[1], mul_(c22, v[2]))), inv);
+}
+
+// ---- the DLT rows of one view (MatrixTriangulator.cpp:16-49), shared by every DLT kernel and the host's tables ----
+// One row (a, b) into the normal equations.
+template <typename T>
+__host__ __device__ __forceinline__ void acc_row(T a0, T a1, T a2, T b, T (&M)[6], T (&v)[3]) {
+  M[0] = fma_(a0, a0, M[0]); M[1] = fma_(a0, a1, M[1]); M[2] = fma_(a0, a2, M[2]); v[0] = fma_(a0, b, v[0]);
+  M[3] = fma_(a1, a1, M[3]); M[4] = fma_(a1, a2, M[4]); v[1] = fma_(a1, b, v[1]);
+  M[5] = fma_(a2, a2, M[5]); v[2] = fma_(a2, b, v[2]);
+}
+
+// How an absent view is kept out of the sums.
+//   MASK_TABLE      FP32: accumulate it at the canonical pixel (0, 0), subtract its constant contribution from a table afterwards
+//                   (DltRig::absent); a caller that passes valid views only (the robust solve) needs nothing else
+//   MASK_SELECT_HI  FP64: clear only the HIGH word of the three coefficients -- what is left is a denormal below 2^-1042
+//                   whose products with the other coefficients (< 2^40) vanish against the sums; half the selects
+// Measured on the FP64 kernel (100 M frames, profiles/r2_dlt_variants.log): table 1.96 ms, select of both words 1.90 ms,
+// high-word select 1.86 ms -- the kernel is bound by the FP64 pipe (time follows the count of FP64 instructions, 2.9 cycles
+// each), so the table's 18 extra DADD per frame pair cost more than the selects it removes from the other pipes.
+enum { MASK_TABLE = 0, MASK_SELECT_HI = 1 };
+__device__ __forceinline__ double mask_coeff(double a, bool ok) { return __hiloint2double(ok ? __double2hiint(a) : 0, __double2loint(a)); }
+
+// One view's two rows a = P[r,0:3] - u P[2,0:3], b = u P[2,3] - P[r,3] (u = x, then y; pixel relative to the rig's
+// pixel origin) into the normal equations.
+template <int MASKING, typename T>
+__host__ __device__ __forceinline__ void dlt_view(const T (&P)[12], T x, T y, bool valid, T (&M)[6], T (&v)[3]) {
+  if constexpr (MASKING == MASK_TABLE) { x = valid ? x : T(0); y = valid ? y : T(0); }  // the canonical pixel
+#ifdef __CUDA_ARCH__
+#pragma unroll
+#endif
+  for (int r = 0; r < 2; r++) {
+    const T u = r == 0 ? x : y;
+    T a0 = fma_(-u, P[8], P[4 * r]), a1 = fma_(-u, P[9], P[4 * r + 1]), a2 = fma_(-u, P[10], P[4 * r + 2]);
+    const T b = fma_(u, P[11], -P[4 * r + 3]);
+    if constexpr (MASKING == MASK_SELECT_HI) { a0 = mask_coeff(a0, valid); a1 = mask_coeff(a1, valid); a2 = mask_coeff(a2, valid); }
+    acc_row<T>(a0, a1, a2, b, M, v);
+  }
+}
+
+// Camera loop over a compile-time class: NC > 0 unrolls NC cameras (static camera indices: the constants are constant-bank
+// operands) and predicates off those >= n; NC = 0 is a rolled loop.  n is the same for the whole grid and every thread walks
+// the same cameras in the same order -- a frame's absent views are predicated off by f, not skipped -- so the rig index is
+// warp-uniform (a divergent index would serialise the constant-bank reads).
+template <int NC, class F>
+__device__ __forceinline__ void for_cams(int n, F&& f) {
+  if constexpr (NC > 0) {
+#pragma unroll
+    for (int c = 0; c < NC; c++)
+      if (c < n) f(c);
+  } else {
+#pragma unroll 1
+    for (int c = 0; c < n; c++) f(c);
+  }
 }
 
 }  // namespace tri

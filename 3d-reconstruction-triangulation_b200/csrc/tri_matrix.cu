@@ -11,7 +11,7 @@
 // the normal-equation solution; cond(A) <= ~5 on real rigs so nothing is lost (SURVEY.md F1).
 // HBM traffic per frame: 8 B x n_cams in, 12 B out.
 //
-// Absent views (round 2, FP32; FP64: MASK_SELECT_HI below): no select, predicate or branch sits in the FMA
+// Absent views (round 2, FP32; FP64: MASK_SELECT_HI, tri_common.cuh): no select, predicate or branch sits in the FMA
 // chain any more.  An absent view's pixel is replaced by a canonical one (the pixel origin of the rig) BEFORE
 // the conversion, every camera is accumulated unconditionally, and what the absent cameras added -- a constant
 // per camera at the canonical pixel -- is taken back after the camera loop from a 256-row table indexed by the
@@ -36,14 +36,6 @@ __device__ __forceinline__ void load12(const float (&src)[12], float (&P)[12]) {
   for (int k = 0; k < 3; k++) { const float4 q = v[k]; P[4 * k] = q.x; P[4 * k + 1] = q.y; P[4 * k + 2] = q.z; P[4 * k + 3] = q.w; }
 }
 
-// One row (a, b) into the normal equations.
-template <typename T>
-__device__ __forceinline__ void acc_row(T a0, T a1, T a2, T b, T (&M)[6], T (&v)[3]) {
-  M[0] = fma_(a0, a0, M[0]); M[1] = fma_(a0, a1, M[1]); M[2] = fma_(a0, a2, M[2]); v[0] = fma_(a0, b, v[0]);
-  M[3] = fma_(a1, a1, M[3]); M[4] = fma_(a1, a2, M[4]); v[1] = fma_(a1, b, v[1]);
-  M[5] = fma_(a2, a2, M[5]); v[2] = fma_(a2, b, v[2]);
-}
-
 // the absent-view table row of `mask` (validity bits of the cameras [8g, 8g+8) at bits 8g..): 10 T per row
 template <typename T>
 __device__ __forceinline__ const T* absent_row(const DltRig<T>& rig, uint32_t mask, int group, int n_in_group) {
@@ -56,15 +48,13 @@ __device__ __forceinline__ void sub_row(const float* row, float (&M)[6], float (
   M[0] -= t0.x; M[1] -= t0.y; M[2] -= t0.z; M[3] -= t0.w; M[4] -= t1.x; M[5] -= t1.y; v[0] -= t1.z; v[1] -= t1.w; v[2] -= t2.x;
 }
 
-// How an absent view is kept out of the sums.
-//   MASK_TABLE      FP32: accumulate it at the canonical pixel, subtract its constant contribution from a table afterwards
-//   MASK_SELECT_HI  FP64: clear only the HIGH word of the three coefficients -- what is left is a denormal below 2^-1042
-//                   whose products with the other coefficients (< 2^40) vanish against the sums; half the selects
-// Measured on the FP64 kernel (100 M frames, profiles/r2_dlt_variants.log): table 1.96 ms, select of both words 1.90 ms,
-// high-word select 1.86 ms -- the kernel is bound by the FP64 pipe (time follows the count of FP64 instructions, 2.9 cycles
-// each), so the table's 18 extra DADD per frame pair cost more than the selects it removes from the other pipes.
-enum { MASK_TABLE = 0, MASK_SELECT_HI = 1 };
-__device__ __forceinline__ double mask_coeff(double a, bool ok) { return __hiloint2double(ok ? __double2hiint(a) : 0, __double2loint(a)); }
+// |A X - b|^2 of one view's two rows (MatrixTriangulator.cpp:55-58), pixel relative to the rig's pixel origin
+template <typename T>
+__device__ __forceinline__ T dlt_residual(const T (&P)[12], T x, T y, const T (&X)[3]) {
+  const T e0 = fma_(fma_(-x, P[8], P[0]), X[0], fma_(fma_(-x, P[9], P[1]), X[1], fma_(fma_(-x, P[10], P[2]), X[2], -fma_(x, P[11], -P[3]))));
+  const T e1 = fma_(fma_(-y, P[8], P[4]), X[0], fma_(fma_(-y, P[9], P[5]), X[1], fma_(fma_(-y, P[10], P[6]), X[2], -fma_(y, P[11], -P[7]))));
+  return fma_(e0, e0, mul_(e1, e1));
+}
 
 template <typename T_, bool CENTRED, int MASKING>
 struct DltPolicy {
@@ -83,15 +73,7 @@ struct DltPolicy {
     T P[12];
     load12(rig.P[c], P);
     if constexpr (CENTRED) { x -= rig.pix0[c][0]; y -= rig.pix0[c][1]; }
-    if constexpr (MASKING == MASK_TABLE) { x = valid ? x : T(0); y = valid ? y : T(0); }  // the canonical pixel
-#pragma unroll
-    for (int r = 0; r < 2; r++) {
-      const T u = r == 0 ? x : y;
-      T a0 = fma_(-u, P[8], P[4 * r]), a1 = fma_(-u, P[9], P[4 * r + 1]), a2 = fma_(-u, P[10], P[4 * r + 2]);
-      const T b = fma_(u, P[11], -P[4 * r + 3]);
-      if constexpr (MASKING == MASK_SELECT_HI) { a0 = mask_coeff(a0, valid); a1 = mask_coeff(a1, valid); a2 = mask_coeff(a2, valid); }
-      acc_row<T>(a0, a1, a2, b, a.M, a.v);
-    }
+    dlt_view<MASKING>(P, x, y, valid, a.M, a.v);
   }
   static __device__ __forceinline__ void add_chunk(const Rig& rig, int c, T x, T y, bool valid, Acc& a) { add(rig, c, x, y, valid, a); }
   // take back what the absent cameras added (group g = cameras 8g .. 8g+7, in order), then the adjugate solve
@@ -105,9 +87,7 @@ struct DltPolicy {
   static __device__ __forceinline__ T residual(const Rig& rig, int c, T x, T y, const T (&X)[3]) {
     const T(&P)[12] = rig.P[c];
     if constexpr (CENTRED) { x -= rig.pix0[c][0]; y -= rig.pix0[c][1]; }
-    const T e0 = fma_(fma_(-x, P[8], P[0]), X[0], fma_(fma_(-x, P[9], P[1]), X[1], fma_(fma_(-x, P[10], P[2]), X[2], -fma_(x, P[11], -P[3]))));
-    const T e1 = fma_(fma_(-y, P[8], P[4]), X[0], fma_(fma_(-y, P[9], P[5]), X[1], fma_(fma_(-y, P[10], P[6]), X[2], -fma_(y, P[11], -P[7]))));
-    return fma_(e0, e0, mul_(e1, e1));
+    return dlt_residual<T>(P, x, y, X);
   }
   static __device__ __forceinline__ double error(T sum, int n) { return sqrt((double)sum / (double)(2 * n)); }
   static __device__ __forceinline__ void to_world(const Rig& rig, T (&X)[3]) {
@@ -132,28 +112,11 @@ struct DltTile64 {
     for (int c = 0; c < NC; c++) {
       double P[12];
       load12(rig.P[c], P);
-      double x[2], y[2];
-      bool ok[2];
-      if constexpr (PIX == PIX_F32) {
-        const Views<float, PIX, 2> q = decode<float, PIX, 2>(raw[c]);
-#pragma unroll
-        for (int j = 0; j < 2; j++) { ok[j] = q.v[j]; x[j] = (double)q.x[j]; y[j] = (double)q.y[j]; }
-      } else {
-        const Views<double, PIX, 2> q = decode<double, PIX, 2>(raw[c]);
-#pragma unroll
-        for (int j = 0; j < 2; j++) { ok[j] = q.v[j]; x[j] = q.x[j]; y[j] = q.y[j]; }
-      }
+      const Views<double, PIX, 2> q = decode<double, PIX, 2>(raw[c]);
 #pragma unroll
       for (int j = 0; j < 2; j++) {
-        mask[j] |= (ok[j] ? 1u : 0u) << c;
-#pragma unroll
-        for (int r = 0; r < 2; r++) {
-          const double u = r == 0 ? x[j] : y[j];
-          double a0 = fma_(-u, P[8], P[4 * r]), a1 = fma_(-u, P[9], P[4 * r + 1]), a2 = fma_(-u, P[10], P[4 * r + 2]);
-          const double b = fma_(u, P[11], -P[4 * r + 3]);
-          a0 = mask_coeff(a0, ok[j]); a1 = mask_coeff(a1, ok[j]); a2 = mask_coeff(a2, ok[j]);
-          acc_row<double>(a0, a1, a2, b, acc[j].M, acc[j].v);
-        }
+        mask[j] |= (q.v[j] ? 1u : 0u) << c;
+        dlt_view<MASK_SELECT_HI>(P, q.x[j], q.y[j], q.v[j], acc[j].M, acc[j].v);
       }
     }
 #pragma unroll
@@ -252,16 +215,13 @@ struct DltX2Tile {
 #pragma unroll
           for (int c = 0; c < NC; c++) {
             const Views<float, PIX, 2> q = decode<float, PIX, 2>(raw[c]);
-            if (q.v[j]) {
-              const float x = q.x[j] + rig.npix0[c][0].x, y = q.y[j] + rig.npix0[c][1].x;
-              const float e0 = fmaf(fmaf(x, rig.N[c][0].x, rig.A[c][0].x), Xr[j][0], fmaf(fmaf(x, rig.N[c][1].x, rig.A[c][1].x), Xr[j][1],
-                               fmaf(fmaf(x, rig.N[c][2].x, rig.A[c][2].x), Xr[j][2], -fmaf(x, rig.N[c][3].x, rig.A[c][3].x))));
-              const float e1 = fmaf(fmaf(y, rig.N[c][0].x, rig.A[c][4].x), Xr[j][0], fmaf(fmaf(y, rig.N[c][1].x, rig.A[c][5].x), Xr[j][1],
-                               fmaf(fmaf(y, rig.N[c][2].x, rig.A[c][6].x), Xr[j][2], -fmaf(y, rig.N[c][3].x, rig.A[c][7].x))));
-              e += fmaf(e0, e0, e1 * e1);
+            if (q.v[j]) {  // the rig's P back from the .x halves (negation is exact)
+              const float2 *A = rig.A[c], *N = rig.N[c];
+              const float P[12] = {A[0].x, A[1].x, A[2].x, -A[3].x, A[4].x, A[5].x, A[6].x, -A[7].x, -N[0].x, -N[1].x, -N[2].x, N[3].x};
+              e += dlt_residual<float>(P, q.x[j] + rig.npix0[c][0].x, q.y[j] + rig.npix0[c][1].x, Xr[j]);
             }
           }
-          err[j] = sqrt((double)e / (double)(2 * __popc(j == 0 ? mask0 : mask1)));
+          err[j] = DltPolicy<float, true, MASK_TABLE>::error(e, __popc(j == 0 ? mask0 : mask1));
         }
       }
       X[j][0] = ok ? Xr[j][0] + rig.origin[0] : 0.f; X[j][1] = ok ? Xr[j][1] + rig.origin[1] : 0.f; X[j][2] = ok ? Xr[j][2] + rig.origin[2] : 0.f;

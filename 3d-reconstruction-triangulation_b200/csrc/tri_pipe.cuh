@@ -35,10 +35,10 @@ __device__ __forceinline__ Views<T, PIX, FPT> decode(const typename RawPix<PIX, 
   } else if constexpr (PIX == PIX_F32 && FPT == 1) {
     r.v[0] = pix_valid(q.x, q.y); r.x[0] = to_real<T>(q.x); r.y[0] = to_real<T>(q.y);
   } else if constexpr (PIX == PIX_U16 && FPT == 2) {
-    r.v[0] = q.x != 0xffffffffu; r.v[1] = q.y != 0xffffffffu;
-    r.x[0] = (T)(q.x & 0xffffu); r.y[0] = (T)(q.x >> 16); r.x[1] = (T)(q.y & 0xffffu); r.y[1] = (T)(q.y >> 16);
+    r.v[0] = pix_valid(q.x); r.v[1] = pix_valid(q.y);
+    r.x[0] = (T)u16_x(q.x); r.y[0] = (T)u16_y(q.x); r.x[1] = (T)u16_x(q.y); r.y[1] = (T)u16_y(q.y);
   } else {
-    r.v[0] = q != 0xffffffffu; r.x[0] = (T)(q & 0xffffu); r.y[0] = (T)(q >> 16);
+    r.v[0] = pix_valid(q); r.x[0] = (T)u16_x(q); r.y[0] = (T)u16_y(q);
   }
   return r;
 }
@@ -92,14 +92,12 @@ struct MaskIsValidity<TS, std::void_t<decltype(TS::MASK_IS_VALIDITY)>> { static 
 // one warp's memory wait hides under another warp's FMAs.  The 12-byte points are transposed through a
 // per-warp shared tile (__syncwarp only) into coalesced 16-byte streaming stores.  (Measured against it in round
 // 1 and dropped: one tile per CTA with up-front vector loads, and a CTA-synchronous TMA ring -- profiles/r1_*.)
-__device__ __forceinline__ void cp_async16(void* smem_dst, const void* gmem_src) {
-  asm volatile("cp.async.cg.shared.global [%0], [%1], 16;" ::"r"(smem_u32(smem_dst)), "l"(gmem_src) : "memory");
-}
-__device__ __forceinline__ void cp_async8(void* smem_dst, const void* gmem_src) {
-  asm volatile("cp.async.ca.shared.global [%0], [%1], 8;" ::"r"(smem_u32(smem_dst)), "l"(gmem_src) : "memory");
-}
-__device__ __forceinline__ void cp_async4(void* smem_dst, const void* gmem_src) {
-  asm volatile("cp.async.ca.shared.global [%0], [%1], 4;" ::"r"(smem_u32(smem_dst)), "l"(gmem_src) : "memory");
+// one RawPix of RB bytes (16 bypasses L1, as only cp.async.cg allows)
+template <int RB>
+__device__ __forceinline__ void cp_async_raw(void* smem_dst, const void* gmem_src) {
+  if constexpr (RB == 16) asm volatile("cp.async.cg.shared.global [%0], [%1], 16;" ::"r"(smem_u32(smem_dst)), "l"(gmem_src) : "memory");
+  else if constexpr (RB == 8) asm volatile("cp.async.ca.shared.global [%0], [%1], 8;" ::"r"(smem_u32(smem_dst)), "l"(gmem_src) : "memory");
+  else asm volatile("cp.async.ca.shared.global [%0], [%1], 4;" ::"r"(smem_u32(smem_dst)), "l"(gmem_src) : "memory");
 }
 __device__ __forceinline__ void cp_async_commit() { asm volatile("cp.async.commit_group;" ::: "memory"); }
 template <int N>
@@ -130,6 +128,11 @@ __device__ __forceinline__ void store_wide(const BatchOut& out, int64_t f0, cons
   }
 }
 
+// dynamic shared memory of a streaming kernel: the ring [stages][cams][BATCH_THREADS] Raw, then the warps' transpose tiles
+constexpr int stream_smem(int stages, int cams, int raw_bytes, int fpt) {
+  return stages * cams * BATCH_THREADS * raw_bytes + (BATCH_THREADS / 32) * 32 * fpt * 12;
+}
+
 template <class TS, int NC, int PIX, int STAGES, int MINB, bool WIDE, bool LAZY = false>
 __global__ void __launch_bounds__(BATCH_THREADS, WIDE ? 1 : MINB)  // the wide instantiation keeps the pixels live for the error pass
 stream_kernel(const __grid_constant__ typename TS::Rig rig, const char* __restrict__ xy, int64_t row_bytes, int64_t n_tiles,
@@ -150,12 +153,7 @@ stream_kernel(const __grid_constant__ typename TS::Rig rig, const char* __restri
   auto prefetch = [&](int s, int64_t t) {
     const char* src = xy + (t * BATCH_THREADS + tid) * RB;
 #pragma unroll
-    for (int c = 0; c < NC; c++) {
-      Raw* dst = slots + (s * NC + c) * BATCH_THREADS + tid;
-      if constexpr (RB == 16) cp_async16(dst, src + c * row_bytes);
-      else if constexpr (RB == 8) cp_async8(dst, src + c * row_bytes);
-      else cp_async4(dst, src + c * row_bytes);
-    }
+    for (int c = 0; c < NC; c++) cp_async_raw<RB>(slots + (s * NC + c) * BATCH_THREADS + tid, src + c * row_bytes);
   };
 #pragma unroll
   for (int s = 0; s < STAGES; s++) {
@@ -224,30 +222,32 @@ static inline bool stream_aligned(const void* xy, int64_t row_bytes, int align, 
            ((uintptr_t)out.mask & 7) || ((uintptr_t)out.err & 15) || ((uintptr_t)out.iters & 7));
 }
 
+// A persistent streaming kernel: as many CTAs as fit on the SMs with `bytes` of dynamic shared memory, at most one per tile.
+template <class K, class... Args>
+static cudaError_t launch_persistent(const LaunchCtx& ctx, K kern, int bytes, int64_t n_tiles, const Args&... args) {
+  cudaError_t err = cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, bytes);
+  if (err != cudaSuccess) return err;
+  int per_sm = 1;
+  err = cudaOccupancyMaxActiveBlocksPerMultiprocessor(&per_sm, kern, BATCH_THREADS, bytes);
+  if (err != cudaSuccess) return err;
+  const int64_t grid = std::min<int64_t>(n_tiles, (int64_t)ctx.sm_count * std::max(per_sm, 1));
+  kern<<<(unsigned)grid, BATCH_THREADS, bytes, ctx.stream>>>(args...);
+  ++*ctx.launches;
+  return cudaGetLastError();
+}
+
 // LAZY: the pixels are read from the slot as the solve needs them (RawSrc) instead of pulled into registers on arrival
 template <class TS, int PIX, int STAGES, int MINB, bool WIDE, bool LAZY>
 static cudaError_t launch_stream_w(const LaunchCtx& ctx, const typename TS::Rig& rig, const char* xy, int n_use, int64_t n_tiles,
                                    int64_t row_bytes, const BatchOut& out, int opt) {
-  constexpr int FPT = TS::FPT;
-  using Raw = typename RawPix<PIX, FPT>::type;
-  cudaError_t err = cudaSuccess;
-#define TRI_CASE(N)                                                                                                     \
-  case N: {                                                                                                             \
-    auto kern = stream_kernel<TS, N, PIX, STAGES, MINB, WIDE, LAZY>;                                                    \
-    constexpr int bytes = STAGES * N * BATCH_THREADS * (int)sizeof(Raw) + (BATCH_THREADS / 32) * 32 * FPT * 12;          \
-    err = cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, bytes);                               \
-    if (err != cudaSuccess) return err;                                                                                 \
-    int per_sm = 1;                                                                                                     \
-    err = cudaOccupancyMaxActiveBlocksPerMultiprocessor(&per_sm, kern, BATCH_THREADS, bytes);                           \
-    if (err != cudaSuccess) return err;                                                                                 \
-    const int64_t grid = std::min<int64_t>(n_tiles, (int64_t)ctx.sm_count * std::max(per_sm, 1));                       \
-    kern<<<(unsigned)grid, BATCH_THREADS, bytes, ctx.stream>>>(rig, xy, row_bytes, n_tiles, out, opt, ctx.d_first_bad,  \
-                                                         ctx.frame_base);                                               \
-  } break;
+  constexpr int RB = (int)sizeof(typename RawPix<PIX, TS::FPT>::type);
+#define TRI_CASE(N)                                                                                                          \
+  case N:                                                                                                                    \
+    return launch_persistent(ctx, stream_kernel<TS, N, PIX, STAGES, MINB, WIDE, LAZY>, stream_smem(STAGES, N, RB, TS::FPT), \
+                             n_tiles, rig, xy, row_bytes, n_tiles, out, opt, ctx.d_first_bad, ctx.frame_base);
   switch (n_use) { TRI_CASE(2) TRI_CASE(3) TRI_CASE(4) TRI_CASE(5) TRI_CASE(6) TRI_CASE(7) TRI_CASE(8) }
 #undef TRI_CASE
-  ++*ctx.launches;
-  return cudaGetLastError();
+  return cudaErrorInvalidValue;  // launch_stream takes 2..8 cameras only
 }
 
 // Launch the streaming kernel on the full tiles of [0, n_frames); *covered = the number of frames it took
@@ -324,12 +324,7 @@ chunk_kernel(const __grid_constant__ typename S::Rig rig, const char* __restrict
     const char* src = xy + (t * BATCH_THREADS + tid) * RB + (int64_t)ch * CHUNK_CAMS * row_bytes;
 #pragma unroll
     for (int c = 0; c < CHUNK_CAMS; c++) {
-      if (ch * CHUNK_CAMS + c < n_use) {
-        Raw* dst = slots + (s * CHUNK_CAMS + c) * BATCH_THREADS + tid;
-        if constexpr (RB == 16) cp_async16(dst, src + c * row_bytes);
-        else if constexpr (RB == 8) cp_async8(dst, src + c * row_bytes);
-        else cp_async4(dst, src + c * row_bytes);
-      }
+      if (ch * CHUNK_CAMS + c < n_use) cp_async_raw<RB>(slots + (s * CHUNK_CAMS + c) * BATCH_THREADS + tid, src + c * row_bytes);
     }
   };
 #pragma unroll
@@ -418,22 +413,14 @@ static cudaError_t launch_chunk(const LaunchCtx& ctx, const typename S::Rig& rig
   if (n_tiles == 0 || n_use <= CHUNK_CAMS || n_use > 4 * CHUNK_CAMS) return cudaSuccess;
   if (out.err) return cudaSuccess;
   if (!stream_aligned(xy, row_bytes, (int)sizeof(Raw), out)) return cudaSuccess;
-  constexpr int bytes = STAGES * CHUNK_CAMS * BATCH_THREADS * (int)sizeof(Raw) + (BATCH_THREADS / 32) * 32 * FPT * 12;
-  auto go = [&](auto kern) -> cudaError_t {
-    cudaError_t err = cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, bytes);
-    if (err != cudaSuccess) return err;
-    int per_sm = 1;
-    err = cudaOccupancyMaxActiveBlocksPerMultiprocessor(&per_sm, kern, BATCH_THREADS, bytes);
-    if (err != cudaSuccess) return err;
-    const int64_t grid = std::min<int64_t>(n_tiles, (int64_t)ctx.sm_count * std::max(per_sm, 1));
-    kern<<<(unsigned)grid, BATCH_THREADS, bytes, ctx.stream>>>(rig, xy, row_bytes, n_tiles, n_use, out, opt, ctx.d_first_bad, ctx.frame_base);
-    return cudaGetLastError();
-  };
-  const cudaError_t err = wants_wide(out) ? go(chunk_kernel<S, PIX, FPT, STAGES, MINB, true>) : go(chunk_kernel<S, PIX, FPT, STAGES, MINB, false>);
-  if (err != cudaSuccess) return err;
-  ++*ctx.launches;
-  *covered = n_tiles * TILE;
-  return cudaSuccess;
+  constexpr int bytes = stream_smem(STAGES, CHUNK_CAMS, (int)sizeof(Raw), FPT);
+  const cudaError_t err =
+      wants_wide(out) ? launch_persistent(ctx, chunk_kernel<S, PIX, FPT, STAGES, MINB, true>, bytes, n_tiles, rig, xy, row_bytes, n_tiles,
+                                          n_use, out, opt, ctx.d_first_bad, ctx.frame_base)
+                      : launch_persistent(ctx, chunk_kernel<S, PIX, FPT, STAGES, MINB, false>, bytes, n_tiles, rig, xy, row_bytes, n_tiles,
+                                          n_use, out, opt, ctx.d_first_bad, ctx.frame_base);
+  if (err == cudaSuccess) *covered = n_tiles * TILE;
+  return err;
 }
 
 // Sub-range helper for the tail after the pipelined tiles.

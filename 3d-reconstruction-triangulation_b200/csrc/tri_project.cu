@@ -72,20 +72,6 @@ __device__ __forceinline__ void proj_store(char* row, int64_t i, bool vis, T u, 
   }
 }
 
-// Camera loop over a compile-time class: NC > 0 unrolls NC cameras and predicates off those >= n (n is the same for
-// the whole grid, so the branch is uniform); NC = 0 is a rolled loop for the rigs above the largest class.
-template <int NC, class F>
-__device__ __forceinline__ void proj_cams(int n, F&& f) {
-  if constexpr (NC > 0) {
-#pragma unroll
-    for (int c = 0; c < NC; c++)
-      if (c < n) f(c);
-  } else {
-#pragma unroll 1
-    for (int c = 0; c < n; c++) f(c);
-  }
-}
-
 // PPT points per thread, PROJ_THREADS apart (each camera's stores stay coalesced along the warp): the camera loop loads a
 // view's constants once for all of them.
 template <typename T, typename In, int PIX, int NC, bool PAIR, int PPT>
@@ -104,7 +90,7 @@ project_kernel(const __grid_constant__ ProjRig<T> rig, const In* __restrict__ xy
       fin[k] = live[k] && proj_load<T, In>(xyz, i0 + k * PROJ_THREADS, rig.d, X[k]);
       m[k] = 0;
     }
-    proj_cams<NC>(n_cams, [&](int c) {
+    for_cams<NC>(n_cams, [&](int c) {
 #pragma unroll
       for (int k = 0; k < PPT; k++) {
         T u, v;

@@ -20,6 +20,11 @@
 
 namespace tri {
 
+// a rig constant of one camera: the scalar of RayFold, or the low half of RayRigX2's pre-duplicated pair
+__device__ __forceinline__ float lo(float v) { return v; }
+__device__ __forceinline__ double lo(double v) { return v; }
+__device__ __forceinline__ float lo(float2 v) { return v.x; }
+
 template <typename T_>
 struct RayPolicy {
   using T = T_;
@@ -35,13 +40,14 @@ struct RayPolicy {
     T so[3] = {0, 0, 0};           // sum ob                   (LM start = mean of origins, :90-98)
     T tr = 0, ku = 0, kn = 0;      // k = kn - ku
   };
-  // u (unnormalised rotated ray) and 1/|v|^2 of one view
-  static __device__ __forceinline__ void ray(const Rig& r, int c, T x, T y, T (&u)[3], T& inv) {
-    u[0] = fma_(r.U0[c][0], x, fma_(r.U1[c][0], y, r.U2[c][0]));
-    u[1] = fma_(r.U0[c][1], x, fma_(r.U1[c][1], y, r.U2[c][1]));
-    u[2] = fma_(r.U0[c][2], x, fma_(r.U1[c][2], y, r.U2[c][2]));
-    const T vx = fma_(r.ax[c], x, r.bx[c]), vy = fma_(r.ay[c], y, r.by[c]);
-    inv = rcp_ray(fma_(vx, vx, fma_(vy, vy, r.dd[c])));
+  // u (unnormalised rotated ray) and 1/|v|^2 of one view; R = RayFold<T>, or RayRigX2 for RayPolicy<float>
+  template <class R>
+  static __device__ __forceinline__ void ray(const R& r, int c, T x, T y, T (&u)[3], T& inv) {
+    u[0] = fma_(lo(r.U0[c][0]), x, fma_(lo(r.U1[c][0]), y, lo(r.U2[c][0])));
+    u[1] = fma_(lo(r.U0[c][1]), x, fma_(lo(r.U1[c][1]), y, lo(r.U2[c][1])));
+    u[2] = fma_(lo(r.U0[c][2]), x, fma_(lo(r.U1[c][2]), y, lo(r.U2[c][2])));
+    const T vx = fma_(lo(r.ax[c]), x, lo(r.bx[c])), vy = fma_(lo(r.ay[c]), y, lo(r.by[c]));
+    inv = rcp_ray(fma_(vx, vx, fma_(vy, vy, lo(r.dd[c]))));
   }
   // the pixel-dependent terms of one view ...
   template <bool BRANCH = true>
@@ -141,10 +147,11 @@ struct RayPolicy {
     iters = it;
   }
   // r_i = |dir_i x (p - o_i)| (Triangulator.cpp:3-9); the reported error is the mean (RayTriangulator.cpp:26)
-  static __device__ __forceinline__ T residual(const Rig& r, int c, T x, T y, const T (&X)[3]) {
+  template <class R>
+  static __device__ __forceinline__ T residual(const R& r, int c, T x, T y, const T (&X)[3]) {
     T u[3], inv;
     ray(r, c, x, y, u, inv);
-    const T w0 = X[0] - r.ob[c][0], w1 = X[1] - r.ob[c][1], w2 = X[2] - r.ob[c][2];
+    const T w0 = X[0] - lo(r.ob[c][0]), w1 = X[1] - lo(r.ob[c][1]), w2 = X[2] - lo(r.ob[c][2]);
     const T c0 = fma_(u[1], w2, -mul_(u[2], w1)), c1 = fma_(u[2], w0, -mul_(u[0], w2)), c2 = fma_(u[0], w1, -mul_(u[1], w0));
     return sqrt(mul_(fma_(c0, c0, fma_(c1, c1, mul_(c2, c2))), inv));
   }
@@ -279,23 +286,14 @@ struct RayX2Tile {
       err[j] = 0;
       iters[j] = ok ? 1 : 0;
       if constexpr (WIDE) {
-        if (ok) {  // mean distance to the rays, the arithmetic of RayPolicy<float>::residual
+        if (ok) {  // mean distance to the rays
           float e = 0;
 #pragma unroll
           for (int c = 0; c < NC; c++) {
             const Views<float, PIX, 2> q = decode<float, PIX, 2>(raw[c]);
-            if (q.v[j]) {
-              const float x = q.x[j], y = q.y[j];
-              const float u0 = fmaf(r.U0[c][0].x, x, fmaf(r.U1[c][0].x, y, r.U2[c][0].x)), u1 = fmaf(r.U0[c][1].x, x, fmaf(r.U1[c][1].x, y, r.U2[c][1].x)),
-                          u2 = fmaf(r.U0[c][2].x, x, fmaf(r.U1[c][2].x, y, r.U2[c][2].x));
-              const float vx = fmaf(r.ax[c].x, x, r.bx[c].x), vy = fmaf(r.ay[c].x, y, r.by[c].x);
-              const float inv = rcp_ray(fmaf(vx, vx, fmaf(vy, vy, r.dd[c].x)));
-              const float w0 = Xr[j][0] - r.ob[c][0].x, w1 = Xr[j][1] - r.ob[c][1].x, w2 = Xr[j][2] - r.ob[c][2].x;
-              const float c0 = fmaf(u1, w2, -__fmul_rn(u2, w1)), c1 = fmaf(u2, w0, -__fmul_rn(u0, w2)), c2 = fmaf(u0, w1, -__fmul_rn(u1, w0));
-              e += sqrtf(__fmul_rn(fmaf(c0, c0, fmaf(c1, c1, __fmul_rn(c2, c2))), inv));
-            }
+            if (q.v[j]) e += RayPolicy<float>::residual(r, c, q.x[j], q.y[j], Xr[j]);
           }
-          err[j] = (double)e / (double)__popc(j == 0 ? mask0 : mask1);
+          err[j] = RayPolicy<float>::error(e, __popc(j == 0 ? mask0 : mask1));
         }
       }
       X[j][0] = ok ? Xr[j][0] + r.origin[0] : 0.f; X[j][1] = ok ? Xr[j][1] + r.origin[1] : 0.f; X[j][2] = ok ? Xr[j][2] + r.origin[2] : 0.f;

@@ -32,20 +32,6 @@ struct __align__(16) RobustRig {
   T tau2;  // max_reproj_px^2: r <= tau  <=>  r^2 <= tau^2
 };
 
-// one view's two DLT rows into the normal equations (the plain path's fma sequence, DltPolicy::add)
-template <typename T>
-__device__ __forceinline__ void robust_add(const T (&P)[12], T x, T y, T (&M)[6], T (&v)[3]) {
-#pragma unroll
-  for (int r = 0; r < 2; r++) {
-    const T u = r == 0 ? x : y;
-    const T a0 = fma_(-u, P[8], P[4 * r]), a1 = fma_(-u, P[9], P[4 * r + 1]), a2 = fma_(-u, P[10], P[4 * r + 2]);
-    const T b = fma_(u, P[11], -P[4 * r + 3]);
-    M[0] = fma_(a0, a0, M[0]); M[1] = fma_(a0, a1, M[1]); M[2] = fma_(a0, a2, M[2]); v[0] = fma_(a0, b, v[0]);
-    M[3] = fma_(a1, a1, M[3]); M[4] = fma_(a1, a2, M[4]); v[1] = fma_(a1, b, v[1]);
-    M[5] = fma_(a2, a2, M[5]); v[2] = fma_(a2, b, v[2]);
-  }
-}
-
 // projective depth w and squared pixel reprojection error r2 of X on a camera, pixel (x, y)
 template <typename T>
 __device__ __forceinline__ void robust_project(const T (&P)[12], const T (&X)[3], T x, T y, T& w, T& r2) {
@@ -56,32 +42,16 @@ __device__ __forceinline__ void robust_project(const T (&P)[12], const T (&X)[3]
   r2 = fma_(du, du, mul_(dv, dv));
 }
 
-// Camera loop of the consensus solve: unrolled over a compile-time count (static camera indices: the constants are
-// constant-bank operands), a plain loop otherwise.  Every thread of a warp walks the same cameras in the same order --
-// a frame's absent views are predicated off, not skipped -- so the rig index is warp-uniform (a divergent index would
-// serialise the constant-bank reads), and a warp costs what its busiest frame costs either way.
-template <int NC, class F>
-__device__ __forceinline__ void for_cams(int c0, int n, F&& f) {
-  if constexpr (NC > 0) {
-#pragma unroll
-    for (int c = 0; c < NC; c++)
-      if (c >= c0) f(c);
-  } else {
-#pragma unroll 1
-    for (int c = c0; c < n; c++) f(c);
-  }
-}
-
-// The consensus solve of one frame.  NC > 0: compile-time camera count; NC = 0: n cameras at run time.
-// pix(c, x, y) -> validity of camera c, (x, y) relative to the rig's pixel origin.  views = the number of valid views
-// (the too-few test of the plain path).
-template <typename T, int NC, class Pix>
+// The consensus solve of one frame over n cameras.  pix(c, x, y) -> validity of camera c, (x, y) relative to the rig's
+// pixel origin.  views = the number of valid views (the too-few test of the plain path).  The camera loops stay rolled
+// (for_cams<0>): unrolled over a compile-time count the compiler keeps every camera's constants and pixels live across the
+// pair loop (FP64 at 8 cameras: 255 registers and spills, against 64 registers rolled).
+template <typename T, class Pix>
 __device__ __forceinline__ void robust_frame(const RobustRig<T>& rig, int n, const Pix& pix, T (&X)[3], uint32_t& mask,
                                              double& err, int& views) {
   const DltRig<T>& d = rig.d;
-  if constexpr (NC > 0) n = NC;
   uint32_t V = 0;
-  for_cams<NC>(0, n, [&](int c) {
+  for_cams<0>(n, [&](int c) {
     T x, y;
     V |= (pix(c, x, y) ? 1u : 0u) << c;
   });
@@ -103,13 +73,13 @@ __device__ __forceinline__ void robust_frame(const RobustRig<T>& rig, int n, con
       T xj, yj;
       if (!pix(j, xj, yj)) continue;
       T M[6] = {0, 0, 0, 0, 0, 0}, v[3] = {0, 0, 0}, H[3];
-      robust_add<T>(d.P[i], xi, yi, M, v);
-      robust_add<T>(d.P[j], xj, yj, M, v);
+      dlt_view<MASK_TABLE>(d.P[i], xi, yi, true, M, v);
+      dlt_view<MASK_TABLE>(d.P[j], xj, yj, true, M, v);
       solve_sym3<T>(M, v, H);
       uint32_t I = 0;
       T s = 0;
       bool front = true;
-      for_cams<NC>(0, n, [&](int c) {
+      for_cams<0>(n, [&](int c) {
         T x, y, w, r2;
         if (!pix(c, x, y)) return;
         robust_project<T>(d.P[c], H, x, y, w, r2);
@@ -125,14 +95,14 @@ __device__ __forceinline__ void robust_frame(const RobustRig<T>& rig, int n, con
 
   // the refit: the DLT over the inliers only, in camera order
   T M[6] = {0, 0, 0, 0, 0, 0}, v[3] = {0, 0, 0};
-  for_cams<NC>(0, n, [&](int c) {
+  for_cams<0>(n, [&](int c) {
     T x, y;
     pix(c, x, y);
-    if (best_I >> c & 1) robust_add<T>(d.P[c], x, y, M, v);
+    if (best_I >> c & 1) dlt_view<MASK_TABLE>(d.P[c], x, y, true, M, v);
   });
   solve_sym3<T>(M, v, X);
   T s = 0;
-  for_cams<NC>(0, n, [&](int c) {
+  for_cams<0>(n, [&](int c) {
     T x, y, w, r2;
     pix(c, x, y);
     robust_project<T>(d.P[c], X, x, y, w, r2);
@@ -158,9 +128,7 @@ struct RobustTile {
       y = q.y[0] - rig.d.pix0[c][1];
       return q.v[0];
     };
-    // the camera loops stay rolled: unrolled over NC the compiler keeps every camera's constants and pixels live across
-    // the pair loop (FP64 at 8 cameras: 255 registers and spills, against 64 registers rolled)
-    robust_frame<T, 0>(rig, NC, pix, X[0], mask[0], err[0], iters[0]);
+    robust_frame<T>(rig, NC, pix, X[0], mask[0], err[0], iters[0]);
   }
 };
 
@@ -178,8 +146,8 @@ __device__ __forceinline__ bool robust_load(const char* xy, int64_t row_bytes, i
     return pix_valid(q.x, q.y);
   } else {
     const unsigned q = __ldg(reinterpret_cast<const unsigned*>(row) + f);
-    x = (T)(q & 0xffffu); y = (T)(q >> 16);
-    return q != 0xffffffffu;
+    x = (T)u16_x(q); y = (T)u16_y(q);
+    return pix_valid(q);
   }
 }
 
@@ -199,7 +167,7 @@ robust_kernel(const __grid_constant__ RobustRig<T> rig, const char* __restrict__
   uint32_t mask;
   double err;
   int views;
-  robust_frame<T, 0>(rig, n_use, pix, X, mask, err, views);
+  robust_frame<T>(rig, n_use, pix, X, mask, err, views);
   if (views < 2) atomicMin(first_bad, (unsigned long long)(frame_base + f));
   if (out.xyz_f32) { float* o = out.xyz_f32 + 3 * f; o[0] = (float)X[0]; o[1] = (float)X[1]; o[2] = (float)X[2]; }
   if (out.xyz_f64) { double* o = out.xyz_f64 + 3 * f; o[0] = X[0]; o[1] = X[1]; o[2] = X[2]; }
