@@ -6,7 +6,6 @@
 
 #include <algorithm>
 #include <string>
-#include <thread>
 #include <vector>
 
 #include "tri_engine.cuh"
@@ -14,7 +13,6 @@
 namespace tri {
 
 static thread_local std::string g_error;
-void set_error(const std::string& s) { g_error = s; }
 int fail(int status, const std::string& s) {
   g_error = s;
   return status;
@@ -23,11 +21,6 @@ int cuda_fail(cudaError_t err, const char* what) {
   g_error = std::string(what) + ": " + cudaGetErrorString(err);
   return TRI_ERR_CUDA;
 }
-#define TRI_CUDA(call)                                         \
-  do {                                                         \
-    cudaError_t err__ = (call);                                \
-    if (err__ != cudaSuccess) return cuda_fail(err__, #call);  \
-  } while (0)
 
 // ---- rig constants ---------------------------------------------------------------------------
 
@@ -243,26 +236,14 @@ static int launch_batch(tri_engine* e, const LaunchCtx& ctx, int mode, unsigned 
   return TRI_OK;
 }
 
-static int ensure(char** p, size_t* cap, size_t need) {
-  if (*cap >= need) return TRI_OK;
-  if (*p) cudaFree(*p);
-  *p = nullptr;
-  *cap = 0;
-  TRI_CUDA(cudaMalloc((void**)p, need));
-  *cap = need;
-  return TRI_OK;
-}
-
-static size_t align_up(size_t v, size_t a) { return (v + a - 1) / a * a; }
-
-// Device entry points without a single pixel row: every frame has too few views -- zero outputs, frame 0 latched.
-static int too_few_device(tri_engine* e, int64_t n_frames, const BatchOut& out, cudaStream_t stream) {
-  TRI_CUDA(cudaMemsetAsync(e->d_first_bad, 0, sizeof(unsigned long long), stream));
-  if (out.xyz_f32) TRI_CUDA(cudaMemsetAsync(out.xyz_f32, 0, sizeof(float) * 3 * n_frames, stream));
-  if (out.xyz_f64) TRI_CUDA(cudaMemsetAsync(out.xyz_f64, 0, sizeof(double) * 3 * n_frames, stream));
-  if (out.mask) TRI_CUDA(cudaMemsetAsync(out.mask, 0, sizeof(uint32_t) * n_frames, stream));
-  if (out.err) TRI_CUDA(cudaMemsetAsync(out.err, 0, sizeof(double) * n_frames, stream));
-  if (out.iters) TRI_CUDA(cudaMemsetAsync(out.iters, 0, sizeof(int32_t) * n_frames, stream));
+// A batch without a single pixel row: every frame has too few views -- zero outputs, frame 0 latched.
+static int too_few(const LaunchCtx& ctx, int64_t n_frames, const BatchOut& out) {
+  TRI_CUDA(cudaMemsetAsync(ctx.d_first_bad, 0, sizeof(unsigned long long), ctx.stream));
+  if (out.xyz_f32) TRI_CUDA(cudaMemsetAsync(out.xyz_f32, 0, sizeof(float) * 3 * n_frames, ctx.stream));
+  if (out.xyz_f64) TRI_CUDA(cudaMemsetAsync(out.xyz_f64, 0, sizeof(double) * 3 * n_frames, ctx.stream));
+  if (out.mask) TRI_CUDA(cudaMemsetAsync(out.mask, 0, sizeof(uint32_t) * n_frames, ctx.stream));
+  if (out.err) TRI_CUDA(cudaMemsetAsync(out.err, 0, sizeof(double) * n_frames, ctx.stream));
+  if (out.iters) TRI_CUDA(cudaMemsetAsync(out.iters, 0, sizeof(int32_t) * n_frames, ctx.stream));
   return TRI_OK;
 }
 
@@ -276,66 +257,106 @@ static int check_robust_args(tri_engine* e, unsigned flags, double max_reproj_px
   return check_batch_args(e, TRI_MATRIX, xy, n_point_cams, n_frames, cam_stride, out, n_use);
 }
 
-// Host-buffer batch: frames stream through N_SLOTS device staging slots, one CUDA stream each, so the
-// H2D copy of a chunk overlaps the kernel of the previous one and the D2H copy of the one before.
-// `launch(ctx, d_xy, n, cam_stride, out)` solves one chunk already on the device.
+// A host buffer of the staging pipeline: `rows` rows of items of `bytes` bytes, row r starting `r * stride` items after
+// `host`.  A null host is an absent buffer: it takes no slot space and is not copied.
+struct RowGroup {
+  void* host;
+  int rows;
+  size_t bytes;
+  int64_t stride;
+};
+// A group's rows in a staging slot: row r at d + r * pitch bytes (d is null for an absent group).
+struct SlotRows {
+  char* d;
+  size_t pitch;
+};
+
+// Host-buffer pipeline: items stream in chunks through N_SLOTS device staging slots, one CUDA stream each, so the H2D
+// copy of a chunk overlaps the kernel of the previous one and the D2H copy of the one before.  For the chunk of n items
+// from f0, on its slot's stream: the [f0, f0 + n) slice of every input row goes H2D, `launch(ctx, n, in, out)` runs on
+// the slot's rows, and the slice of every output row comes back D2H, each in the order the groups are listed.
 template <class Launch>
-static int run_host_pipeline(tri_engine* e, unsigned flags, int fmt, const void* xy, int n_use, int64_t n_frames, int64_t cam_stride,
-                             int64_t chunk, const tri_batch_out* out, int64_t* first_bad_frame, const char* too_few_msg, Launch launch) {
-  const size_t pb = pix_bytes(fmt);
-  if (n_frames <= chunk) chunk = (n_frames + 1) / 2 * 2;  // one chunk
-  const size_t in_row = align_up((size_t)chunk * pb, 256);
-  const size_t o_xyz32 = 0;
-  const size_t o_xyz64 = o_xyz32 + (out->xyz_f32 ? align_up((size_t)chunk * 12, 256) : 0);
-  const size_t o_mask = o_xyz64 + (out->xyz_f64 ? align_up((size_t)chunk * 24, 256) : 0);
-  const size_t o_err = o_mask + (out->mask ? align_up((size_t)chunk * 4, 256) : 0);
-  const size_t o_iters = o_err + (out->err ? align_up((size_t)chunk * 8, 256) : 0);
-  const size_t out_bytes = o_iters + (out->iters ? align_up((size_t)chunk * 4, 256) : 0);
-  const int n_slots = n_frames > chunk ? N_SLOTS : 1;
-  int st;
-  for (int i = 0; i < n_slots; i++) {
-    if ((st = ensure(&e->slots[i].d_in, &e->slots[i].in_cap, in_row * std::max(n_use, 1))) != TRI_OK) return st;
-    if ((st = ensure(&e->slots[i].d_out, &e->slots[i].out_cap, out_bytes)) != TRI_OK) return st;
-  }
-  unsigned long long* latch = e->d_first_bad + 1;  // the host path's own latch: a pending one of the device entry point stays
-  TRI_CUDA(cudaMemsetAsync(latch, 0xff, sizeof(unsigned long long), e->slots[0].stream));
-  TRI_CUDA(cudaStreamSynchronize(e->slots[0].stream));
-  const char* src = static_cast<const char*>(xy);
+static int run_staged(tri_engine* e, int64_t n_items, int64_t chunk, const std::vector<RowGroup>& in,
+                      const std::vector<RowGroup>& out, Launch launch) {
+  const int n_slots = n_items > chunk ? N_SLOTS : 1;
+  // slot buffers: the present groups back to back, every row at a 256-byte aligned offset
+  auto pitch = [&](const RowGroup& g) { return up256((size_t)chunk * g.bytes); };
+  auto bytes = [&](const std::vector<RowGroup>& groups) {
+    size_t b = 0;
+    for (const RowGroup& g : groups) b += g.host ? g.rows * pitch(g) : 0;
+    return b;
+  };
+  auto place = [&](const std::vector<RowGroup>& groups, DevBuf& buf) {
+    std::vector<SlotRows> rows;
+    char* p = buf.as<char>();
+    for (const RowGroup& g : groups) {
+      rows.push_back({g.host ? p : nullptr, pitch(g)});
+      if (g.host) p += g.rows * pitch(g);
+    }
+    return rows;
+  };
+  auto copy = [&](const std::vector<RowGroup>& groups, const std::vector<SlotRows>& rows, int64_t f0, int64_t n, bool h2d,
+                  cudaStream_t stream) -> int {
+    for (size_t i = 0; i < groups.size(); i++)
+      for (int r = 0; rows[i].d && r < groups[i].rows; r++) {
+        char* h = static_cast<char*>(groups[i].host) + (r * groups[i].stride + f0) * groups[i].bytes;
+        char* d = rows[i].d + r * rows[i].pitch;
+        TRI_CUDA(cudaMemcpyAsync(h2d ? d : h, h2d ? h : d, (size_t)n * groups[i].bytes,
+                                 h2d ? cudaMemcpyHostToDevice : cudaMemcpyDeviceToHost, stream));
+      }
+    return TRI_OK;
+  };
   // the chunk loop; on any failure the copies already queued into the caller's buffers are drained before returning
   auto run = [&]() -> int {
-    int k = 0;
-    for (int64_t f0 = 0; f0 < n_frames; f0 += chunk, k++) {
+    for (int i = 0; i < n_slots; i++) {
+      TRI_CUDA(e->slots[i].in.alloc(bytes(in)));
+      TRI_CUDA(e->slots[i].out.alloc(bytes(out)));
+    }
+    int k = 0, st;
+    for (int64_t f0 = 0; f0 < n_items; f0 += chunk, k++) {
       Slot& s = e->slots[k % n_slots];
-      const int64_t n = std::min(chunk, n_frames - f0);
+      const int64_t n = std::min(chunk, n_items - f0);
+      const std::vector<SlotRows> d_in = place(in, s.in), d_out = place(out, s.out);
       TRI_CUDA(cudaStreamSynchronize(s.stream));  // slot free (its previous D2H has landed)
-      for (int c = 0; c < n_use; c++)
-        TRI_CUDA(cudaMemcpyAsync(s.d_in + (size_t)c * in_row, src + ((size_t)c * cam_stride + f0) * pb, (size_t)n * pb,
-                                 cudaMemcpyHostToDevice, s.stream));
-      BatchOut o{out->xyz_f32 ? (float*)(s.d_out + o_xyz32) : nullptr, out->xyz_f64 ? (double*)(s.d_out + o_xyz64) : nullptr,
-                 out->mask ? (uint32_t*)(s.d_out + o_mask) : nullptr, out->err ? (double*)(s.d_out + o_err) : nullptr,
-                 out->iters ? (int32_t*)(s.d_out + o_iters) : nullptr};
-      if (n_use == 0) {
-        TRI_CUDA(cudaMemsetAsync(s.d_out, 0, out_bytes, s.stream));
-        TRI_CUDA(cudaMemsetAsync(latch, 0, sizeof(unsigned long long), s.stream));
-      } else {
-        const int st2 = launch(e->ctx(s.stream, f0, true), (const void*)s.d_in, n, (int64_t)(in_row / pb), o);
-        if (st2 != TRI_OK) return st2;
-      }
-      if (out->xyz_f32) TRI_CUDA(cudaMemcpyAsync(out->xyz_f32 + 3 * f0, o.xyz_f32, (size_t)n * 12, cudaMemcpyDeviceToHost, s.stream));
-      if (out->xyz_f64) TRI_CUDA(cudaMemcpyAsync(out->xyz_f64 + 3 * f0, o.xyz_f64, (size_t)n * 24, cudaMemcpyDeviceToHost, s.stream));
-      if (out->mask) TRI_CUDA(cudaMemcpyAsync(out->mask + f0, o.mask, (size_t)n * 4, cudaMemcpyDeviceToHost, s.stream));
-      if (out->err) TRI_CUDA(cudaMemcpyAsync(out->err + f0, o.err, (size_t)n * 8, cudaMemcpyDeviceToHost, s.stream));
-      if (out->iters) TRI_CUDA(cudaMemcpyAsync(out->iters + f0, o.iters, (size_t)n * 4, cudaMemcpyDeviceToHost, s.stream));
+      if ((st = copy(in, d_in, f0, n, true, s.stream)) != TRI_OK) return st;
+      if ((st = launch(e->ctx(s.stream, f0, true), n, d_in.data(), d_out.data())) != TRI_OK) return st;
+      if ((st = copy(out, d_out, f0, n, false, s.stream)) != TRI_OK) return st;
     }
     for (int i = 0; i < n_slots; i++) TRI_CUDA(cudaStreamSynchronize(e->slots[i].stream));
     return TRI_OK;
   };
-  if ((st = run()) != TRI_OK) {
+  const int st = run();
+  if (st != TRI_OK) {
     const std::string why = g_error;
     for (int i = 0; i < n_slots; i++) cudaStreamSynchronize(e->slots[i].stream);  // nothing is left in flight into the caller's memory
-    cudaMemset(latch, 0xff, sizeof(unsigned long long));
     cudaGetLastError();
     return fail(st, why);
+  }
+  return TRI_OK;
+}
+
+// Host-buffer batch (plain or robust): the pixel rows in, the outputs asked for back, through the staging pipeline.
+// `launch(ctx, d_xy, n, cam_stride, out)` solves one chunk already on the device.
+template <class Launch>
+static int run_batch_host(tri_engine* e, unsigned flags, int fmt, const void* xy, int n_use, int64_t n_frames, int64_t cam_stride,
+                          int64_t chunk, const tri_batch_out* out, int64_t* first_bad_frame, const char* too_few_msg, Launch launch) {
+  const size_t pb = pix_bytes(fmt);
+  if (n_frames <= chunk) chunk = (n_frames + 1) / 2 * 2;  // one chunk
+  unsigned long long* latch = e->d_first_bad + 1;  // the host path's own latch: a pending one of the device entry point stays
+  TRI_CUDA(cudaMemsetAsync(latch, 0xff, sizeof(unsigned long long), e->slots[0].stream));
+  TRI_CUDA(cudaStreamSynchronize(e->slots[0].stream));
+  const int st = run_staged(
+      e, n_frames, chunk, {{const_cast<void*>(xy), n_use, pb, cam_stride}},
+      {{out->xyz_f32, 1, 12, 0}, {out->xyz_f64, 1, 24, 0}, {out->mask, 1, 4, 0}, {out->err, 1, 8, 0}, {out->iters, 1, 4, 0}},
+      [&](const LaunchCtx& ctx, int64_t n, const SlotRows* d_in, const SlotRows* d_out) {
+        const BatchOut o{(float*)d_out[0].d, (double*)d_out[1].d, (uint32_t*)d_out[2].d, (double*)d_out[3].d, (int32_t*)d_out[4].d};
+        if (n_use == 0) return too_few(ctx, n, o);
+        return launch(ctx, (const void*)d_in[0].d, n, (int64_t)(d_in[0].pitch / pb), o);
+      });
+  if (st != TRI_OK) {
+    cudaMemset(latch, 0xff, sizeof(unsigned long long));
+    cudaGetLastError();
+    return st;
   }
   unsigned long long v = 0;
   TRI_CUDA(cudaMemcpy(&v, latch, sizeof(v), cudaMemcpyDeviceToHost));
@@ -363,58 +384,6 @@ static int check_project_args(tri_engine* e, unsigned flags, const float* xyz_f3
     for (int c = 0; c < e->n_cams; c++)
       if (e->cams[c].width > 65535 || e->cams[c].height > 65535)
         return fail(TRI_ERR_ARG, "TRI_PIX_U16: a camera is larger than 65535 pixels, its pixels could collide with the missing marker");
-  return TRI_OK;
-}
-
-// Host-buffer projection: the batch pipeline with the copy directions swapped.  Points go H2D chunk by chunk through
-// the N_SLOTS staging slots, the kernel writes the chunk's pixel rows and masks into the slot, and one D2H copy per
-// camera row (plus one for the masks) lands them in the caller's cam_stride-strided rows.
-static int run_project_pipeline(tri_engine* e, bool f32, int fmt, const float* xyz_f32, const double* xyz_f64, int64_t n_points,
-                                void* xy, int64_t cam_stride, uint32_t* mask) {
-  const size_t pb = pix_bytes(fmt), in_pp = xyz_f32 ? 12 : 24;
-  const int nc = e->n_cams;
-  // ~64 MB of output rows per slot: large enough for full-rate copies, small enough to pipeline
-  const size_t out_pp = (xy ? nc * pb : 0) + (mask ? 4 : 0);
-  int64_t chunk = std::min<int64_t>(std::max<int64_t>((int64_t)((64u << 20) / out_pp) / 256 * 256, 1 << 16), 4 << 20);
-  if (n_points <= chunk) chunk = n_points;
-  const size_t row = align_up((size_t)chunk * pb, 256);
-  const size_t o_mask = xy ? row * nc : 0;
-  const size_t out_bytes = o_mask + (mask ? align_up((size_t)chunk * 4, 256) : 0);
-  const int n_slots = n_points > chunk ? N_SLOTS : 1;
-  int st;
-  for (int i = 0; i < n_slots; i++) {
-    if ((st = ensure(&e->slots[i].d_in, &e->slots[i].in_cap, align_up((size_t)chunk * in_pp, 256))) != TRI_OK) return st;
-    if ((st = ensure(&e->slots[i].d_out, &e->slots[i].out_cap, out_bytes)) != TRI_OK) return st;
-  }
-  const char* src = xyz_f32 ? (const char*)xyz_f32 : (const char*)xyz_f64;
-  char* dst = static_cast<char*>(xy);
-  auto run = [&]() -> int {
-    int k = 0;
-    for (int64_t p0 = 0; p0 < n_points; p0 += chunk, k++) {
-      Slot& s = e->slots[k % n_slots];
-      const int64_t n = std::min(chunk, n_points - p0);
-      TRI_CUDA(cudaStreamSynchronize(s.stream));  // slot free (its previous D2H has landed)
-      TRI_CUDA(cudaMemcpyAsync(s.d_in, src + (size_t)p0 * in_pp, (size_t)n * in_pp, cudaMemcpyHostToDevice, s.stream));
-      uint32_t* d_mask = mask ? (uint32_t*)(s.d_out + o_mask) : nullptr;
-      const cudaError_t err = launch_project(e->ctx(s.stream, p0, true), f32, fmt, e->rig64, e->rig32, e->cams, nc,
-                                             xyz_f32 ? (const float*)s.d_in : nullptr, xyz_f64 ? (const double*)s.d_in : nullptr, n,
-                                             xy ? s.d_out : nullptr, (int64_t)(row / pb), d_mask);
-      if (err != cudaSuccess) return cuda_fail(err, "kernel launch");
-      if (xy)
-        for (int c = 0; c < nc; c++)
-          TRI_CUDA(cudaMemcpyAsync(dst + ((size_t)c * cam_stride + p0) * pb, s.d_out + (size_t)c * row, (size_t)n * pb,
-                                   cudaMemcpyDeviceToHost, s.stream));
-      if (mask) TRI_CUDA(cudaMemcpyAsync(mask + p0, d_mask, (size_t)n * 4, cudaMemcpyDeviceToHost, s.stream));
-    }
-    for (int i = 0; i < n_slots; i++) TRI_CUDA(cudaStreamSynchronize(e->slots[i].stream));
-    return TRI_OK;
-  };
-  if ((st = run()) != TRI_OK) {
-    const std::string why = g_error;
-    for (int i = 0; i < n_slots; i++) cudaStreamSynchronize(e->slots[i].stream);  // nothing is left in flight into the caller's memory
-    cudaGetLastError();
-    return fail(st, why);
-  }
   return TRI_OK;
 }
 
@@ -475,19 +444,15 @@ void tri_destroy(tri_engine* e) {
   if (!e) return;
   DeviceGuard g(e->device);
   cudaDeviceSynchronize();
-  for (int i = 0; i < N_SLOTS; i++) {
-    if (e->slots[i].d_in) cudaFree(e->slots[i].d_in);
-    if (e->slots[i].d_out) cudaFree(e->slots[i].d_out);
+  for (int i = 0; i < N_SLOTS; i++)
     if (e->slots[i].stream) cudaStreamDestroy(e->slots[i].stream);
-  }
   if (e->cls_work && e->cls_work_free) e->cls_work_free(e->cls_work);
-  if (e->d_scratch) cudaFree(e->d_scratch);
   if (e->stream) cudaStreamDestroy(e->stream);
   if (e->d_first_bad) cudaFree(e->d_first_bad);
   if (e->rig32.absent) cudaFree(const_cast<float*>(e->rig32.absent));
   if (e->fold64.mask_table) cudaFree(const_cast<double*>(e->fold64.mask_table));
   if (e->fold32.mask_table) cudaFree(const_cast<float*>(e->fold32.mask_table));
-  delete e;
+  delete e;  // the DevBuf members free the staging slots and the scratch
 }
 
 int tri_engine_device(const tri_engine* e) { return e ? e->device : -1; }
@@ -503,7 +468,7 @@ int tri_triangulate_points_device(tri_engine* e, int mode, unsigned flags, const
   if (n_frames == 0) return TRI_OK;
   DeviceGuard g(e->device);
   BatchOut out{d_out->xyz_f32, d_out->xyz_f64, d_out->mask, d_out->err, d_out->iters};
-  if (n_use == 0) return too_few_device(e, n_frames, out, (cudaStream_t)stream);
+  if (n_use == 0) return too_few(e->ctx((cudaStream_t)stream), n_frames, out);
   return launch_batch(e, e->ctx((cudaStream_t)stream), mode, flags, fmt, d_xy, n_use, n_frames, cam_stride, out);
 }
 
@@ -580,11 +545,11 @@ int tri_triangulate_points(tri_engine* e, int mode, unsigned flags, const void* 
   // chunk: large enough to run the copy engines at full rate, small enough to pipeline
   int64_t chunk = n_frames >= (16 << 20) ? (4 << 20) : (1 << 20);  // measured: 4 Mi-frame chunks run PCIe at 63 GB/s, 1 Mi at 60.6
   if (mode == TRI_RAY && (flags & TRI_RAY_REFERENCE_LM)) chunk = 1 << 18;
-  return run_host_pipeline(e, flags, fmt, xy, n_use, n_frames, cam_stride, chunk, out, first_bad_frame,
-                           mode == TRI_MATRIX ? "Too few rays are found" : "Too few detections are found",
-                           [&](const LaunchCtx& ctx, const void* d_in, int64_t n, int64_t stride, const BatchOut& o) {
-                             return launch_batch(e, ctx, mode, flags, fmt, d_in, n_use, n, stride, o);
-                           });
+  return run_batch_host(e, flags, fmt, xy, n_use, n_frames, cam_stride, chunk, out, first_bad_frame,
+                        mode == TRI_MATRIX ? "Too few rays are found" : "Too few detections are found",
+                        [&](const LaunchCtx& ctx, const void* d_in, int64_t n, int64_t stride, const BatchOut& o) {
+                          return launch_batch(e, ctx, mode, flags, fmt, d_in, n_use, n, stride, o);
+                        });
 }
 
 int tri_triangulate_points_robust_device(tri_engine* e, unsigned flags, double max_reproj_px, const void* d_xy, int n_point_cams,
@@ -596,7 +561,7 @@ int tri_triangulate_points_robust_device(tri_engine* e, unsigned flags, double m
   if (n_frames == 0) return TRI_OK;
   DeviceGuard g(e->device);
   BatchOut out{d_out->xyz_f32, d_out->xyz_f64, d_out->mask, d_out->err, nullptr};
-  if (n_use == 0) return too_few_device(e, n_frames, out, (cudaStream_t)stream);
+  if (n_use == 0) return too_few(e->ctx((cudaStream_t)stream), n_frames, out);
   const cudaError_t err = launch_robust(e->ctx((cudaStream_t)stream), (flags & TRI_F32) != 0, fmt, e->rig64, e->rig32, max_reproj_px,
                                         d_xy, n_use, n_frames, cam_stride, out);
   return err == cudaSuccess ? TRI_OK : cuda_fail(err, "kernel launch");
@@ -612,13 +577,13 @@ int tri_triangulate_points_robust(tri_engine* e, unsigned flags, double max_repr
   if (n_frames == 0) return TRI_OK;
   DeviceGuard g(e->device);
   // the solve is compute-bound (pairs x views per frame), so the copies hide under it at the plain path's 1 Mi-frame chunk
-  return run_host_pipeline(e, flags, fmt, xy, n_use, n_frames, cam_stride, (int64_t)1 << 20, out, first_bad_frame,
-                           "Too few rays are found",
-                           [&](const LaunchCtx& ctx, const void* d_in, int64_t n, int64_t stride, const BatchOut& o) {
-                             const cudaError_t err = launch_robust(ctx, (flags & TRI_F32) != 0, fmt, e->rig64, e->rig32, max_reproj_px,
-                                                                   d_in, n_use, n, stride, o);
-                             return err == cudaSuccess ? TRI_OK : cuda_fail(err, "kernel launch");
-                           });
+  return run_batch_host(e, flags, fmt, xy, n_use, n_frames, cam_stride, (int64_t)1 << 20, out, first_bad_frame,
+                        "Too few rays are found",
+                        [&](const LaunchCtx& ctx, const void* d_in, int64_t n, int64_t stride, const BatchOut& o) {
+                          const cudaError_t err = launch_robust(ctx, (flags & TRI_F32) != 0, fmt, e->rig64, e->rig32, max_reproj_px,
+                                                                d_in, n_use, n, stride, o);
+                          return err == cudaSuccess ? TRI_OK : cuda_fail(err, "kernel launch");
+                        });
 }
 
 int tri_project_points_device(tri_engine* e, unsigned flags, const float* d_xyz_f32, const double* d_xyz_f64, int64_t n_points,
@@ -638,7 +603,21 @@ int tri_project_points(tri_engine* e, unsigned flags, const float* xyz_f32, cons
   const int st = check_project_args(e, flags, xyz_f32, xyz_f64, n_points, xy, cam_stride, mask, &fmt);
   if (st != TRI_OK || n_points == 0) return st;
   DeviceGuard g(e->device);
-  return run_project_pipeline(e, (flags & TRI_F32) != 0, fmt, xyz_f32, xyz_f64, n_points, xy, cam_stride, mask);
+  const size_t pb = pix_bytes(fmt), in_pp = xyz_f32 ? 12 : 24;
+  const int nc = e->n_cams;
+  // ~64 MB of output rows per slot: large enough for full-rate copies, small enough to pipeline
+  const size_t out_pp = (xy ? nc * pb : 0) + (mask ? 4 : 0);
+  int64_t chunk = std::min<int64_t>(std::max<int64_t>((int64_t)((64u << 20) / out_pp) / 256 * 256, 1 << 16), 4 << 20);
+  if (n_points <= chunk) chunk = n_points;
+  const void* xyz = xyz_f32 ? (const void*)xyz_f32 : (const void*)xyz_f64;
+  return run_staged(e, n_points, chunk, {{const_cast<void*>(xyz), 1, in_pp, 0}}, {{xy, nc, pb, cam_stride}, {mask, 1, 4, 0}},
+                    [&](const LaunchCtx& ctx, int64_t n, const SlotRows* d_in, const SlotRows* d_out) {
+                      const cudaError_t err = launch_project(ctx, (flags & TRI_F32) != 0, fmt, e->rig64, e->rig32, e->cams, nc,
+                                                             xyz_f32 ? (const float*)d_in[0].d : nullptr,
+                                                             xyz_f64 ? (const double*)d_in[0].d : nullptr, n, d_out[0].d,
+                                                             (int64_t)(d_out[0].pitch / pb), (uint32_t*)d_out[1].d);
+                      return err == cudaSuccess ? TRI_OK : cuda_fail(err, "kernel launch");
+                    });
 }
 
 int tri_triangulate_points_multi(tri_engine* const* engines, int n_engines, int mode, unsigned flags, const void* xy,
@@ -653,32 +632,25 @@ int tri_triangulate_points_multi(tri_engine* const* engines, int n_engines, int 
   if (st != TRI_OK) return st;
   if ((st = pix_format(flags, &fmt)) != TRI_OK) return st;
   const size_t pb = pix_bytes(fmt);
-  std::vector<int> status(n_engines, TRI_OK);
   std::vector<int64_t> bad(n_engines, -1);
-  std::vector<std::string> msg(n_engines);
-  std::vector<std::thread> workers;
   auto cut = [&](int g) {  // even boundaries keep every shard's rows vector-aligned
     int64_t b = n_frames * g / n_engines;
     return g >= n_engines ? n_frames : std::min<int64_t>(n_frames, b + (b & 1));
   };
-  for (int g = 0; g < n_engines; g++) {
-    workers.emplace_back([&, g]() {
-      const int64_t b = cut(g), e = cut(g + 1);
-      if (e <= b) return;
-      tri_batch_out o{out->xyz_f32 ? out->xyz_f32 + 3 * b : nullptr, out->xyz_f64 ? out->xyz_f64 + 3 * b : nullptr,
-                      out->mask ? out->mask + b : nullptr, out->err ? out->err + b : nullptr, out->iters ? out->iters + b : nullptr};
-      status[g] = tri_triangulate_points(engines[g], mode, flags | TRI_ALLOW_TOO_FEW, static_cast<const char*>(xy) + (size_t)b * pb,
-                                         n_point_cams, e - b, cam_stride, &o, &bad[g]);
-      if (status[g] != TRI_OK) msg[g] = tri_last_error();
-      if (bad[g] >= 0) bad[g] += b;
-    });
-  }
-  for (std::thread& t : workers) t.join();
+  st = fan_out(n_engines, [&](int g) -> int {
+    const int64_t b = cut(g), e = cut(g + 1);
+    if (e <= b) return TRI_OK;
+    tri_batch_out o{out->xyz_f32 ? out->xyz_f32 + 3 * b : nullptr, out->xyz_f64 ? out->xyz_f64 + 3 * b : nullptr,
+                    out->mask ? out->mask + b : nullptr, out->err ? out->err + b : nullptr, out->iters ? out->iters + b : nullptr};
+    const int rc = tri_triangulate_points(engines[g], mode, flags | TRI_ALLOW_TOO_FEW, static_cast<const char*>(xy) + (size_t)b * pb,
+                                          n_point_cams, e - b, cam_stride, &o, &bad[g]);
+    if (bad[g] >= 0) bad[g] += b;
+    return rc;
+  });
+  if (st != TRI_OK) return st;
   int64_t first = -1;
-  for (int g = 0; g < n_engines; g++) {
-    if (status[g] != TRI_OK) return fail(status[g], msg[g]);
+  for (int g = 0; g < n_engines; g++)
     if (bad[g] >= 0 && (first < 0 || bad[g] < first)) first = bad[g];
-  }
   if (first_bad_frame) *first_bad_frame = first;
   if (first >= 0 && !(flags & TRI_ALLOW_TOO_FEW))
     return fail(TRI_ERR_TOO_FEW, mode == TRI_MATRIX ? "Too few rays are found" : "Too few detections are found");

@@ -26,7 +26,6 @@
 
 #include <algorithm>
 #include <string>
-#include <thread>
 #include <vector>
 
 #include "tri_classify.cuh"
@@ -822,23 +821,6 @@ link_kernel(const __grid_constant__ RayRig ray, ClsParams p, const int2* __restr
   }
 }
 
-// Grow-only device buffer: the classifier's work space lives on the engine across calls (cudaMalloc /
-// cudaFree of a few hundred MB per call cost up to a second, far more than the kernels).
-struct DevBuf {
-  void* p = nullptr;
-  size_t cap = 0;
-  ~DevBuf() { if (p) cudaFree(p); }
-  cudaError_t alloc(size_t bytes) {
-    if (bytes <= cap && p) return cudaSuccess;
-    if (p) cudaFree(p);
-    p = nullptr; cap = 0;
-    cudaError_t e = cudaMalloc(&p, bytes ? bytes : 1);
-    if (e == cudaSuccess) cap = bytes ? bytes : 1;
-    return e;
-  }
-  template <typename T> T* as() { return static_cast<T*>(p); }
-};
-
 // What (A) hands to (B) for one batch of frames.  Two sets: (A) fills one while (B) reads the other.
 struct LinkInput {
   DevBuf lrec, loff, lcnt, hdr, fdet, fdoff, fdcnt;
@@ -888,12 +870,6 @@ static void free_cls_work(void* w) { delete static_cast<ClsWork*>(w); }
 }  // namespace tri
 
 using namespace tri;
-
-#define TRI_CUDA(call)                                         \
-  do {                                                         \
-    cudaError_t err__ = (call);                                \
-    if (err__ != cudaSuccess) return cuda_fail(err__, #call);  \
-  } while (0)
 
 namespace tri {
 cudaError_t launch_lazy_link(cudaStream_t s, const DltRig<double>& dlt, const RayRig& ray, const ClsParams& p, int n_seq, const int2* d_seq,
@@ -1021,6 +997,78 @@ void cls_stats(tri_classify_stats* stats, const ClsCounters& h, int max_frontier
   stats->ties = (int64_t)h.ties; stats->max_frontier = max_frontier;
 }
 
+// The engine's classifier work space, created on first use.
+ClsWork& cls_work(tri_engine* e) {
+  if (!e->cls_work) { e->cls_work = new ClsWork(); e->cls_work_free = free_cls_work; }
+  return *static_cast<ClsWork*>(e->cls_work);
+}
+
+// The detection CSR of n_frames frames onto the device, and room for the enumeration's counters.
+int cls_upload(tri_engine* e, ClsWork& W, const int32_t* det_offsets, const double* dets_xy, int n_frames, int64_t n_det) {
+  cudaStream_t s = e->stream;
+  const size_t n_offs = (size_t)e->n_cams * (n_frames + 1);
+  TRI_CUDA(W.offs.alloc(sizeof(int32_t) * n_offs));
+  TRI_CUDA(W.dets.alloc(sizeof(double) * 2 * n_det));
+  TRI_CUDA(W.ctr.alloc(sizeof(ClsCounters)));
+  TRI_CUDA(cudaMemcpyAsync(W.offs.p, det_offsets, sizeof(int32_t) * n_offs, cudaMemcpyHostToDevice, s));
+  if (n_det) TRI_CUDA(cudaMemcpyAsync(W.dets.p, dets_xy, sizeof(double) * 2 * n_det, cudaMemcpyHostToDevice, s));
+  return TRI_OK;
+}
+
+// Output bytes: paths [drone][frame][xyz] doubles, assign [drone][frame][camera] and phase [drone][frame] bytes.
+struct ClsOutBytes {
+  size_t paths, assign, phase;
+};
+ClsOutBytes cls_out_bytes(const ClsParams& p) {
+  return {sizeof(double) * 3 * p.n_drones * (size_t)p.n_frames, (size_t)p.n_drones * p.n_frames * p.n_cams, (size_t)p.n_drones * p.n_frames};
+}
+
+// The linking pass's outputs, cleared (assign to -1), and its n_state link states, copied from state_in or zeroed.
+int cls_outputs(tri_engine* e, ClsWork& W, const ClsParams& p, int n_state, const void* state_in) {
+  cudaStream_t s = e->stream;
+  const ClsOutBytes b = cls_out_bytes(p);
+  TRI_CUDA(W.paths.alloc(b.paths));
+  TRI_CUDA(W.assign.alloc(b.assign));
+  TRI_CUDA(W.phase.alloc(b.phase));
+  TRI_CUDA(W.state.alloc(sizeof(LinkState) * (size_t)n_state));
+  TRI_CUDA(W.ctr_link.alloc(sizeof(ClsCounters)));
+  TRI_CUDA(cudaMemsetAsync(W.ctr_link.p, 0, sizeof(ClsCounters), s));
+  TRI_CUDA(cudaMemsetAsync(W.paths.p, 0, b.paths, s));
+  TRI_CUDA(cudaMemsetAsync(W.assign.p, 0xff, b.assign, s));
+  TRI_CUDA(cudaMemsetAsync(W.phase.p, 0, b.phase, s));
+  if (state_in) TRI_CUDA(cudaMemcpyAsync(W.state.p, state_in, sizeof(LinkState) * (size_t)n_state, cudaMemcpyHostToDevice, s));
+  else TRI_CUDA(cudaMemsetAsync(W.state.p, 0, sizeof(LinkState) * (size_t)n_state, s));
+  return TRI_OK;
+}
+
+// D2H of the outputs asked for (paths always), queued on the engine's stream.
+int cls_copy_out(tri_engine* e, ClsWork& W, const ClsParams& p, double* out_paths, int8_t* out_assign, uint8_t* out_phase) {
+  cudaStream_t s = e->stream;
+  const ClsOutBytes b = cls_out_bytes(p);
+  TRI_CUDA(cudaMemcpyAsync(out_paths, W.paths.p, b.paths, cudaMemcpyDeviceToHost, s));
+  if (out_assign) TRI_CUDA(cudaMemcpyAsync(out_assign, W.assign.p, b.assign, cudaMemcpyDeviceToHost, s));
+  if (out_phase) TRI_CUDA(cudaMemcpyAsync(out_phase, W.phase.p, b.phase, cudaMemcpyDeviceToHost, s));
+  return TRI_OK;
+}
+
+// After the linking passes: the outputs (and the last link state, if state_out is given) to the host, the
+// combination-capacity check, the statistics.
+int cls_collect(tri_engine* e, ClsWork& W, const ClsParams& p, double* out_paths, int8_t* out_assign, uint8_t* out_phase,
+                void* state_out, int max_frontier, tri_classify_stats* stats) {
+  cudaStream_t s = e->stream;
+  const int st = cls_copy_out(e, W, p, out_paths, out_assign, out_phase);
+  if (st != TRI_OK) return st;
+  if (state_out) TRI_CUDA(cudaMemcpyAsync(state_out, W.state.p, sizeof(LinkState), cudaMemcpyDeviceToHost, s));
+  ClsCounters h{}, hl{};
+  TRI_CUDA(cudaMemcpyAsync(&h, W.ctr.p, sizeof(h), cudaMemcpyDeviceToHost, s));
+  TRI_CUDA(cudaMemcpyAsync(&hl, W.ctr_link.p, sizeof(hl), cudaMemcpyDeviceToHost, s));
+  TRI_CUDA(cudaStreamSynchronize(s));
+  if (hl.overflow_final) return fail(TRI_ERR_CAPACITY, "more than 128 disjoint combinations kept in one frame");
+  h.phase1 = hl.phase1; h.phase2 = hl.phase2;
+  cls_stats(stats, h, max_frontier, W);
+  return TRI_OK;
+}
+
 // Classify n_seq independent sequences laid back to back in one CSR of n_frames frames (seq_bounds[s] .. seq_bounds[s+1]).
 int cls_run(tri_engine* e, int mode, unsigned flags, int n_drones, const int32_t* det_offsets, const double* dets_xy, int n_frames,
             int n_seq, const int32_t* seq_bounds, double* out_paths, int8_t* out_assign, uint8_t* out_phase, tri_classify_stats* stats) {
@@ -1035,31 +1083,14 @@ int cls_run(tri_engine* e, int mode, unsigned flags, int n_drones, const int32_t
   DeviceGuard g(e->device);
   cudaStream_t s = e->stream;
   ClsParams p = cls_params(e, mode, flags, n_drones, n_frames);
-  if (!e->cls_work) { e->cls_work = new ClsWork(); e->cls_work_free = free_cls_work; }
-  ClsWork& W = *static_cast<ClsWork*>(e->cls_work);
+  ClsWork& W = cls_work(e);
   W.pending = false;
   TRI_CUDA(W.collect(0));  // (a linking pass left behind by a call that failed half-way)
   TRI_CUDA(W.collect(1));
   W.enumerate_ms = W.link_ms = 0;
-  const size_t n_offs = (size_t)C * (n_frames + 1);
-  const size_t sz_paths = sizeof(double) * 3 * n_drones * (size_t)n_frames, sz_assign = (size_t)n_drones * n_frames * C,
-               sz_phase = (size_t)n_drones * n_frames;
   const bool multi = n_seq > 1;
-  TRI_CUDA(W.offs.alloc(sizeof(int32_t) * n_offs));
-  TRI_CUDA(W.dets.alloc(sizeof(double) * 2 * n_det));
-  TRI_CUDA(W.paths.alloc(sz_paths));
-  TRI_CUDA(W.assign.alloc(sz_assign));
-  TRI_CUDA(W.phase.alloc(sz_phase));
-  TRI_CUDA(W.state.alloc(sizeof(LinkState) * (size_t)std::max(n_seq, 1)));
-  TRI_CUDA(W.ctr.alloc(sizeof(ClsCounters)));
-  TRI_CUDA(W.ctr_link.alloc(sizeof(ClsCounters)));
-  TRI_CUDA(cudaMemcpyAsync(W.offs.p, det_offsets, sizeof(int32_t) * n_offs, cudaMemcpyHostToDevice, s));
-  if (n_det) TRI_CUDA(cudaMemcpyAsync(W.dets.p, dets_xy, sizeof(double) * 2 * n_det, cudaMemcpyHostToDevice, s));
-  TRI_CUDA(cudaMemsetAsync(W.ctr_link.p, 0, sizeof(ClsCounters), s));
-  TRI_CUDA(cudaMemsetAsync(W.paths.p, 0, sz_paths, s));
-  TRI_CUDA(cudaMemsetAsync(W.assign.p, 0xff, sz_assign, s));
-  TRI_CUDA(cudaMemsetAsync(W.phase.p, 0, sz_phase, s));
-  TRI_CUDA(cudaMemsetAsync(W.state.p, 0, sizeof(LinkState) * (size_t)std::max(n_seq, 1), s));
+  if ((st = cls_upload(e, W, det_offsets, dets_xy, n_frames, n_det)) != TRI_OK) return st;
+  if ((st = cls_outputs(e, W, p, std::max(n_seq, 1), nullptr)) != TRI_OK) return st;
   TRI_CUDA(cudaMemsetAsync(W.ctr.p, 0, sizeof(ClsCounters), s));
   std::vector<int2> seq;
   if (multi) {  // every sequence links on its own warp: all frames are enumerated first, in one batch
@@ -1080,9 +1111,7 @@ int cls_run(tri_engine* e, int mode, unsigned flags, int n_drones, const int32_t
                               out_phase ? W.phase.as<uint8_t>() : nullptr, W.ctr.as<ClsCounters>()));
     e->launches++;
     TRI_CUDA(cudaEventRecord(W.ev[2], s));
-    TRI_CUDA(cudaMemcpyAsync(out_paths, W.paths.p, sz_paths, cudaMemcpyDeviceToHost, s));
-    if (out_assign) TRI_CUDA(cudaMemcpyAsync(out_assign, W.assign.p, sz_assign, cudaMemcpyDeviceToHost, s));
-    if (out_phase) TRI_CUDA(cudaMemcpyAsync(out_phase, W.phase.p, sz_phase, cudaMemcpyDeviceToHost, s));
+    if ((st = cls_copy_out(e, W, p, out_paths, out_assign, out_phase)) != TRI_OK) return st;
     ClsCounters hz{};
     TRI_CUDA(cudaMemcpyAsync(&hz, W.ctr.p, sizeof(hz), cudaMemcpyDeviceToHost, s));
     TRI_CUDA(cudaStreamSynchronize(s));
@@ -1139,17 +1168,7 @@ int cls_run(tri_engine* e, int mode, unsigned flags, int n_drones, const int32_t
   }
   TRI_CUDA(W.collect(0));
   TRI_CUDA(W.collect(1));
-  ClsCounters hl{};
-  TRI_CUDA(cudaMemcpyAsync(out_paths, W.paths.p, sz_paths, cudaMemcpyDeviceToHost, s));
-  if (out_assign) TRI_CUDA(cudaMemcpyAsync(out_assign, W.assign.p, sz_assign, cudaMemcpyDeviceToHost, s));
-  if (out_phase) TRI_CUDA(cudaMemcpyAsync(out_phase, W.phase.p, sz_phase, cudaMemcpyDeviceToHost, s));
-  TRI_CUDA(cudaMemcpyAsync(&h, W.ctr.p, sizeof(h), cudaMemcpyDeviceToHost, s));
-  TRI_CUDA(cudaMemcpyAsync(&hl, W.ctr_link.p, sizeof(hl), cudaMemcpyDeviceToHost, s));
-  TRI_CUDA(cudaStreamSynchronize(s));
-  if (hl.overflow_final) return fail(TRI_ERR_CAPACITY, "more than 128 disjoint combinations kept in one frame");
-  h.phase1 = hl.phase1; h.phase2 = hl.phase2;
-  cls_stats(stats, h, max_frontier, W);
-  return TRI_OK;
+  return cls_collect(e, W, p, out_paths, out_assign, out_phase, nullptr, max_frontier, stats);
 }
 
 }  // namespace
@@ -1183,11 +1202,9 @@ extern "C" int tri_classify_begin(tri_engine* e, int mode, unsigned flags, int n
   int64_t n_det = 0;
   int st = cls_check(e, mode, n_drones, det_offsets, dets_xy, n_frames, &n_det);
   if (st != TRI_OK) return st;
-  const int C = e->n_cams;
   DeviceGuard g(e->device);
   cudaStream_t s = e->stream;
-  if (!e->cls_work) { e->cls_work = new ClsWork(); e->cls_work_free = free_cls_work; }
-  ClsWork& W = *static_cast<ClsWork*>(e->cls_work);
+  ClsWork& W = cls_work(e);
   W.pending = false;
   W.enumerate_ms = W.link_ms = 0;
   ClsParams p = cls_params(e, mode, flags, n_drones, n_frames);
@@ -1195,12 +1212,7 @@ extern "C" int tri_classify_begin(tri_engine* e, int mode, unsigned flags, int n
   W.job = p;
   W.job_max_frontier = 0;
   if (n_frames == 0) { W.pending = true; return TRI_OK; }
-  const size_t n_offs = (size_t)C * (n_frames + 1);
-  TRI_CUDA(W.offs.alloc(sizeof(int32_t) * n_offs));
-  TRI_CUDA(W.dets.alloc(sizeof(double) * 2 * n_det));
-  TRI_CUDA(W.ctr.alloc(sizeof(ClsCounters)));
-  TRI_CUDA(cudaMemcpyAsync(W.offs.p, det_offsets, sizeof(int32_t) * n_offs, cudaMemcpyHostToDevice, s));
-  if (n_det) TRI_CUDA(cudaMemcpyAsync(W.dets.p, dets_xy, sizeof(double) * 2 * n_det, cudaMemcpyHostToDevice, s));
+  if ((st = cls_upload(e, W, det_offsets, dets_xy, n_frames, n_det)) != TRI_OK) return st;
   int cap = 1 << 14;
   long long leaf_cap = std::max<long long>(4ll << 20, 1024ll * n_frames);
   for (;;) {  // the whole shard's candidates stay resident: on overflow grow the buffers and enumerate again
@@ -1225,44 +1237,19 @@ extern "C" int tri_classify_finish(tri_engine* e, const void* state_in, void* st
   if (!W.pending) return fail(TRI_ERR_ARG, "tri_classify_finish without tri_classify_begin");
   W.pending = false;
   const ClsParams p = W.job;
-  const int C = p.n_cams, n_frames = p.n_frames, n_drones = p.n_drones;
   if (stats) memset(stats, 0, sizeof(*stats));
-  if (n_frames == 0) {
+  if (p.n_frames == 0) {
     if (state_out) { if (state_in) memcpy(state_out, state_in, sizeof(LinkState)); else memset(state_out, 0, sizeof(LinkState)); }
     return TRI_OK;
   }
   if (!out_paths) return fail(TRI_ERR_ARG, "bad output arguments");
   DeviceGuard g(e->device);
-  cudaStream_t s = e->stream;
-  const size_t sz_paths = sizeof(double) * 3 * n_drones * (size_t)n_frames, sz_assign = (size_t)n_drones * n_frames * C,
-               sz_phase = (size_t)n_drones * n_frames;
-  TRI_CUDA(W.paths.alloc(sz_paths));
-  TRI_CUDA(W.assign.alloc(sz_assign));
-  TRI_CUDA(W.phase.alloc(sz_phase));
-  TRI_CUDA(W.state.alloc(sizeof(LinkState)));
-  TRI_CUDA(W.ctr_link.alloc(sizeof(ClsCounters)));
-  TRI_CUDA(cudaMemsetAsync(W.ctr_link.p, 0, sizeof(ClsCounters), s));
-  TRI_CUDA(cudaMemsetAsync(W.paths.p, 0, sz_paths, s));
-  TRI_CUDA(cudaMemsetAsync(W.assign.p, 0xff, sz_assign, s));
-  TRI_CUDA(cudaMemsetAsync(W.phase.p, 0, sz_phase, s));
-  if (state_in) TRI_CUDA(cudaMemcpyAsync(W.state.p, state_in, sizeof(LinkState), cudaMemcpyHostToDevice, s));
-  else TRI_CUDA(cudaMemsetAsync(W.state.p, 0, sizeof(LinkState), s));
-  TRI_CUDA(cudaStreamSynchronize(s));  // the linking pass runs on its own stream
-  int st = cls_link(e, W, 0, p, 1, nullptr, 0, out_assign != nullptr, out_phase != nullptr, W.job_max_frontier);
+  int st = cls_outputs(e, W, p, 1, state_in);
   if (st != TRI_OK) return st;
+  TRI_CUDA(cudaStreamSynchronize(e->stream));  // the linking pass runs on its own stream
+  if ((st = cls_link(e, W, 0, p, 1, nullptr, 0, out_assign != nullptr, out_phase != nullptr, W.job_max_frontier)) != TRI_OK) return st;
   TRI_CUDA(W.collect(0));
-  ClsCounters h{}, hl{};
-  TRI_CUDA(cudaMemcpyAsync(out_paths, W.paths.p, sz_paths, cudaMemcpyDeviceToHost, s));
-  if (out_assign) TRI_CUDA(cudaMemcpyAsync(out_assign, W.assign.p, sz_assign, cudaMemcpyDeviceToHost, s));
-  if (out_phase) TRI_CUDA(cudaMemcpyAsync(out_phase, W.phase.p, sz_phase, cudaMemcpyDeviceToHost, s));
-  if (state_out) TRI_CUDA(cudaMemcpyAsync(state_out, W.state.p, sizeof(LinkState), cudaMemcpyDeviceToHost, s));
-  TRI_CUDA(cudaMemcpyAsync(&h, W.ctr.p, sizeof(h), cudaMemcpyDeviceToHost, s));
-  TRI_CUDA(cudaMemcpyAsync(&hl, W.ctr_link.p, sizeof(hl), cudaMemcpyDeviceToHost, s));
-  TRI_CUDA(cudaStreamSynchronize(s));
-  if (hl.overflow_final) return fail(TRI_ERR_CAPACITY, "more than 128 disjoint combinations kept in one frame");
-  h.phase1 = hl.phase1; h.phase2 = hl.phase2;
-  cls_stats(stats, h, W.job_max_frontier, W);
-  return TRI_OK;
+  return cls_collect(e, W, p, out_paths, out_assign, out_phase, state_out, W.job_max_frontier, stats);
 }
 
 // One C++ process driving several GPUs: every engine enumerates its contiguous frame range on its own host thread,
@@ -1299,17 +1286,10 @@ extern "C" int tri_classify_multi(tri_engine* const* engines, int n_engines, int
       base += b - a;
     }
   }
-  std::vector<int> status(n_engines, TRI_OK);
-  std::vector<std::string> msg(n_engines);
-  std::vector<std::thread> workers;
-  for (int g = 0; g < n_engines; g++)
-    workers.emplace_back([&, g]() {
-      status[g] = tri_classify_begin(engines[g], mode, flags, n_drones, offs[g].data(), dets[g].empty() ? nullptr : dets[g].data(), cut(g + 1) - cut(g));
-      if (status[g] != TRI_OK) msg[g] = tri_last_error();
-    });
-  for (std::thread& t : workers) t.join();
-  for (int g = 0; g < n_engines; g++)
-    if (status[g] != TRI_OK) return fail(status[g], msg[g]);
+  const int rc = fan_out(n_engines, [&](int g) {
+    return tri_classify_begin(engines[g], mode, flags, n_drones, offs[g].data(), dets[g].empty() ? nullptr : dets[g].data(), cut(g + 1) - cut(g));
+  });
+  if (rc != TRI_OK) return rc;
   if (stats) memset(stats, 0, sizeof(*stats));
   std::vector<unsigned char> state(sizeof(LinkState), 0);
   for (int g = 0; g < n_engines; g++) {

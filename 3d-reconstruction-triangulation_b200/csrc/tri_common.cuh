@@ -200,8 +200,6 @@ struct LaunchCtx {
   int64_t* launches;
 };
 
-enum RaySolver { RAY_ANALYTIC_LM = 0, RAY_REFERENCE_LM = 1, RAY_CLOSED_FORM = 2 };
-
 cudaError_t launch_ray_fold(const LaunchCtx& ctx, bool lm, bool f32, int pixfmt, const RayFold<double>& r64,
                             const RayFold<float>& r32, const void* d_xy, int n_use, int64_t n_frames,
                             int64_t cam_stride, const BatchOut& out);

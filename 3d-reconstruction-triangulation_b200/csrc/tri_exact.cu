@@ -126,28 +126,9 @@ dist_from_ray_kernel(const __grid_constant__ RayRig rig, int64_t n, const int32_
   out[i] = ref::dist_from_ray(rig, cam_idx[i], xy[2 * i], xy[2 * i + 1], p);
 }
 
-static int ensure_scratch(tri_engine* e, size_t need) {
-  if (e->scratch_cap >= need) return TRI_OK;
-  if (e->d_scratch) cudaFree(e->d_scratch);
-  e->d_scratch = nullptr;
-  e->scratch_cap = 0;
-  cudaError_t err = cudaMalloc((void**)&e->d_scratch, need);
-  if (err != cudaSuccess) return cuda_fail(err, "cudaMalloc(scratch)");
-  e->scratch_cap = need;
-  return TRI_OK;
-}
-
-static size_t up256(size_t v) { return (v + 255) / 256 * 256; }
-
 }  // namespace tri
 
 using namespace tri;
-
-#define TRI_CUDA(call)                                         \
-  do {                                                         \
-    cudaError_t err__ = (call);                                \
-    if (err__ != cudaSuccess) return cuda_fail(err__, #call);  \
-  } while (0)
 
 extern "C" {
 
@@ -170,9 +151,8 @@ int tri_triangulate_subsets(tri_engine* e, int mode, unsigned flags, int64_t n_i
   const size_t b_offs = up256(sizeof(int32_t) * (n_items + 1)), b_cam = up256(sizeof(int32_t) * total),
                b_xy = up256(sizeof(double) * 2 * total), b_xyz = up256(sizeof(double) * 3 * n_items),
                b_err = up256(sizeof(double) * n_items), b_it = up256(sizeof(int32_t) * n_items);
-  int st = ensure_scratch(e, b_offs + b_cam + b_xy + b_xyz + b_err + b_it + 256);
-  if (st != TRI_OK) return st;
-  char* p = e->d_scratch;
+  TRI_CUDA(e->scratch.alloc(b_offs + b_cam + b_xy + b_xyz + b_err + b_it + 256));
+  char* p = e->scratch.as<char>();
   int32_t* d_offs = (int32_t*)p; p += b_offs;
   int32_t* d_cam = (int32_t*)p; p += b_cam;
   double* d_xy = (double*)p; p += b_xy;
@@ -207,9 +187,8 @@ int tri_dist_from_ray(tri_engine* e, int64_t n, const int32_t* cam_idx, const do
   DeviceGuard g(e->device);
   const size_t b_cam = up256(sizeof(int32_t) * n), b_xy = up256(sizeof(double) * 2 * n), b_p = up256(sizeof(double) * 3 * n),
                b_o = up256(sizeof(double) * n);
-  int st = ensure_scratch(e, b_cam + b_xy + b_p + b_o);
-  if (st != TRI_OK) return st;
-  char* p = e->d_scratch;
+  TRI_CUDA(e->scratch.alloc(b_cam + b_xy + b_p + b_o));
+  char* p = e->scratch.as<char>();
   int32_t* d_cam = (int32_t*)p; p += b_cam;
   double* d_xy = (double*)p; p += b_xy;
   double* d_p = (double*)p; p += b_p;

@@ -129,14 +129,16 @@ def test_too_few_status_matches_plain(torch):
     assert ref["status"] == O.ERR_TOO_FEW and ref["first_bad_frame"] == 1234
 
 
-def test_device_entry_point_matches_host(torch):
+def check_device_entry_point_matches_host(torch, n, p_missing, blank):
+    """The robust device and host calls on n frames with frame `blank` emptied: the same outputs bit for bit, and the
+    first frame with fewer than 2 views (found from the data) reported by both and by the plain host call."""
     cams = rig(8)
     eng = T.Engine(cams, 0)
-    n = 300001
-    xy = S.generate_frames(cams, n, p_outlier=0.1, device="cuda:0")
-    xy[:, 77777] = -1.0
-    first = eng.triangulate_points(T.MATRIX, xy.cpu().numpy(), T.ALLOW_TOO_FEW, want=("xyz_f32", "mask"))["first_bad_frame"]
-    assert 0 <= first <= 77777
+    xy = S.generate_frames(cams, n, p_missing=p_missing, p_outlier=0.1, device="cuda:0")
+    xy[:, blank] = -1.0
+    views = ((xy[..., 0] != -1) & (xy[..., 1] != -1)).sum(0)
+    first = int(torch.nonzero(views < 2)[0])
+    assert eng.triangulate_points(T.MATRIX, xy.cpu().numpy(), T.ALLOW_TOO_FEW, want=("xyz_f32", "mask"))["first_bad_frame"] == first
     for fl in (0, T.F32):
         dev = eng.triangulate_points_robust_device(xy, TAU, T.ALLOW_TOO_FEW | fl, want=("xyz_f64", "xyz_f32", "mask", "err"))
         st, bad = eng.device_status()
@@ -146,6 +148,17 @@ def test_device_entry_point_matches_host(torch):
         for k in ("xyz_f64", "xyz_f32", "err"):
             assert np.array_equal(dev[k].cpu().numpy(), host[k], equal_nan=True), k
         assert np.array_equal(dev["mask"].cpu().numpy().view(np.uint32), host["mask"])
+    return first
+
+
+def test_device_entry_point_matches_host(torch):
+    check_device_entry_point_matches_host(torch, 300001, 0.2, 77777)
+
+
+def test_device_entry_point_matches_host_across_chunks(torch):
+    # 2.5 chunks of the host path, no view missing, so the first frame with too few views is the emptied one, in the
+    # second chunk: the host latch has to report its global index
+    assert check_device_entry_point_matches_host(torch, 2621447, 0.0, 1500000) == 1500000
 
 
 def test_argument_checks(torch):
